@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- Msamples/s of the per-pixel radiance loop (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c2|c3|c4|c5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c2|c3|c4|c5] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Timed workload (config.workload), default c2 = BASELINE.json configs[1]: procedural Cornell box (diffuse walls +
@@ -29,6 +29,14 @@ gather is inside every timed step.
            is followed by 1 s of the same steps so that the sampler sees the load, and `window` says which samples count
 
 --impl reference times the CPU implementation (see reference_arm()); it never loads the product library.
+
+--dump-outputs DIR writes the frame the last timed step delivered to rank 0 -- DIR/radiance.npy (h,w,3) and DIR/rgb.npy
+(h,w,3, the RGB888 bytes), both float32 -- so that two builds can be compared output for output: the inputs depend
+only on the arguments (builtin scene, SEED). A frame larger than DUMP_MAX_BYTES (C5) is cut to DUMP_PIXELS pixels
+drawn with a fixed seed, whose row-major indices go to DIR/pixel_index.npy (float64). The copy into host buffers
+allocated before the warm-up (under 1 ms for C2) and a barrier sit between the timed steps and the 1 s of the same
+steps a short timed region is followed by, so `clocks` may differ slightly from a run without the flag; the timed
+value does not include them.
 """
 import argparse
 import hashlib
@@ -61,6 +69,9 @@ CONFIGS = {
 PARITY_TOL = 1e-2       # same-seed relRMSE per window (SURVEY.md 8(c))
 WINDOW = (64, 36)       # parity window size in pixels
 WINDOW_AT = ((0.5, 0.5), (0.3, 0.74), (0.68, 0.74), (0.08, 0.1))  # centres (fraction of w, h): middle, both spheres, a corner
+DUMP_MAX_BYTES = 64 * 10 ** 6  # --dump-outputs: a 1080p frame (49.8 MB as float32) is written whole
+DUMP_PIXELS = 1 << 20          # pixels kept of a larger frame (33.6 MB with their indices)
+DUMP_SEED = 0
 
 
 def env_int(name, default):
@@ -240,6 +251,21 @@ def window_parity(cfg, frame_rad, threads):
                 len(out), WINDOW[0], WINDOW[1]), "ok": bool(worst <= PARITY_TOL and all(o["oracle_mean"] > 0 for o in out))}
 
 
+def dump_outputs(out_dir, rad, rgb):
+    """--dump-outputs: the frame (radiance (h,w,3) float32, rgb (h,w,3) uint8) as DIR/<name>.npy in float32, cut to a
+    seeded sample of DUMP_PIXELS pixels (plus their indices) when the whole frame would exceed DUMP_MAX_BYTES."""
+    import numpy as np
+    h, w, _ = rad.shape
+    arrays = {"radiance": rad, "rgb": rgb}
+    if 2 * rad.size * 4 > DUMP_MAX_BYTES:
+        idx = np.sort(np.random.default_rng(DUMP_SEED).choice(h * w, DUMP_PIXELS, replace=False))
+        arrays = {k: a.reshape(h * w, 3)[idx] for k, a in arrays.items()}
+        arrays["pixel_index"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a if a.dtype == np.float64 else a.astype(np.float32))
+
+
 # ---------------------------------------------------------------------------------------------
 class Job:
     """One config on this rank's GPU: scene upload, shared frame (or NCCL gather buffers), the step."""
@@ -308,6 +334,26 @@ class Job:
             if read_rad:
                 self.host_rad.copy_(self.f_rad, non_blocking=True)
 
+    def frame_buffers(self):
+        """Pinned host buffers for read_frame."""
+        torch = self.mods[1]
+        c = self.cfg
+        return (torch.empty(c["h"] * c["w"] * 3, dtype=torch.float32).pin_memory(),
+                torch.empty(c["h"] * c["w"] * 3, dtype=torch.uint8).pin_memory())
+
+    def read_frame(self, rad, rgb):
+        """Rank 0, after the last step has completed: (radiance (h,w,3) float32, rgb (h,w,3) uint8) copied into the
+        frame_buffers() rad, rgb."""
+        torch = self.mods[1]
+        c = self.cfg
+        if self.shared is not None:
+            self.shared.read(rgb=rgb.data_ptr(), rad=rad.data_ptr(), stream=self.stream)
+        else:
+            rad.copy_(self.f_rad, non_blocking=True)
+            rgb.copy_(self.f_rgb, non_blocking=True)
+        torch.cuda.synchronize()
+        return rad.numpy().reshape(c["h"], c["w"], 3), rgb.numpy().reshape(c["h"], c["w"], 3)
+
     def check_frame(self):
         """Raises if a device-side wait of the shared frame gave up (G19_ERR_TIMEOUT)."""
         if self.shared is not None:
@@ -332,7 +378,13 @@ def main():
     ap.add_argument("--gather", default="frame", choices=["frame", "nccl"],
                     help="frame: every rank's resolve kernel stores its pixels straight into rank 0's frame over "
                          "NVLink (fused gather, no collective); nccl: compact tile arrays + torch.distributed.gather")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the frame of the last timed step as DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the frames of --impl ours")
     if args.impl == "reference":
         return reference_arm(args)
 
@@ -520,6 +572,7 @@ def main():
     samples_per_step = W * H * SPP
     job = Job(mods, cfg, rank, world, local, args.gather, args.spp_per_pass)
     rt = job.rt
+    dump_bufs = job.frame_buffers() if args.dump_outputs and rank == 0 else None
     sampler = ClockSampler(local)
     if rank == 0:  # rank 0's GPU is the one reported (eight nvidia-smi processes starting at once take seconds to come up)
         sampler.start()
@@ -536,6 +589,11 @@ def main():
     barrier()
     wall1 = time.time()
     ms = max_over_ranks(e0.elapsed_time(e1)) / args.steps
+    frame_out = None
+    if args.dump_outputs:
+        if rank == 0:
+            frame_out = job.read_frame(*dump_bufs)
+        barrier()  # no rank renders the next frame into rank 0's until its copy has landed
     short = ms * args.steps < 1000.0
     if short:  # a short timed region (N = 8: 40 ms): keep the same load up until the sampler has seen it
         for _ in range(int(math.ceil(1000.0 / max(ms, 1e-3)))):  # the same count on every rank (ms is the max over ranks)
@@ -645,6 +703,8 @@ def main():
             "e2e": e2e, "gpu_launches": int(launches), "clocks": clocks, "parity": parity, "roofline": roofline,
             "cpu_baseline": cpu, "other_configs": others,
         }
+        if frame_out is not None:
+            dump_outputs(args.dump_outputs, *frame_out)
         print(json.dumps(line))
         bad = [("timed config " + args.config, parity)] + [(o["config"], o["parity"]) for o in others]
         for name, p in bad:

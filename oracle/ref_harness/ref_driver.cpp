@@ -2,7 +2,8 @@
 //
 // TEST INFRASTRUCTURE ONLY (oracle/): nothing in the product path may link or
 // load this. It is compiled by oracle/Makefile from the sources where they lie
-// under /root/reference (never copied) into oracle/_ref/libg19ref.so.
+// in the reference checkout named by G19_REFERENCE (never copied) into
+// oracle/_ref/libg19ref.so.
 //
 // What it exposes:
 //   * g19ref_render      -- RayTracer::run verbatim (reference raytracer.h:23-87)
@@ -21,7 +22,7 @@
 #include <unordered_map>
 #include <vector>
 
-#include "raytracer.h" // the reference's, via -I/root/reference/include
+#include "raytracer.h" // the reference's, via -I$G19_REFERENCE/include
 
 #include "g19.h" // descriptor structs only
 

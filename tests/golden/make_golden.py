@@ -1,9 +1,9 @@
 """Generates tests/golden/ref_golden.npz from the UNMODIFIED reference (oracle/_ref/libg19ref.so).
 
-Run HERE (the container that has /root/reference), after `make -C oracle ref`:
+Run where a checkout of the reference exists, after `make -C oracle ref G19_REFERENCE=<checkout>`:
     python tests/golden/make_golden.py
 The .npz travels with the repo, so the oracle stays pinned to the reference's own outputs on
-boxes where neither /root/reference nor the compiled oracle/_ref exist.
+machines where neither the reference sources nor the compiled oracle/_ref exist.
 Contents (all produced by calling the reference's public API through oracle/ref_harness):
   c1_sha256, c1_hist        RayTracer::run(500,500) on the main.cpp:24-57 scene
   kat_*                     main.cpp:90-133 entity_test / bbox_test vectors

@@ -2,7 +2,7 @@
 ids AT THE SIZE BASELINE.json states (1920x1080), so that the north-star's "primary hits bit-exact" is checked where
 it is claimed and not only on toy frames (VERDICT r01 weak 4, SURVEY.md hard part 8).
 
-Run HERE (the container that has /root/reference), after `make -C oracle ref`:
+Run where a checkout of the reference exists, after `make -C oracle ref G19_REFERENCE=<checkout>`:
     python tests/golden/make_golden_1080p.py        (about 2 minutes on 8 cores)
 Contents (all from RayTracer::run's own loop, reference include/raytracer.h:41-74, through oracle/ref_harness):
   cornell_ids      (1080, 1920) int8   the walls-first Cornell box (configs[1]/[2] geometry), whole frame

@@ -10,6 +10,8 @@ import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 BIN = os.path.join(ROOT, "tools", "bin", "g19_headless")
+# a checkout of preon7/2019global, optional: the same variable and default oracle/Makefile builds oracle/_ref from
+REFERENCE = os.environ.get("G19_REFERENCE") or os.path.join(os.path.dirname(ROOT), "2019global")
 C1_SHA = "9ab0129419a4c328d4ea865adf74b66e3c91d10c6190cc34373fa2b0187bba85"
 
 
@@ -23,13 +25,13 @@ def _ppm(path):
 
 def test_headers_compile_against_shim_and_glm():
     """No GPU needed: the headers build with the built-in vector shim and, when the reference is
-    mounted, against its vendored GLM (what a real drop-in build uses)."""
+    named by G19_REFERENCE, against its vendored GLM (what a real drop-in build uses)."""
     if not os.path.exists(os.path.join(ROOT, "2019global_b200", "lib2019global_b200.so")):
         pytest.skip("library not built")
     base = ["g++", "-std=c++14", "-fsyntax-only", "-DG19_NO_QT", "-I", os.path.join(ROOT, "include"),
             os.path.join(ROOT, "tools", "g19_headless.cpp")]
     subprocess.run(base, check=True)
-    glm = "/root/reference/3rd_party"
+    glm = os.path.join(REFERENCE, "3rd_party")
     if os.path.isdir(glm):
         subprocess.run(base + ["-I", glm], check=True)
 
@@ -86,10 +88,10 @@ def test_reference_main_cpp_helpers_compile_against_these_headers(tmp_path):
     entity_test, matrix_test, bbox_test -- reference main.cpp:63-133, everything below main()) are compiled, text
     unchanged, against include/*.h + the reference's vendored GLM; the scene literal (main.cpp:24-57) is compiled
     the same way with the Gui lines dropped. A signature or public member that drifted away from the reference's
-    classes fails here. Only runs where the reference is mounted (this container)."""
-    main_cpp = "/root/reference/main.cpp"
+    classes fails here. Only runs where G19_REFERENCE names a checkout of the reference."""
+    main_cpp = os.path.join(REFERENCE, "main.cpp")
     if not os.path.exists(main_cpp):
-        pytest.skip("reference sources not mounted")
+        pytest.skip("no checkout of the reference (G19_REFERENCE, default ../2019global)")
     lines = open(main_cpp).read().split("\n")
     helpers = "\n".join(lines[62:133])                       # main.cpp:63-133
     literal = "\n".join(l for l in lines[23:57] if "Gui" not in l and "window" not in l)  # main.cpp:24-57
@@ -98,7 +100,7 @@ def test_reference_main_cpp_helpers_compile_against_these_headers(tmp_path):
                    '#include "entities.h"\n#include "octree.h"\n#include "glm/ext.hpp"\n'
                    "void entity_test();\nvoid bbox_test();\nvoid matrix_test();\nvoid insert_tris(Octree& scene);\n"
                    "void scene_literal() {\n" + literal + "\n}\n" + helpers + "\n")
-    cmd = ["g++", "-std=c++14", "-fsyntax-only", "-DG19_NO_QT", "-I", os.path.join(ROOT, "include"), "-I", "/root/reference/3rd_party",
-           str(src)]
+    cmd = ["g++", "-std=c++14", "-fsyntax-only", "-DG19_NO_QT", "-I", os.path.join(ROOT, "include"), "-I",
+           os.path.join(REFERENCE, "3rd_party"), str(src)]
     r = subprocess.run(cmd, capture_output=True, text=True)
     assert r.returncode == 0, r.stderr[-3000:]

@@ -15,7 +15,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 def test_two_ranks_bit_identical_to_one():
     import torch
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs 2 GPUs (covered by tools/dist_check.py under gpurun --gpus 2; profiles/README.md)")
+        pytest.skip("needs 2 GPUs (tools/dist_check.py under torchrun with 2 ranks; profiles/README.md)")
     s = socket.socket()
     s.bind(("127.0.0.1", 0))
     port = s.getsockname()[1]

@@ -4,7 +4,9 @@ Three anchors, strongest first:
   1. the compiled, unmodified reference (oracle/_ref/libg19ref.so) when it is present --
      byte equality on everything the reference's public API exposes;
   2. tests/golden/ref_golden.npz -- outputs of that same compiled reference, committed
-     (generator: tests/golden/make_golden.py), so the pin survives without /root/reference;
+     (generator: tests/golden/make_golden.py), so the pin survives without the reference sources;
+     tests/golden/ref_live.npz (generator: tests/golden/make_golden_live.py) holds what the comparisons
+     with oracle/_ref below compare with, so they run where it is not built;
   3. the vectors SURVEY.md section 4 derived from the reference's own dead test functions
      (main.cpp:90-133) and the config-1 sha256 / hit histogram.
 """
@@ -14,10 +16,12 @@ import os
 import numpy as np
 import pytest
 
-from util import mirror, probe_rays, quiet_stdout, zoo
+from util import (assert_same, live_frame_scenes, live_frames, live_golden, live_material, live_zoo, material_descs, mirror,
+                  probe_rays, reference_checker, zoo)
 
 C1_SHA = "9ab0129419a4c328d4ea865adf74b66e3c91d10c6190cc34373fa2b0187bba85"
 GOLD = np.load(os.path.join(os.path.dirname(__file__), "golden", "ref_golden.npz"))
+LIVE = live_golden()
 
 
 def test_config1_sha256_and_histogram(g19, abi, oracle):
@@ -94,72 +98,49 @@ def test_frames_against_golden(g19, abi, oracle):
     assert np.array_equal(t["ids"], GOLD["height_ids"])
 
 
-# ---- live against the compiled reference (skipped where oracle/_ref is absent) ------------------
-def test_live_reference_zoo(g19, oracle, reflib):
+# ---- against the reference: tests/golden/ref_live.npz always, oracle/_ref live where it is built -----------
+def test_live_reference_zoo(g19, oracle):
     z = zoo(g19)
-    a, b = mirror(reflib, z), mirror(oracle, z)
+    got = live_zoo(oracle, z)
+    assert_same(got, {k: LIVE[k] for k in got})
+    b = mirror(oracle, z)
     for i in range(len(z)):
-        assert a.bbox(i).tobytes() == b.bbox(i).tobytes()
-        assert a.triangles(i).tobytes() == b.triangles(i).tobytes()
-        o, d = probe_rays(5000, seed=100 + i)
-        h1, p1, n1 = a.intersect(i, o, d)
-        h2, p2, n2 = b.intersect(i, o, d)
-        assert np.array_equal(h1, h2)
-        m = h1.astype(bool)
-        assert p1[m].tobytes() == p2[m].tobytes() and n1[m].tobytes() == n2[m].tobytes()
-        with quiet_stdout():
-            uv1 = a.texcoord(i, p1[m][:300])
-        assert np.array_equal(uv1, b.texcoord(i, p1[m][:300]))
-    rng = np.random.default_rng(1)
-    tri = rng.uniform(-5, 5, (50, 9))
-    for t in tri:
-        assert a.triangle_derived(t).tobytes() == b.triangle_derived(t).tobytes()
+        assert b.bbox(i).tobytes() == GOLD["zoo_%d_bbox" % i].tobytes()
+        assert b.triangles(i).tobytes() == GOLD["zoo_%d_tris" % i].tobytes()
+    ref = reference_checker()
+    if ref is not None:
+        assert_same(live_zoo(ref, z), got)
+        a = mirror(ref, z)
+        for i in range(len(z)):
+            assert a.bbox(i).tobytes() == b.bbox(i).tobytes()
+            assert a.triangles(i).tobytes() == b.triangles(i).tobytes()
 
 
-def test_live_reference_frames(g19, abi, oracle, reflib):
-    for which, n, (w, h) in ((abi.SCENE_DEFAULT, 0, (120, 120)), (abi.SCENE_CORNELL, 0, (64, 36)),
-                             (abi.SCENE_CORNELL_GLASS, 0, (48, 48)), (abi.SCENE_HEIGHTFIELD, 20, (48, 27))):
-        sc, cam, light = g19.Octree.builtin(which, n=n, w=w, h=h)
-        a = mirror(reflib, sc).trace(cam, light, w, h, threads=4)
-        b = mirror(oracle, sc).trace(cam, light, w, h, threads=4)
-        for k in ("ids", "points", "normals", "rgb"):
-            assert a[k].tobytes() == b[k].tobytes(), (which, k)
-        assert np.array_equal(mirror(reflib, sc).render(cam, light, w, h), a["rgb"])  # run() itself
+def test_live_reference_frames(g19, abi, oracle):
+    got = live_frames(oracle, g19, abi)
+    assert_same(got, {k: LIVE[k] for k in got})
+    for which, _, _ in live_frame_scenes(abi):
+        assert np.array_equal(got["frame_%d_run" % which], got["frame_%d_rgb" % which])  # run() itself
+    ref = reference_checker()
+    if ref is not None:
+        assert_same(live_frames(ref, g19, abi), got)
 
 
-def test_live_reference_material_fields(g19, abi, oracle, reflib):
+def test_live_reference_material_fields(g19, oracle):
     """Material's public fields beyond `color` (reference include/material.h:24-29: diffuse_color, specular_color,
     shader_parameters, specular_power) travel in g19_entity_desc: a caller who assigns them after construction gets
     the reference's own blinn_phong_texture result (material.h:48-62), byte for byte, from the restatement -- and a
-    frame shaded with them equals the compiled reference's."""
-    rng = np.random.default_rng(11)
-    custom = dict(shader_parameters=(0.25, 0.5, 0.6), specular_color=(0.9, 0.4, 0.2), specular_power=9.0, diffuse_color=(0.1, 0.2, 0.3))
-    descs = [g19.ImpSphere((3, 1, 0), 2.0, (1, 0, 2), **custom),
-             g19.ImpTriangle((4, -5, -3), (4, 5, -3), (4, 0, 4), (0, 1, 1), **custom),
-             g19.ImpSphere((3, -3, 2), 1.5, (0, 1, 0))]  # untouched Material: the defaults
+    frame shaded with them equals the reference's."""
+    descs = material_descs(g19)
     assert descs[0].material_set == 1 and descs[2].material_set == 0
-    a = reflib.scene((-20,) * 3, (20,) * 3, descs)
-    b = oracle.scene((-20,) * 3, (20,) * 3, descs)
-    for i in range(3):
-        for _ in range(40):
-            o = (-10, 0, 0)
-            p = rng.uniform(-3, 3, 3)
-            n = rng.normal(size=3)
-            n /= np.linalg.norm(n)
-            d = p - np.array(o)
-            light = rng.uniform(-10, 10, 3)
-            u, v = (int(x) for x in rng.integers(0, 200, 2))
-            with quiet_stdout():
-                ca = a.shade(i, o, d, light, p, n, u, v)
-            cb = b.shade(i, o, d, light, p, n, u, v)
-            assert ca.tobytes() == cb.tobytes(), (i, ca, cb)
-    cam = g19.Camera((-10, 0, 0), (1, 0, 0), 0.02)
-    with quiet_stdout():
-        fa = a.trace(cam, (-8, 6, 9), 96, 96, want=("rgb", "ids"), threads=2)
-    fb = b.trace(cam, (-8, 6, 9), 96, 96, want=("rgb", "ids"), threads=2)
-    assert np.array_equal(fa["ids"], fb["ids"]) and np.array_equal(fa["rgb"], fb["rgb"])
-    assert (fa["ids"] >= 0).sum() > 500
+    got = live_material(oracle, g19)
+    assert_same(got, {k: LIVE[k] for k in got})
+    ref = reference_checker()
+    if ref is not None:
+        assert_same(live_material(ref, g19), got)
+    assert (got["material_ids"] >= 0).sum() > 500
     # the custom fields do change the picture
+    cam = g19.Camera((-10, 0, 0), (1, 0, 0), 0.02)
     plain = oracle.scene((-20,) * 3, (20,) * 3, [g19.ImpSphere((3, 1, 0), 2.0, (1, 0, 2)), g19.ImpTriangle((4, -5, -3), (4, 5, -3), (4, 0, 4), (0, 1, 1)),
                                                  descs[2]]).trace(cam, (-8, 6, 9), 96, 96, want=("rgb",), threads=2)
-    assert not np.array_equal(plain["rgb"], fb["rgb"])
+    assert not np.array_equal(plain["rgb"], got["material_rgb"])

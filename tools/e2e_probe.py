@@ -1,6 +1,6 @@
 import importlib, os, sys, time
 import torch
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 g19 = importlib.import_module("2019global_b200"); abi = g19.abi
 W,H,SPP,D=1920,1080,64,5
 sc, cam, light = g19.Octree.builtin(abi.SCENE_CORNELL, n=0, w=W, h=H)
