@@ -1,7 +1,7 @@
 """ctypes mirror of include/g19.h (struct layouts and enum values only)."""
 import ctypes as C
 
-ABI_VERSION = 5
+ABI_VERSION = 6
 
 # enum g19_entity_kind (reference include/entities.h, one value per class)
 IMP_SPHERE, IMP_TRIANGLE, EXP_RECTANGLE, EXP_BOX, EXP_SPHERE, EXP_QUAD, EXP_CUBE, EXP_CONE = range(8)
@@ -16,6 +16,8 @@ SHAPES_REF, SHAPES_FIXED = 0, 1
 SCENE_DEFAULT, SCENE_CORNELL, SCENE_CORNELL_GLASS, SCENE_HEIGHTFIELD, SCENE_HEIGHTFIELD_ROOM = range(5)
 # status
 OK, ERR_INVALID, ERR_NO_DEVICE, ERR_CUDA, ERR_NO_SCENE, ERR_CANCELLED, ERR_LIMIT, ERR_REJECTED, ERR_TIMEOUT = range(9)
+# g19_cast_rays flags
+CAST_ANY_HIT, CAST_COUNT = 1, 2
 K_EXTEND, K_SHADE, K_SHADOW, K_ACCUM, K_REF_VIS, K_REF_SHADE, K_OTHER = range(7)
 CLASS_NAMES = ["raygen_extend", "bounce", "shadow", "accumulate", "ref_visibility", "ref_shade", "other", "_"]
 

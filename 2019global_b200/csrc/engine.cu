@@ -83,6 +83,9 @@ struct g19_ctx {
     // frame buffers for the host-pointer entry point
     DevBuf rgb_f, ids_f, rad_f;
     PathWork work;
+    // ray queries (g19_cast_rays*): their own state, no render buffer
+    PathCastWork cast;
+    DevBuf cast_io; // g19_cast_rays: the rays and the outputs staged on the device
 
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
     cudaEvent_t cls0 = nullptr, cls1 = nullptr;
@@ -609,9 +612,10 @@ void g19_destroy(g19_ctx* ctx) {
     cudaDeviceSynchronize();
     for (DevBuf* b : {&ctx->heavy, &ctx->ref_nodes, &ctx->ref_ents, &ctx->ref_entities, &ctx->ref_tris, &ctx->ids_l, &ctx->points_l,
                       &ctx->normals_l, &ctx->rgb_l, &ctx->colour_l, &ctx->counters, &ctx->rgb_f, &ctx->ids_f,
-                      &ctx->rad_f})
+                      &ctx->rad_f, &ctx->cast_io})
         b->release();
     path_release(ctx->path, ctx->work);
+    ctx->cast.counters.release();
     if (ctx->ev0) cudaEventDestroy(ctx->ev0);
     if (ctx->ev1) cudaEventDestroy(ctx->ev1);
     if (ctx->cls0) cudaEventDestroy(ctx->cls0);
@@ -672,6 +676,7 @@ static int render_any(g19_ctx* ctx, const g19_camera* cam, const double light[3]
     ctx->cancel.store(0);
     ctx->progress_milli.store(0);
     ctx->stats = g19_stats{};
+    ctx->cast.counts_pending = false; // (the statistics now belong to this render)
     TileMap map = make_tile_map(p->width, p->height, p->rank, p->world);
     G19_CUDA(ctx, cudaEventRecord(ctx->ev0, s));
     if (p->mode == G19_MODE_REF) {
@@ -1020,6 +1025,7 @@ int g19_get_stats(g19_ctx* ctx, g19_stats* out) {
         ctx->stats.render_ms = ms;
         std::string perr;
         int rc = path_finish_stats(ctx->work, ctx->stats, perr);
+        if (rc == G19_OK) rc = path_cast_finish_stats(ctx->cast, ctx->stats, perr);
         if (rc != G19_OK) {
             ctx->err = perr;
             return rc;
@@ -1027,6 +1033,69 @@ int g19_get_stats(g19_ctx* ctx, g19_stats* out) {
         ctx->stats_pending = false;
     }
     *out = ctx->stats;
+    return G19_OK;
+}
+
+// ---- ray queries ------------------------------------------------------------------------------------
+static int check_cast(g19_ctx* ctx, int32_t n, const float* rays, uint32_t flags, const int32_t* ids, const float* t,
+                      const float* normals) {
+    if (!ctx) return G19_ERR_INVALID;
+    const char* bad = nullptr;
+    if (n < 0) bad = "n < 0";
+    else if (n > 0 && (!rays || !ids)) bad = "rays and out_entity are required";
+    else if (reinterpret_cast<uintptr_t>(rays) % 16 != 0) bad = "rays must be 16-byte aligned";
+    else if ((flags & ~(G19_CAST_ANY_HIT | G19_CAST_COUNT)) != 0u) bad = "unknown flag bits";
+    else if ((flags & G19_CAST_ANY_HIT) && (t || normals)) bad = "an any-hit cast has no t or normal outputs";
+    if (bad) {
+        ctx->err = std::string("g19_cast_rays: ") + bad;
+        return G19_ERR_INVALID;
+    }
+    if (!ctx->has_scene) return G19_ERR_NO_SCENE;
+    return G19_OK;
+}
+
+int g19_cast_rays_device(g19_ctx* ctx, int32_t n, const float* d_rays, uint32_t flags, int32_t* d_entity, float* d_t,
+                         float* d_normal, void* stream) {
+    int rc = check_cast(ctx, n, d_rays, flags, d_entity, d_t, d_normal);
+    if (rc != G19_OK || n == 0) return rc;
+    G19_CUDA(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    ctx->stats = g19_stats{};
+    ctx->stats_pending = false;
+    ctx->work.totals_pending = false; // (the statistics now belong to this cast)
+    G19_CUDA(ctx, cudaEventRecord(ctx->ev0, s));
+    std::string perr;
+    rc = path_cast(ctx->path, ctx->cast, ctx->tune, n, d_rays, flags, d_entity, d_t, d_normal, s, ctx->sm_count, ctx->stats, perr);
+    if (rc != G19_OK) {
+        ctx->err = perr;
+        return rc;
+    }
+    G19_CUDA(ctx, cudaEventRecord(ctx->ev1, s));
+    ctx->stats_pending = true;
+    return G19_OK;
+}
+
+int g19_cast_rays(g19_ctx* ctx, int32_t n, const float* rays, uint32_t flags, int32_t* out_entity, float* out_t,
+                  float* out_normal) {
+    int rc = check_cast(ctx, n, rays, flags, out_entity, out_t, out_normal);
+    if (rc != G19_OK || n == 0) return rc;
+    G19_CUDA(ctx, cudaSetDevice(ctx->device));
+    // one buffer: rays (32 B per ray) | ids | t | normals
+    const size_t un = size_t(n), b_rays = un * 32, b_ids = (un * 4 + 15) & ~size_t(15), b_t = (un * 4 + 15) & ~size_t(15);
+    G19_CUDA(ctx, ctx->cast_io.ensure(b_rays + b_ids + b_t + un * 12));
+    char* base = ctx->cast_io.as<char>();
+    float* d_rays = reinterpret_cast<float*>(base);
+    int32_t* d_ids = reinterpret_cast<int32_t*>(base + b_rays);
+    float* d_t = out_t ? reinterpret_cast<float*>(base + b_rays + b_ids) : nullptr;
+    float* d_nrm = out_normal ? reinterpret_cast<float*>(base + b_rays + b_ids + b_t) : nullptr;
+    cudaStream_t s = ctx->stream;
+    G19_CUDA(ctx, cudaMemcpyAsync(d_rays, rays, b_rays, cudaMemcpyHostToDevice, s));
+    rc = g19_cast_rays_device(ctx, n, d_rays, flags, d_ids, d_t, d_nrm, s);
+    if (rc != G19_OK) return rc;
+    G19_CUDA(ctx, cudaMemcpyAsync(out_entity, d_ids, un * 4, cudaMemcpyDeviceToHost, s));
+    if (out_t) G19_CUDA(ctx, cudaMemcpyAsync(out_t, d_t, un * 4, cudaMemcpyDeviceToHost, s));
+    if (out_normal) G19_CUDA(ctx, cudaMemcpyAsync(out_normal, d_nrm, un * 12, cudaMemcpyDeviceToHost, s));
+    G19_CUDA(ctx, cudaStreamSynchronize(s));
     return G19_OK;
 }
 

@@ -826,6 +826,46 @@ struct ClassClock { // non-blocking CUDA-event bracket around each launch group
 
 } // namespace
 
+PassArgs path_pass_setup(const PathSceneBuffers& b, const PathTuning& tune, bool count) {
+    PassArgs pa{};
+    pa.scene = b.view;
+    pa.kind_mask = (b.has_bsdf[G19_BSDF_DIFFUSE] ? 1u : 0u) | (b.has_bsdf[G19_BSDF_MIRROR] ? 2u : 0u) |
+                   (b.has_bsdf[G19_BSDF_GLASS] ? 4u : 0u);
+
+    // stage the breadth-first prefix of the tree and the first primitives (<= ~24 KB)
+    pa.stage_nodes = std::min(b.view.n_nodes, 1024);
+    // flat scene (one leaf, <= 192 primitives): intersection + shading records and lights staged whole;
+    // a tree scene reaches its primitives through leaf index lists, so only the node prefix is staged
+    const bool flat = b.view.n_nodes == 1 && b.view.n_index == b.view.n_prims && b.view.n_prims <= 192;
+    pa.stage_prims = flat ? b.view.n_prims : 0;
+    pa.stage_cold = flat ? b.view.n_prims : 0;
+    pa.stage_lights = (pa.stage_cold > 0 && b.view.n_lights <= 32) ? b.view.n_lights : 0;
+    if (b.view.n_lights > 32) pa.stage_cold = 0; // not a "flat, fully staged" scene: the generic kernels take it
+    pa.stack_levels = b.view.tree_depth + 1;
+    // tree scenes: the bounce kernels queue their rays (2 per vertex at most) for trace_kernel
+    pa.refill = tune.refill;
+    // tree walk: leaf tests spread over the whole warp, 8 primitives per ray and round (heightfield 1080p x 32 spp:
+    // sequential 4 per round 107.1 ms, cooperative 4 / 8 / 16 per round 115.4 / 104.9 / 105.4)
+    pa.coop_leaf = tune.coop_leaf;
+    pa.walk_steps = tune.walk_steps > 0 ? tune.walk_steps : (tune.walk ? 2 : 4); // measured (room scene, ms per 1080p x 64 spp): new walk 2 / 4 / 8 steps = 780 / 838 / 961
+    pa.leaf_batch = tune.leaf_batch > 0 ? tune.leaf_batch : (pa.coop_leaf ? 16 : 4); // cooperative: the whole leaf in one go (leaf max 8 / 12 / 16 at batch 16: 97.7 / 96.9 / 97.8 ms)
+    pa.raygen_occ = tune.raygen_occ;
+    pa.trace_occ = tune.trace_occ;
+    pa.bounce_occ = tune.bounce_occ;
+    pa.bvh_spec = tune.bvh_spec;
+    pa.fold_last = 0;
+    pa.walk = tune.walk ? (count ? 2 : 1) : 0; // the new walk counts its node / primitive tests when asked (params.profile)
+    if (tune.walk >= 3 && b.view.bvh_root != 0xffffffffu && b.view.bvh_nodes) {
+        pa.walk = tune.walk == 4 ? (count ? 6 : 5) : 3; // bounding-volume hierarchy, binary / 4-wide (the latter counts its tests when asked)
+        // node visits per round, room scene: binary 4 / 6 / 8 / 12 = 437 / 423 / 418 / 418 ms; 4-wide 4 / 6 / 8 / 12 = 346 / 345 / 364 / 382 ms
+        if (tune.walk_steps <= 0) pa.walk_steps = tune.walk == 4 ? 5 : 8;
+        pa.stack_levels = std::max(pa.stack_levels, tune.bvh_stack);
+        pa.coop_leaf = 0;
+        pa.stage_nodes = 0; // no octree prefix in shared memory: the L1 the walk lives off is what the carve-out leaves
+    }
+    return pa;
+}
+
 int path_render(PathSceneBuffers& b, PathWork& w, const PathRenderArgs& a, g19_stats& stats, std::string& err) {
     const g19_params& p = a.params;
     if (p.spp < 1 || p.max_depth < 0 || p.max_depth > kMaxPathDepth || (p.max_depth == 0 && !a.ids_l)) {
@@ -836,8 +876,7 @@ int path_render(PathSceneBuffers& b, PathWork& w, const PathRenderArgs& a, g19_s
     const size_t npix = size_t(a.map.n_local_pix);
     if (npix == 0) return G19_OK;
     path_clear_launch_error();
-    PassArgs pa0{};
-    pa0.scene = b.view;
+    PassArgs pa0 = path_pass_setup(b, a.tune, p.profile != 0);
     for (int k = 0; k < 3; ++k) {
         pa0.cam.pos[k] = float(a.cam.pos[k]);
         pa0.cam.top_left[k] = float(a.cam.top_left[k]);
@@ -847,40 +886,6 @@ int path_render(PathSceneBuffers& b, PathWork& w, const PathRenderArgs& a, g19_s
     pa0.map = a.map;
     pa0.seed = p.seed;
     pa0.max_depth = p.max_depth;
-    pa0.kind_mask = (b.has_bsdf[G19_BSDF_DIFFUSE] ? 1u : 0u) | (b.has_bsdf[G19_BSDF_MIRROR] ? 2u : 0u) |
-                    (b.has_bsdf[G19_BSDF_GLASS] ? 4u : 0u);
-
-    // stage the breadth-first prefix of the tree and the first primitives (<= ~24 KB)
-    pa0.stage_nodes = std::min(b.view.n_nodes, 1024);
-    // flat scene (one leaf, <= 192 primitives): intersection + shading records and lights staged whole;
-    // a tree scene reaches its primitives through leaf index lists, so only the node prefix is staged
-    const bool flat = b.view.n_nodes == 1 && b.view.n_index == b.view.n_prims && b.view.n_prims <= 192;
-    pa0.stage_prims = flat ? b.view.n_prims : 0;
-    pa0.stage_cold = flat ? b.view.n_prims : 0;
-    pa0.stage_lights = (pa0.stage_cold > 0 && b.view.n_lights <= 32) ? b.view.n_lights : 0;
-    if (b.view.n_lights > 32) pa0.stage_cold = 0; // not a "flat, fully staged" scene: the generic kernels take it
-    pa0.stack_levels = b.view.tree_depth + 1;
-    // tree scenes: the bounce kernels queue their rays (2 per vertex at most) for trace_kernel
-    pa0.refill = a.tune.refill;
-    // tree walk: leaf tests spread over the whole warp, 8 primitives per ray and round (heightfield 1080p x 32 spp:
-    // sequential 4 per round 107.1 ms, cooperative 4 / 8 / 16 per round 115.4 / 104.9 / 105.4)
-    pa0.coop_leaf = a.tune.coop_leaf;
-    pa0.walk_steps = a.tune.walk_steps > 0 ? a.tune.walk_steps : (a.tune.walk ? 2 : 4); // measured (room scene, ms per 1080p x 64 spp): new walk 2 / 4 / 8 steps = 780 / 838 / 961
-    pa0.leaf_batch = a.tune.leaf_batch > 0 ? a.tune.leaf_batch : (pa0.coop_leaf ? 16 : 4); // cooperative: the whole leaf in one go (leaf max 8 / 12 / 16 at batch 16: 97.7 / 96.9 / 97.8 ms)
-    pa0.raygen_occ = a.tune.raygen_occ;
-    pa0.trace_occ = a.tune.trace_occ;
-    pa0.bounce_occ = a.tune.bounce_occ;
-    pa0.bvh_spec = a.tune.bvh_spec;
-    pa0.fold_last = 0;
-    pa0.walk = a.tune.walk ? (p.profile ? 2 : 1) : 0; // the new walk counts its node / primitive tests under params.profile
-    if (a.tune.walk >= 3 && b.view.bvh_root != 0xffffffffu && b.view.bvh_nodes) {
-        pa0.walk = a.tune.walk == 4 ? (p.profile ? 6 : 5) : 3; // bounding-volume hierarchy, binary / 4-wide (the latter counts its tests under params.profile)
-        // node visits per round, room scene: binary 4 / 6 / 8 / 12 = 437 / 423 / 418 / 418 ms; 4-wide 4 / 6 / 8 / 12 = 346 / 345 / 364 / 382 ms
-        if (a.tune.walk_steps <= 0) pa0.walk_steps = a.tune.walk == 4 ? 5 : 8;
-        pa0.stack_levels = std::max(pa0.stack_levels, a.tune.bvh_stack);
-        pa0.coop_leaf = 0;
-        pa0.stage_nodes = 0; // no octree prefix in shared memory: the L1 the walk lives off is what the carve-out leaves
-    }
     const bool fused = path_scene_is_flat(pa0); // flat scenes trace inside the bounce kernels
     // primary-hit AOV: the un-jittered ray of every pixel (the reference's ray) through this engine's structures
     if (a.ids_l) {
@@ -1300,6 +1305,52 @@ int path_finish_stats(PathWork& w, g19_stats& stats, std::string& err) {
         if (cudaEventElapsedTime(&ms, w.events[i], w.events[i + 1]) == cudaSuccess) stats.class_ms[w.event_class[i / 2]] += ms;
     }
     w.totals_pending = false;
+    return G19_OK;
+}
+
+int path_cast(const PathSceneBuffers& b, PathCastWork& cw, const PathTuning& tune, int32_t n, const float* d_rays, uint32_t flags,
+              int32_t* d_ids, float* d_t, float* d_normals, cudaStream_t stream, int sm_count, g19_stats& stats, std::string& err) {
+    const bool any = (flags & G19_CAST_ANY_HIT) != 0u, count = (flags & G19_CAST_COUNT) != 0u;
+    cudaError_t e = cw.counters.ensure(10 * sizeof(unsigned long long));
+    if (e == cudaSuccess) e = cudaMemsetAsync(cw.counters.p, 0, 10 * sizeof(unsigned long long), stream);
+    if (e != cudaSuccess) {
+        err = std::string("path_cast: ") + cudaGetErrorString(e);
+        return G19_ERR_CUDA;
+    }
+    PassArgs pa = path_pass_setup(b, tune, count);
+    pa.totals = static_cast<unsigned long long*>(cw.counters.p);
+    CastArgs c;
+    c.rays = reinterpret_cast<const float4*>(d_rays);
+    c.ids = d_ids;
+    c.t = d_t;
+    c.normals = d_normals;
+    c.n = uint32_t(n);
+    c.cursor = reinterpret_cast<uint32_t*>(pa.totals + 9);
+    path_clear_launch_error();
+    launch_cast(pa, c, any, sm_count, stream);
+    if (const char* le = path_launch_error()) {
+        err = le;
+        path_clear_launch_error();
+        cudaGetLastError();
+        return G19_ERR_CUDA;
+    }
+    (any ? stats.shadow_segments : stats.extend_segments) = uint64_t(n);
+    stats.kernel_launches = 1;
+    cw.counts_pending = count;
+    return G19_OK;
+}
+
+int path_cast_finish_stats(PathCastWork& cw, g19_stats& stats, std::string& err) {
+    if (!cw.counts_pending) return G19_OK;
+    unsigned long long h[2];
+    cudaError_t e = cudaMemcpy(h, static_cast<const unsigned long long*>(cw.counters.p) + 7, sizeof h, cudaMemcpyDeviceToHost);
+    if (e != cudaSuccess) {
+        err = std::string("path_cast_finish_stats: ") + cudaGetErrorString(e);
+        return G19_ERR_CUDA;
+    }
+    stats.node_tests = h[0];
+    stats.prim_tests = h[1];
+    cw.counts_pending = false;
     return G19_OK;
 }
 

@@ -226,6 +226,15 @@ int path_build_top_table(const PathNodeD* d_nodes, int top_level, uint2* d_table
 int path_upload(PathSceneBuffers& b, const g19_scene& scene, const PathTuning& tune, cudaStream_t stream, std::string& err);
 int path_render(PathSceneBuffers& b, PathWork& w, const PathRenderArgs& a, g19_stats& stats, std::string& err);
 int path_finish_stats(PathWork& w, g19_stats& stats, std::string& err);
+// Batched ray queries (g19_cast_rays) against the PATH view, on `stream`. Their state is their own, so a cast leaves every
+// render buffer as it was.
+struct PathCastWork {
+    DeviceArray counters;        // uint64[10]: walk tallies at [7] / [8] (where flush_walk_counts adds them), ray cursor at [9]
+    bool counts_pending = false; // the last call was a counting cast whose tallies g19_get_stats has not read yet
+};
+int path_cast(const PathSceneBuffers& b, PathCastWork& cw, const PathTuning& tune, int32_t n, const float* d_rays, uint32_t flags,
+              int32_t* d_ids, float* d_t, float* d_normals, cudaStream_t stream, int sm_count, g19_stats& stats, std::string& err);
+int path_cast_finish_stats(PathCastWork& cw, g19_stats& stats, std::string& err);
 void path_release(PathSceneBuffers& b, PathWork& w);
 
 // ---- path_kernels.cu -------------------------------------------------------
@@ -281,6 +290,9 @@ struct PassArgs {
     int32_t walk;          // tree walk variant (PathTuning::walk); +2 when the walk counts its node / primitive tests
 };
 
+// path.cu: the PassArgs fields that follow from the scene and the tuning alone (staging sizes, walk and its knobs);
+// count = the walk tallies its node / primitive tests
+PassArgs path_pass_setup(const PathSceneBuffers& b, const PathTuning& tune, bool count);
 void launch_raygen_extend(const PassArgs& a, int sm_count, cudaStream_t s);
 // false = nothing to launch for this (bounce, kind): specular vertices on the last segment
 bool launch_bounce(const PassArgs& a, int bounce, int kind, int sm_count, cudaStream_t s);
@@ -297,6 +309,17 @@ bool path_scene_is_flat(const PassArgs& a);
 bool launch_bounce_first_fused(const PassArgs& a, int sm_count, cudaStream_t s);
 void launch_accumulate(const PassArgs& a, cudaStream_t s);
 void launch_primary(const PassArgs& a, int32_t* ids_l, double* points_l, double* normals_l, int sm_count, cudaStream_t s);
+// batched ray queries (g19_cast_rays): n ray records of two float4 (origin, tmax) (direction, -) -> entity id per ray and,
+// when non-null, t and the normal (3 floats); cursor = the tree kernel's ray fetch counter (zeroed by the caller)
+struct CastArgs {
+    const float4* rays;
+    int32_t* ids;
+    float* t;
+    float* normals;
+    uint32_t n;
+    uint32_t* cursor;
+};
+void launch_cast(const PassArgs& a, const CastArgs& c, bool any, int sm_count, cudaStream_t s);
 void launch_resolve(const TileMap& map, const float* accum, int spp, float* rad_l, uint8_t* rgb_l, cudaStream_t s);
 const char* path_launch_error(); // first failed launch/attribute call since the last clear, or nullptr
 void path_clear_launch_error();

@@ -2311,6 +2311,30 @@ template <bool COOP, int WALK, int OCC = 3> __global__ void __launch_bounds__(kT
 // mode: the ids must equal REF's wherever "last hit wins" coincides with "nearest hit" (tests/test_path_link.py),
 // and with max_depth = 0 these three arrays feed the reference's own shade (ref_shade_kernel), so the default
 // scene closes the loop through the PATH pipeline.
+
+// The entity a hit on primitive `prim` at p (ray direction d) reports, and its normal: for a triangle or parallelogram
+// the geometric normal turned against the ray, for a sphere (p - c) / r. primary_kernel and cast_kernel share it.
+template <bool ALL>
+__device__ __forceinline__ int32_t hit_entity(const SceneAccess<ALL>& S, uint32_t prim, float3 p, float3 d, float3& ng) {
+    const float4 r0 = S.hot_row(prim, 0), tag = S.hot_row(prim, 3);
+    float4 c0, c1;
+    S.cold(prim, c0, c1);
+    ng = f3(c0.x, c0.y, c0.z);
+    int half = 0;
+    if (tag.z == 0.0f) {
+        ng = (p - f3(r0.x, r0.y, r0.z)) * __fdividef(1.0f, r0.w);
+    } else {
+        if (tag.z > 1.5f) { // merged parallelogram: which of its two triangles (the builder's b1 >= b2 rule)
+            const float4 r1 = S.hot_row(prim, 1);
+            const float b1 = fmaf(r0.x, p.x, fmaf(r0.y, p.y, fmaf(r0.z, p.z, r0.w)));
+            const float b2 = fmaf(r1.x, p.x, fmaf(r1.y, p.y, fmaf(r1.z, p.z, r1.w)));
+            half = b1 >= b2 ? 0 : 1;
+        }
+        if (dot(ng, d) > 0.0f) ng = -ng;
+    }
+    return S.g->prim_entity[2 * size_t(prim) + half];
+}
+
 template <bool ALL>
 __global__ void __launch_bounds__(kThreads, 2) primary_kernel(const PassArgs a, int32_t* __restrict__ ids, double* __restrict__ points,
                                                               double* __restrict__ normals) {
@@ -2344,23 +2368,8 @@ __global__ void __launch_bounds__(kThreads, 2) primary_kernel(const PassArgs a, 
             double px = DBL_MAX, py = DBL_MAX, pz = DBL_MAX, nx = 0, ny = 0, nz = 0; // a miss looks like REF's (ref_visibility_kernel)
             if (hit) {
                 const float3 p = o + d * t;
-                const float4 r0 = S.hot_row(prim, 0), tag = S.hot_row(prim, 3);
-                float4 c0, c1;
-                S.cold(prim, c0, c1);
-                float3 ng = f3(c0.x, c0.y, c0.z);
-                int half = 0;
-                if (tag.z == 0.0f) {
-                    ng = (p - f3(r0.x, r0.y, r0.z)) * __fdividef(1.0f, r0.w);
-                } else {
-                    if (tag.z > 1.5f) { // merged parallelogram: which of its two triangles (the builder's b1 >= b2 rule)
-                        const float4 r1 = S.hot_row(prim, 1);
-                        const float b1 = fmaf(r0.x, p.x, fmaf(r0.y, p.y, fmaf(r0.z, p.z, r0.w)));
-                        const float b2 = fmaf(r1.x, p.x, fmaf(r1.y, p.y, fmaf(r1.z, p.z, r1.w)));
-                        half = b1 >= b2 ? 0 : 1;
-                    }
-                    if (dot(ng, d) > 0.0f) ng = -ng;
-                }
-                id = a.scene.prim_entity[2 * size_t(prim) + half];
+                float3 ng;
+                id = hit_entity(S, prim, p, d, ng);
                 px = double(p.x); py = double(p.y); pz = double(p.z);
                 nx = double(ng.x); ny = double(ng.y); nz = double(ng.z);
             }
@@ -2369,6 +2378,102 @@ __global__ void __launch_bounds__(kThreads, 2) primary_kernel(const PassArgs a, 
             if (normals) { normals[lp] = nx; normals[size_t(n) + lp] = ny; normals[2 * size_t(n) + lp] = nz; }
         }
     }
+}
+
+// ---- batched ray queries (g19_cast_rays) ---------------------------------------------------------
+// Rays in, hits out, through the render's own structures: the pair loops of a flat scene, the selected walk of a tree
+// scene. A ray record is two float4, (origin, tmax) and (direction, -). It is invalid -- a miss, never walked -- when
+// its origin or direction is not finite, its direction is zero or its tmax is not > 0 (NaN included).
+__device__ __forceinline__ bool finite_f(float x) { return (__float_as_uint(x) & 0x7f800000u) != 0x7f800000u; }
+__device__ __forceinline__ bool cast_ray(const CastArgs& c, uint32_t i, float3& o, float3& d, float& tmax) {
+    const float4 r0 = ld_stream(c.rays + 2 * size_t(i)), r1 = ld_stream(c.rays + 2 * size_t(i) + 1);
+    o = f3(r0.x, r0.y, r0.z);
+    d = f3(r1.x, r1.y, r1.z);
+    tmax = fminf(r0.w, FLT_MAX); // (an infinite bound is FLT_MAX, the bound of the render's camera rays)
+    const float m = fmaxf(fabsf(d.x), fmaxf(fabsf(d.y), fabsf(d.z)));
+    if (!(finite_f(o.x) && finite_f(o.y) && finite_f(o.z) && finite_f(d.x) && finite_f(d.y) && finite_f(d.z) && m > 0.0f &&
+          r0.w > 0.0f))
+        return false;
+    // sphere_hit assumes a unit direction; a power-of-two prescale keeps dot(d, d) clear of overflow and of flushed
+    // denormals (and is exact, so an ordinary direction normalises exactly as the render's do)
+    d = normalize(d * (m > 0x1p32f ? 0x1p-80f : (m < 0x1p-32f ? 0x1p80f : 1.0f)));
+    return true;
+}
+// Outputs of ray i: entity id (push order) and, where asked for, t along the unit direction and the normal
+// (hit_entity's rule); a miss is -1, +inf, (0, 0, 0).
+template <bool ALL>
+__device__ __forceinline__ void cast_store(const CastArgs& c, const SceneAccess<ALL>& S, uint32_t i, uint32_t prim, float3 o, float3 d,
+                                           float t) {
+    int32_t id = -1;
+    float3 ng = f3(0.f, 0.f, 0.f);
+    if (prim != kInvalid) id = hit_entity(S, prim, o + d * t, d, ng);
+    else t = __int_as_float(0x7f800000);
+    c.ids[i] = id;
+    if (c.t) c.t[i] = t;
+    if (c.normals) {
+        c.normals[3 * size_t(i)] = ng.x;
+        c.normals[3 * size_t(i) + 1] = ng.y;
+        c.normals[3 * size_t(i) + 2] = ng.z;
+    }
+}
+
+// Flat scenes: one ray per thread over the staged scene. An any-hit query takes the nearest-hit loop with the ray's own
+// bound: a hit below tmax exists exactly when the nearest one is below it, and the shadow half of trace_flat<true> runs
+// the same arithmetic per ray (its other half would test a switched-off ray for nothing).
+__global__ void __launch_bounds__(kThreads, 4) cast_flat_kernel(const PassArgs a, const CastArgs c) {
+    const SceneAccess<true> S = stage_scene<true>(a);
+    for (uint32_t i = blockIdx.x * kThreads + threadIdx.x; i < c.n; i += gridDim.x * kThreads) {
+        float3 o, d;
+        float tmax, t = 0.0f;
+        uint32_t prim = kInvalid;
+        bool occ;
+        if (cast_ray(c, i, o, d, tmax)) trace_flat<false>(S, o, d, tmax, d, -1.0f, t, prim, occ);
+        cast_store(c, S, i, prim, o, d, t);
+    }
+}
+
+// Tree scenes: trace_kernel's persistent scheme over the caller's rays -- the warp interleaves the walks of 32 rays in
+// rounds, a lane that finishes writes its ray's outputs, and once PassArgs::refill lanes are idle the warp pulls that many
+// new rays with one atomic on the cast's cursor. ANY = occlusion query: the walks stop at the first hit below tmax.
+template <bool COOP, int WALK, bool ANY, int OCC = 3>
+__global__ void __launch_bounds__(kThreads, OCC) cast_kernel(const PassArgs a, const CastArgs c) {
+    const SceneAccess<false> S = stage_scene<false>(a);
+    const uint32_t lane = threadIdx.x & 31u;
+    typename WalkOf<WALK>::type w = {};
+    unsigned cnt_node = 0, cnt_prim = 0;
+    bool have = false, more = true;
+    uint32_t ray = 0; // index of the lane's ray
+    while (true) {
+        bool finished = false;
+        const uint32_t idle = __ballot_sync(kFull, !have);
+        if (more && idle != 0u && (__popc(idle) >= a.refill || idle == kFull)) {
+            const uint32_t cnt = __popc(idle);
+            uint32_t base = 0;
+            if (lane == 0) base = atomicAdd(c.cursor, cnt);
+            base = __shfl_sync(kFull, base, 0);
+            if (base + cnt >= c.n) more = false; // all rays handed out (warp-uniform)
+            const uint32_t at = base + __popc(idle & ((1u << lane) - 1u));
+            if (!have && at < c.n) {
+                ray = at;
+                float3 o, d;
+                float tmax;
+                if (!cast_ray(c, at, o, d, tmax)) cast_store(c, S, at, kInvalid, o, d, 0.0f);
+                else if (w.init(S, o, d, tmax, ANY)) finished = true; // missed the root box / one-leaf scene / a big primitive
+                else have = true;
+            }
+        }
+        if (__ballot_sync(kFull, have || finished) == 0u) {
+            if (!more) break;
+            continue;
+        }
+        if (w.template step<false, COOP>(S, have)) { // all 32 lanes: one round
+            finished = true;
+            have = false;
+            if (WALK == 2 || WALK == 6) walk_counts(w, cnt_node, cnt_prim); // (rays that walked, as traverse() counts)
+        }
+        if (finished) cast_store(c, S, ray, w.best_prim, w.o, w.d, w.best);
+    }
+    if (WALK == 2 || WALK == 6) flush_walk_counts(a, cnt_node, cnt_prim);
 }
 
 // ---- accumulate / resolve ---------------------------------------------------------------
@@ -2662,6 +2767,27 @@ void launch_primary(const PassArgs& a, int32_t* ids_l, double* points_l, double*
     kernel<<<grid, kThreads, smem, s>>>(b, ids_l, points_l, normals_l);
     const cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) note_launch_error("primary kernel launch", e, smem, grid);
+}
+
+// The same walk, leaf mode and occupancy launch_trace picks for the render, in its any-hit or nearest-hit form.
+template <bool ANY> static void (*cast_tree_kernel(const PassArgs& a))(PassArgs, CastArgs) {
+    if (a.walk == 6) return cast_kernel<false, 6, ANY, 3>;
+    if (a.walk == 5) return a.trace_occ == 4 ? cast_kernel<false, 5, ANY, 4> : cast_kernel<false, 5, ANY, 3>;
+    if (a.walk == 3) return a.trace_occ == 4 ? cast_kernel<false, 3, ANY, 4> : cast_kernel<false, 3, ANY, 3>;
+    if (a.walk == 2) return a.coop_leaf ? cast_kernel<true, 2, ANY> : cast_kernel<false, 2, ANY>;
+    if (a.walk == 1) return a.coop_leaf ? (a.trace_occ == 4 ? cast_kernel<true, 1, ANY, 4> : cast_kernel<true, 1, ANY, 3>) : cast_kernel<false, 1, ANY>;
+    return a.coop_leaf ? cast_kernel<true, 0, ANY> : cast_kernel<false, 0, ANY>;
+}
+
+void launch_cast(const PassArgs& a, const CastArgs& c, bool any, int sm_count, cudaStream_t s) {
+    if (c.n == 0) return;
+    const size_t smem = path_smem_bytes(a);
+    void (*kernel)(PassArgs, CastArgs) = all_staged(a) ? cast_flat_kernel : (any ? cast_tree_kernel<true>(a) : cast_tree_kernel<false>(a));
+    int grid = persistent_grid(kernel, smem, sm_count);
+    grid = std::min<int64_t>(grid, (int64_t(c.n) + kThreads - 1) / kThreads);
+    kernel<<<grid, kThreads, smem, s>>>(a, c);
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) note_launch_error("cast kernel launch", e, smem, grid);
 }
 
 void launch_resolve(const TileMap& map, const float* accum, int spp, float* rad_l, uint8_t* rgb_l, cudaStream_t s) {

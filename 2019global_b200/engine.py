@@ -33,7 +33,7 @@ EXPORTS = [
     "g19_render_to_frame", "g19_frame_wait", "g19_frame_release", "g19_frame_timeouts",
     "g19_frame_read", "g19_render_progressive", "g19_render_tiles_device", "g19_untile_device", "g19_tile_pixels",
     "g19_probe_texcoord", "g19_probe_shade", "g19_probe_path_tree", "g19_entity_bbox", "g19_entity_triangles",
-    "g19_frame_status", "g19_tune", "g19_scene_set_shapes",
+    "g19_frame_status", "g19_tune", "g19_scene_set_shapes", "g19_cast_rays", "g19_cast_rays_device",
 ]
 
 
@@ -102,6 +102,9 @@ def lib():
         L.g19_frame_timeouts.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(C.c_uint)]
         L.g19_frame_status.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
         L.g19_tune.argtypes = [C.c_void_p, C.c_char_p, C.c_char_p]
+        L.g19_cast_rays.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p]
+        L.g19_cast_rays_device.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p,
+                                           C.c_void_p]
         _lib = L
     return _lib
 
@@ -303,6 +306,35 @@ class RayTracer:
         return self._check(self._L.g19_render_device(self.h, C.byref(self.camera), abi.d3(self.light), C.byref(p),
                                                      C.c_void_p(d_rgb), C.c_void_p(d_ids), C.c_void_p(d_rad),
                                                      C.c_void_p(stream)), allow=(abi.ERR_CANCELLED,))
+
+    def cast(self, origins, dirs, tmax=None, any_hit=False, want_normals=False, count=False):
+        """Batched ray queries against the PATH view of the scene (g19_cast_rays, blocking). origins, dirs: (n, 3);
+        tmax: scalar or (n,), None = unbounded. Returns {"ids": (n,) int32 entity ids (-1 = miss), "t": (n,) float32
+        distances along the unit direction (+inf = miss; None for any_hit), "normals": (n, 3) float32 or None}.
+        any_hit: occlusion query (ids = an entity hit below tmax, or -1)."""
+        o = np.asarray(origins, dtype=np.float32).reshape(-1, 3)
+        d = np.asarray(dirs, dtype=np.float32).reshape(-1, 3)
+        n = o.shape[0]
+        if d.shape[0] != n:
+            raise ValueError("origins and dirs must both be (n, 3)")
+        buf = np.zeros(n * 8 + 4, np.float32)  # the records must start on a 16-byte boundary
+        skip = (-buf.ctypes.data % 16) // 4
+        rays = buf[skip:skip + n * 8].reshape(n, 8)
+        rays[:, 0:3] = o
+        rays[:, 3] = np.inf if tmax is None else np.broadcast_to(np.asarray(tmax, dtype=np.float32), (n,))
+        rays[:, 4:7] = d
+        ids = np.empty(n, np.int32)
+        t = None if any_hit else np.empty(n, np.float32)
+        nrm = np.empty((n, 3), np.float32) if want_normals and not any_hit else None
+        flags = (abi.CAST_ANY_HIT if any_hit else 0) | (abi.CAST_COUNT if count else 0)
+        self._check(self._L.g19_cast_rays(self.h, n, _ptr(rays), flags, _ptr(ids), _ptr(t), _ptr(nrm)))
+        return {"ids": ids, "t": t, "normals": nrm}
+
+    def cast_device(self, n, d_rays, d_ids, d_t=0, d_normals=0, flags=0, stream=0):
+        """Asynchronous g19_cast_rays_device on device pointers (ints, e.g. torch.Tensor.data_ptr()): d_rays n x 8 float32,
+        16-byte aligned; d_ids n int32; d_t n float32 and d_normals n x 3 float32 optional (0)."""
+        return self._check(self._L.g19_cast_rays_device(self.h, int(n), C.c_void_p(d_rays), int(flags), C.c_void_p(d_ids),
+                                                        C.c_void_p(d_t), C.c_void_p(d_normals), C.c_void_p(stream)))
 
     def tune(self, key, value=None):
         """g19_tune: set one tuning knob ("lanes", "no_merge", ...); value None = back to the default."""

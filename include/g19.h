@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define G19_ABI_VERSION 5
+#define G19_ABI_VERSION 6
 
 /* ---- status codes ------------------------------------------------------- */
 enum {
@@ -250,6 +250,42 @@ int g19_render_device(g19_ctx* ctx, const g19_camera* camera, const double light
                       const g19_params* params, uint8_t* d_rgb888, int32_t* d_hit_id,
                       float* d_radiance, void* stream);
 int g19_get_stats(g19_ctx* ctx, g19_stats* out);
+
+/* Batched ray queries: what does each ray hit first, or is anything in its way (Embree's rtcIntersect /
+ * rtcOccluded, OptiX's closest-hit / any-hit). No counterpart in the reference: its Octree::intersect
+ * (octree.h:46-68) returns candidates, not hits.
+ *   scene       the PATH view of the last g19_upload_scene, with the shapes that upload used (G19_SHAPES_REF /
+ *               G19_SHAPES_FIXED); REF mode's octree and its "last candidate wins" rule are not involved
+ *   rays        n x 8 floats (ox, oy, oz, tmax, dx, dy, dz, 0), 16-byte aligned. The direction need not be unit
+ *               length: it is normalised, and t is the distance along the unit direction
+ *   invalid     a non-finite origin or direction, a zero direction, or tmax not > 0 (NaN included): a miss,
+ *               nothing traversed
+ *   hit         the nearest primitive with 0 <= t < tmax, by the render's own hit functions. A ray that starts on a
+ *               surface may hit it at t = 0: offset origins off surfaces (the engine offsets by 1e-3 along the normal)
+ *   outputs     out_entity n int32 (required): the entity id (push order; a merged parallelogram reports the
+ *               triangle the hit lies in, as hit_id_out of g19_render does); out_t n floats and out_normal n x 3
+ *               floats (both nullable): t and the normal -- the geometric normal turned against the ray for
+ *               triangles, (p - c) / r for spheres. A miss is entity -1, t = +inf, normal (0, 0, 0)
+ *   G19_CAST_ANY_HIT  occlusion query: out_entity = an entity hit with t < tmax (which one is unspecified), or -1;
+ *               out_t and out_normal must be NULL
+ *   G19_CAST_COUNT    tally node / primitive tests into g19_stats (tree scenes, with walks that count: 1 and 4)
+ *   structure   flat scenes: the packed pair loops over the staged scene; tree scenes: the walk g19_tune("walk")
+ *               selects, with the render's knobs (walk_steps, bvh_stack, coop_leaf, refill, trace_occ)
+ *   stats       g19_get_stats then reports the cast: extend_segments = n (nearest hit) or shadow_segments = n
+ *               (any hit), kernel_launches, render_ms (device time), node_tests / prim_tests with G19_CAST_COUNT
+ *   errors      G19_ERR_INVALID: ctx NULL, n < 0, rays or out_entity NULL with n > 0, rays not 16-byte aligned,
+ *               out_t / out_normal with G19_CAST_ANY_HIT, unknown flag bits; G19_ERR_NO_SCENE before any upload.
+ *               n == 0 returns G19_OK and launches nothing
+ * A cast touches no render buffer: a render's output does not depend on casts before it. One call per context at a
+ * time, as for renders.
+ * g19_cast_rays: HOST pointers, blocking; the rays are staged in a device buffer the context keeps (grown on demand).
+ * g19_cast_rays_device: DEVICE pointers, asynchronous on `stream` (a cudaStream_t, NULL = legacy default).     */
+#define G19_CAST_ANY_HIT 1u
+#define G19_CAST_COUNT 2u
+int g19_cast_rays(g19_ctx* ctx, int32_t n, const float* rays, uint32_t flags,
+                  int32_t* out_entity, float* out_t, float* out_normal);
+int g19_cast_rays_device(g19_ctx* ctx, int32_t n, const float* d_rays, uint32_t flags,
+                         int32_t* d_entity, float* d_t, float* d_normal, void* stream);
 
 /* Multi-GPU (SURVEY.md 8(e)): one process and one g19_ctx per GPU, image
  * tiles interleaved by params->rank/world. A rank's pixels form a compact

@@ -3,10 +3,14 @@
 // push_back forwards each entity's descriptor to a g19_scene, where the
 // reference's build (partition / push_obj, octree.h:75-129) is mirrored bug for
 // bug on the host (csrc/scene.cpp) and later flattened to HBM. intersect() is a
-// GPU probe returning the reference's candidate list. handle() is the one
-// addition the reference cannot offer (its Node/_root are private): the way for
-// RayTracer to reach the tree.
+// GPU probe returning the reference's candidate list. Two additions the
+// reference does not offer: handle() (its Node/_root are private), the way for
+// RayTracer to reach the tree, and nearest(), batched nearest-hit queries
+// (g19_cast_rays) for picking.
 #pragma once
+#include <algorithm>
+#include <cstddef>
+#include <limits>
 #include <memory>
 #include <vector>
 #include "bbox.h"
@@ -48,6 +52,31 @@ class Octree {
     }
 
     // additions
+    // What each ray hits first (nearest hit, g19_cast_rays over PATH mode's structures): the entity, or nullptr for a
+    // miss; t (nullable) receives the distance along the normalised direction (+inf for a miss). What a viewer needs
+    // for picking: the entity under the mouse.
+    std::vector<Entity*> nearest(const std::vector<Ray>& rays, std::vector<double>* t = nullptr) const {
+        std::lock_guard<std::mutex> lock(g19::detail::probe_mutex());
+        g19_ctx* ctx = g19::detail::probe_ctx();
+        g19::detail::upload_cached(_scene.get(), _serial, _version);
+        const size_t n = rays.size();
+        std::vector<float> rec(8 * n, 0.0f); // (origin, tmax | direction, 0) per ray
+        for (size_t i = 0; i < n; ++i) {
+            const Ray& r = rays[i];
+            const float v[8] = {float(r.origin.x), float(r.origin.y), float(r.origin.z), std::numeric_limits<float>::infinity(),
+                                float(r.dir.x), float(r.dir.y), float(r.dir.z), 0.0f};
+            std::copy(v, v + 8, rec.begin() + std::ptrdiff_t(8 * i));
+        }
+        std::vector<int32_t> ids(n);
+        std::vector<float> tf(t ? n : 0);
+        g19::detail::check(g19_cast_rays(ctx, int32_t(n), rec.data(), 0u, ids.data(), t ? tf.data() : nullptr, nullptr), ctx,
+                           "g19_cast_rays");
+        std::vector<Entity*> out(n, nullptr);
+        for (size_t i = 0; i < n; ++i)
+            if (ids[i] >= 0) out[i] = _entities[size_t(ids[i])];
+        if (t) t->assign(tf.begin(), tf.end());
+        return out;
+    }
     const g19_scene* handle() const { return _scene.get(); }
     unsigned version() const { return _version; }
     const std::vector<Entity*>& entities() const { return _entities; }
