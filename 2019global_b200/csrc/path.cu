@@ -174,7 +174,7 @@ static inline float cell_edge(float root_lo, float root_size, int level, uint32_
 
 void path_tuning_from_env(PathTuning& t) {
     static const char* const keys[] = {"lanes", "pass_slots", "no_merge", "leaf_max", "refill", "coop_leaf", "walk_steps",
-                                       "leaf_batch", "raygen_occ", "tree_build", "debug_tree", "walk", "trace_occ", "l2_persist", "bounce_occ", "top_level", "ref_heavy", "sort_rays", "upload_threads", "bvh_leaf", "bvh_spec", "bvh_stack", "fuse_first", "fold_last", "overlap_frames"};
+                                       "leaf_batch", "raygen_occ", "tree_build", "debug_tree", "walk", "trace_occ", "l2_persist", "bounce_occ", "top_level", "ref_heavy", "sort_rays", "upload_threads", "bvh_leaf", "bvh_spec", "bvh_stack", "fuse_first", "fold_last", "overlap_frames", "flat_uniform"};
     for (const char* k : keys) {
         std::string env = "G19_";
         for (const char* c = k; *c; ++c) env += char(std::toupper(*c));
@@ -204,6 +204,7 @@ bool path_tuning_set(PathTuning& t, const char* key, const char* value) {
     else if (k == "overlap_frames") t.overlap_frames = num(def.overlap_frames, 0, 1);
     else if (k == "fold_last") t.fold_last = num(def.fold_last, 0, 1);
     else if (k == "fuse_first") t.fuse_first = num(def.fuse_first, 0, 1);
+    else if (k == "flat_uniform") t.flat_uniform = num(def.flat_uniform, 0, 1);
     else if (k == "bvh_stack") t.bvh_stack = num(def.bvh_stack, 4, 64);
     else if (k == "bvh_spec") t.bvh_spec = num(def.bvh_spec, 0, 3);
     else if (k == "bvh_leaf") t.bvh_leaf = num(def.bvh_leaf, 1, 8);
@@ -618,6 +619,21 @@ int path_upload(PathSceneBuffers& b, const g19_scene& scene, const PathTuning& t
     // count with NaNs: every comparison on a NaN fails, so a padding record is never hit.
     std::vector<float> pairs;
     if (!on_device && nodes.size() == 1) build_pairs(hot, 0, size_t(n_par), size_t(n_tri), hot.size() - size_t(n_par) - size_t(n_tri), pairs);
+    {
+        const size_t p_par = (size_t(n_par) + 1) / 2, p_tri = (size_t(n_tri) + 1) / 2;
+        const size_t p_sph = (hot.size() - size_t(n_par) - size_t(n_tri) + 1) / 2;
+        b.upairs = FlatPairsU{};
+        b.upairs_fit = !pairs.empty() && p_par <= size_t(kUniPlanarPairs) && p_tri <= size_t(kUniPlanarPairs) &&
+                       p_sph <= size_t(kUniSpherePairs);
+        if (b.upairs_fit) {
+            const float* src = pairs.data();
+            std::memcpy(b.upairs.par, src, p_par * sizeof b.upairs.par[0]);
+            src += p_par * 24;
+            std::memcpy(b.upairs.tri, src, p_tri * sizeof b.upairs.tri[0]);
+            src += p_tri * 24;
+            std::memcpy(b.upairs.sph, src, p_sph * sizeof b.upairs.sph[0]);
+        }
+    }
     auto up = [&](DeviceArray& d, const void* src, size_t bytes) -> cudaError_t {
         cudaError_t e = d.ensure(bytes ? bytes : 16);
         if (e != cudaSuccess || !bytes) return e;
@@ -854,6 +870,8 @@ PassArgs path_pass_setup(const PathSceneBuffers& b, const PathTuning& tune, bool
     pa.bounce_occ = tune.bounce_occ;
     pa.bvh_spec = tune.bvh_spec;
     pa.fold_last = 0;
+    pa.flat_uniform = tune.flat_uniform && b.upairs_fit ? 1 : 0;
+    pa.upairs = &b.upairs;
     pa.walk = tune.walk ? (count ? 2 : 1) : 0; // the new walk counts its node / primitive tests when asked (params.profile)
     if (tune.walk >= 3 && b.view.bvh_root != 0xffffffffu && b.view.bvh_nodes) {
         pa.walk = tune.walk == 4 ? (count ? 6 : 5) : 3; // bounding-volume hierarchy, binary / 4-wide (the latter counts its tests when asked)

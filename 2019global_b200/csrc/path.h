@@ -63,6 +63,19 @@ struct PathSceneD {
     uint32_t bvh_root;       // node index, leaf reference, or 0xffffffff (nothing in the hierarchy)
 };
 
+// A flat scene's primitive pairs (PathSceneD::pairs, same record layout), passed to the flat bounce kernels as a launch
+// parameter of their own when every kind group fits: their pair loops are then unrolled to these capacities and read the
+// coefficients as constant-bank (uniform) operands instead of per-thread registers loaded from shared memory. Not a
+// __constant__ symbol: several contexts and lanes render concurrently. 1664 B of the 32 KB parameter space; not in
+// PassArgs, which every other kernel gets too.
+constexpr int kUniPlanarPairs = 8; // per planar kind (parallelograms, triangles)
+constexpr int kUniSpherePairs = 4;
+struct FlatPairsU {
+    ulonglong2 par[kUniPlanarPairs][6]; // rows a, b, c of two parallelograms, every coefficient a float2
+    ulonglong2 tri[kUniPlanarPairs][6];
+    ulonglong2 sph[kUniSpherePairs][2]; // (-centre, radius^2) of two spheres
+};
+
 struct PathCamera { // float copies of the reference basis (RefCamera)
     float pos[3], top_left[3], left[3], up[3];
 };
@@ -89,6 +102,8 @@ struct PathSceneBuffers {
     DeviceArray nodes, prim_index, hot, cold, materials, lights, pairs, prim_entity, top;
     DeviceArray bvh_nodes, bvh4_nodes, bvh_prims, bvh_big, bvh_big_pairs;
     PathSceneD view{};
+    FlatPairsU upairs{};       // view.pairs again, for the flat bounce kernels' FlatPairsU parameter
+    bool upairs_fit = false;   // the scene is flat and its kind groups fit FlatPairsU
     bool has_bsdf[4] = {false, false, false, false};
     unsigned long long upload_serial = 0; // counts path_upload calls: a new number = a different scene
 };
@@ -167,6 +182,7 @@ struct PathTuning {
     int overlap_frames = 1;   // frames rendered back to back: the side lanes start the next frame's passes behind their own, not behind the join
     int fold_last = 1;        // flat scenes: a path's last vertex (next-event estimation only) is shaded by the launch that finds it
     int fuse_first = 1;       // flat scenes: trace the camera segment inside the first bounce's launch (no raygen kernel; camera records only for hits on mirror / glass)
+    int flat_uniform = 1;     // flat scenes whose pairs fit FlatPairsU: the bounce kernels' pair loops read them from the launch parameters
     int bvh_stack = kBvhSmemStack; // walk=3/4: levels of the postponed-children stack in shared memory (1 KB per level and CTA)
     int bvh_spec = 1;         // walk=3: a lane that reaches a leaf postpones it and keeps descending
     int bvh_leaf = 4;         // walk=3: primitives per BVH leaf at most (1..8; read at scene upload)
@@ -288,6 +304,8 @@ struct PassArgs {
     int32_t bvh_spec;      // BvhWalk: speculative traversal (PathTuning::bvh_spec)
     int32_t fold_last;     // this launch shades the path's last vertex in place (flat scenes, bounce max_depth - 2)
     int32_t walk;          // tree walk variant (PathTuning::walk); +2 when the walk counts its node / primitive tests
+    int32_t flat_uniform;  // the flat bounce kernels trace through their FlatPairsU parameter (unrolled pair loops)
+    const FlatPairsU* upairs; // host memory (PathSceneBuffers::upairs): what the launchers pass as that parameter
 };
 
 // path.cu: the PassArgs fields that follow from the scene and the tuning alone (staging sizes, walk and its knobs);

@@ -130,6 +130,7 @@ template <bool ALL> struct SceneAccess {
     const float4* cold_s;
     const float4* lights_s;
     const ulonglong2* pairs_s; // flat scenes: primitive PAIRS, one float2 per coefficient (trace_flat)
+    const FlatPairsU* upairs;  // the same pairs in the flat bounce kernels' launch parameters (trace_flat<UNI>; set by those kernels)
     uint32_t* stack;
     int n_nodes_s;
     int walk_steps;      // tree walk: cell moves per round
@@ -361,23 +362,38 @@ template <int KIND> __device__ __forceinline__ bool plane_inside(float u, float 
 // padded to an even count with a NaN record that can never be hit); the position in its group IS
 // the primitive id.
 template <int KIND, bool DUAL>
+__device__ __forceinline__ void plane_pair(const ulonglong2* rec, uint32_t id, float3 o, const RayDir& d1, const RayDir& d0,
+                                           uint32_t& lim1, uint32_t& lim0, uint32_t& hit_k) {
+    const PlaneOrigin2 po = plane_origin2(rec, o);
+    f2 u, v, t;
+    plane_uvt2(rec, po, d1, u, v, t);
+    float ua, ub, va, vb, ta, tb;
+    upk(u, ua, ub); upk(v, va, vb); upk(t, ta, tb);
+    if (plane_inside<KIND>(ua, va) & (__float_as_uint(ta) < lim1)) { lim1 = __float_as_uint(ta); hit_k = id; }
+    if (plane_inside<KIND>(ub, vb) & (__float_as_uint(tb) < lim1)) { lim1 = __float_as_uint(tb); hit_k = id + 1u; }
+    if (DUAL) {
+        plane_uvt2(rec, po, d0, u, v, t);
+        upk(u, ua, ub); upk(v, va, vb); upk(t, ta, tb);
+        if ((plane_inside<KIND>(ua, va) & (__float_as_uint(ta) < lim0)) | (plane_inside<KIND>(ub, vb) & (__float_as_uint(tb) < lim0)))
+            lim0 = 0u;
+    }
+}
+template <int KIND, bool DUAL>
 __device__ __forceinline__ void plane_pairs(const ulonglong2* rec, uint32_t n_pairs, uint32_t id0, float3 o, const RayDir& d1,
                                             const RayDir& d0, uint32_t& lim1, uint32_t& lim0, uint32_t& hit_k) {
 #pragma unroll 1
-    for (uint32_t j = 0; j < n_pairs; ++j, rec += 6) {
-        const PlaneOrigin2 po = plane_origin2(rec, o);
-        f2 u, v, t;
-        plane_uvt2(rec, po, d1, u, v, t);
-        float ua, ub, va, vb, ta, tb;
-        upk(u, ua, ub); upk(v, va, vb); upk(t, ta, tb);
-        if (plane_inside<KIND>(ua, va) & (__float_as_uint(ta) < lim1)) { lim1 = __float_as_uint(ta); hit_k = id0 + 2u * j; }
-        if (plane_inside<KIND>(ub, vb) & (__float_as_uint(tb) < lim1)) { lim1 = __float_as_uint(tb); hit_k = id0 + 2u * j + 1u; }
-        if (DUAL) {
-            plane_uvt2(rec, po, d0, u, v, t);
-            upk(u, ua, ub); upk(v, va, vb); upk(t, ta, tb);
-            if ((plane_inside<KIND>(ua, va) & (__float_as_uint(ta) < lim0)) | (plane_inside<KIND>(ub, vb) & (__float_as_uint(tb) < lim0)))
-                lim0 = 0u;
-        }
+    for (uint32_t j = 0; j < n_pairs; ++j, rec += 6) plane_pair<KIND, DUAL>(rec, id0 + 2u * j, o, d1, d0, lim1, lim0, hit_k);
+}
+// The pairs of the launch parameters (FlatPairsU): the loop is unrolled to the capacity and left at the group's count (warp-uniform), so
+// every coefficient sits at a fixed constant-bank offset and is read as a uniform operand of the FFMA2s -- no per-thread
+// registers and no shared-memory loads for the 24 coefficients of a pair, no loop counter or record pointer.
+template <int KIND, bool DUAL>
+__device__ __forceinline__ void plane_pairs_u(const ulonglong2 (&rec)[kUniPlanarPairs][6], uint32_t n_pairs, uint32_t id0, float3 o,
+                                              const RayDir& d1, const RayDir& d0, uint32_t& lim1, uint32_t& lim0, uint32_t& hit_k) {
+#pragma unroll
+    for (uint32_t j = 0; j < uint32_t(kUniPlanarPairs); ++j) {
+        if (j >= n_pairs) break;
+        plane_pair<KIND, DUAL>(rec[j], id0 + 2u * j, o, d1, d0, lim1, lim0, hit_k);
     }
 }
 // Sphere pair record = 2 x ulonglong2: (-cx, -cy | -cz, r^2). Unit direction, discriminant from the
@@ -394,6 +410,22 @@ __device__ __forceinline__ void sphere_roots2(f2 ocx, f2 ocy, f2 ocz, f2 rr, con
     tb = min(__float_as_uint(-b1 - s1), __float_as_uint(s1 - b1));
 }
 template <bool DUAL>
+__device__ __forceinline__ void sphere_pair(const ulonglong2* rec, uint32_t id, float3 o, const RayDir& r1, const RayDir& r0,
+                                            uint32_t& lim1, uint32_t& lim0, uint32_t& hit_k) {
+    const ulonglong2 c0 = rec[0], c1 = rec[1];
+    const f2 ocx = add2(c0.x, bc(o.x)), ocy = add2(c0.y, bc(o.y)), ocz = add2(c1.x, bc(o.z));
+    uint32_t ta, tb;
+    sphere_roots2(ocx, ocy, ocz, c1.y, r1, ta, tb);
+    if (ta < lim1) { lim1 = ta; hit_k = id; }
+    if (tb < lim1) { lim1 = tb; hit_k = id + 1u; }
+    if (DUAL) {
+        sphere_roots2(ocx, ocy, ocz, c1.y, r0, ta, tb);
+        if ((ta < lim0) | (tb < lim0)) lim0 = 0u;
+    }
+}
+// UNI: the pairs come from the launch parameters (S.upairs; the scene fits FlatPairsU: PassArgs::flat_uniform) instead of
+// shared memory.
+template <bool DUAL, bool UNI = false>
 __device__ __forceinline__ void trace_flat(const SceneAccess<true>& S, float3 o, float3 d1, float tmax1, float3 d0,
                                            float tmax0, float& best, uint32_t& best_k, bool& occluded) {
     uint32_t lim1 = range_limit(tmax1), lim0 = DUAL ? range_limit(tmax0) : 0u;
@@ -401,24 +433,23 @@ __device__ __forceinline__ void trace_flat(const SceneAccess<true>& S, float3 o,
     const uint32_t n_par = uint32_t(S.g->n_par), n_tri = uint32_t(S.g->n_tri), n = uint32_t(S.g->n_prims);
     const uint32_t p_par = (n_par + 1u) >> 1, p_tri = (n_tri + 1u) >> 1, p_sph = (n - n_par - n_tri + 1u) >> 1;
     const RayDir r1 = ray_dir(d1), r0 = ray_dir(d0);
-    const ulonglong2* rec = S.pairs_s;
-    plane_pairs<2, DUAL>(rec, p_par, 0u, o, r1, r0, lim1, lim0, hit_k);
-    rec += 6u * p_par;
-    plane_pairs<1, DUAL>(rec, p_tri, n_par, o, r1, r0, lim1, lim0, hit_k);
-    rec += 6u * p_tri;
-#pragma unroll 1
-    for (uint32_t j = 0; j < p_sph; ++j, rec += 2) {
-        const ulonglong2 c0 = rec[0], c1 = rec[1];
-        const f2 ocx = add2(c0.x, bc(o.x)), ocy = add2(c0.y, bc(o.y)), ocz = add2(c1.x, bc(o.z));
-        uint32_t ta, tb;
-        sphere_roots2(ocx, ocy, ocz, c1.y, r1, ta, tb);
-        const uint32_t id = n_par + n_tri + 2u * j;
-        if (ta < lim1) { lim1 = ta; hit_k = id; }
-        if (tb < lim1) { lim1 = tb; hit_k = id + 1u; }
-        if (DUAL) {
-            sphere_roots2(ocx, ocy, ocz, c1.y, r0, ta, tb);
-            if ((ta < lim0) | (tb < lim0)) lim0 = 0u;
+    if (UNI) {
+        const FlatPairsU& P = *S.upairs;
+        plane_pairs_u<2, DUAL>(P.par, p_par, 0u, o, r1, r0, lim1, lim0, hit_k);
+        plane_pairs_u<1, DUAL>(P.tri, p_tri, n_par, o, r1, r0, lim1, lim0, hit_k);
+#pragma unroll
+        for (uint32_t j = 0; j < uint32_t(kUniSpherePairs); ++j) {
+            if (j >= p_sph) break;
+            sphere_pair<DUAL>(P.sph[j], n_par + n_tri + 2u * j, o, r1, r0, lim1, lim0, hit_k);
         }
+    } else {
+        const ulonglong2* rec = S.pairs_s;
+        plane_pairs<2, DUAL>(rec, p_par, 0u, o, r1, r0, lim1, lim0, hit_k);
+        rec += 6u * p_par;
+        plane_pairs<1, DUAL>(rec, p_tri, n_par, o, r1, r0, lim1, lim0, hit_k);
+        rec += 6u * p_tri;
+#pragma unroll 1
+        for (uint32_t j = 0; j < p_sph; ++j, rec += 2) sphere_pair<DUAL>(rec, n_par + n_tri + 2u * j, o, r1, r0, lim1, lim0, hit_k);
     }
     best = __uint_as_float(lim1);
     best_k = hit_k;
@@ -1786,7 +1817,7 @@ __device__ __forceinline__ void prefetch_rec(const RecView& r, uint32_t pos, boo
 // FOLD (flat scenes, the bounce before the last): the vertex the continuation ray finds would be the path's
 // last one -- next-event estimation only. It is shaded right here (light sample + shadow ray) instead of being written as a
 // 64-byte record for a launch of its own to read back: same arithmetic in the same order, one launch per pass fewer.
-template <int KIND, bool FIRST, bool LAST, bool SPEC, bool SPLIT = false, bool FUSED = false, bool FOLD = false>
+template <int KIND, bool FIRST, bool LAST, bool SPEC, bool SPLIT = false, bool FUSED = false, bool FOLD = false, bool UNI = false>
 __device__ __forceinline__ void bounce_flat_body(const PassArgs& a, const int bounce, const SceneAccess<true>& S, const uint32_t n,
                                                  const uint32_t cta, const uint32_t n_cta, RecStage<!FIRST>& stage) {
     constexpr bool kDiffuse = KIND == Q_DIFFUSE;
@@ -1825,7 +1856,9 @@ __device__ __forceinline__ void bounce_flat_body(const PassArgs& a, const int bo
             uint32_t pr = kInvalid;
             int spec_kind = -1; // SPEC: the camera ray met a mirror / glass surface: that vertex goes to its material's queue
             float4 seen = make_float4(0.f, 0.f, 0.f, 0.f); // what a path that ends on the camera segment delivers
-            if (nearest<true>(S, live, o, d, t, pr)) {
+            bool unused_occ;
+            trace_flat<false, UNI>(S, o, d, live ? FLT_MAX : -1.0f, d, -1.0f, t, pr, unused_occ); // = nearest<true>
+            if (pr != kInvalid) {
                 const float4 tag = S.hot_row(pr, 3);
                 const int bsdf = __float_as_int(tag.y);
                 if (bsdf == G19_BSDF_EMITTER) { // directly visible light: the path ends here
@@ -1904,25 +1937,25 @@ __device__ __forceinline__ void bounce_flat_body(const PassArgs& a, const int bo
                     bool unused;
                     float ts;
                     uint32_t ps;
-                    trace_flat<false>(S, sh.no, sh.w, sh.tmax_s, sh.w, -1.0f, ts, ps, unused);
+                    trace_flat<false, UNI>(S, sh.no, sh.w, sh.tmax_s, sh.w, -1.0f, ts, ps, unused);
                     blocked = ps != kInvalid;
                 }
                 if (cont) {
                     bool unused;
-                    trace_flat<false>(S, sh.no, sh.nd, FLT_MAX, sh.nd, -1.0f, t_hit, prim_hit, unused);
+                    trace_flat<false, UNI>(S, sh.no, sh.nd, FLT_MAX, sh.nd, -1.0f, t_hit, prim_hit, unused);
                 }
             } else if (kDiffuse && !LAST) {
                 if (sh.want_shadow || cont)
-                    trace_flat<true>(S, sh.no, sh.nd, cont ? FLT_MAX : -1.0f, sh.w, sh.tmax_s, t_hit, prim_hit, blocked);
+                    trace_flat<true, UNI>(S, sh.no, sh.nd, cont ? FLT_MAX : -1.0f, sh.w, sh.tmax_s, t_hit, prim_hit, blocked);
             } else if (kDiffuse) { // LAST: the shadow ray alone
                 if (sh.want_shadow) {
                     bool unused;
-                    trace_flat<false>(S, sh.no, sh.w, sh.tmax_s, sh.w, -1.0f, t_hit, prim_hit, unused);
+                    trace_flat<false, UNI>(S, sh.no, sh.w, sh.tmax_s, sh.w, -1.0f, t_hit, prim_hit, unused);
                     blocked = prim_hit != kInvalid;
                 }
             } else if (cont) {
                 bool unused;
-                trace_flat<false>(S, sh.no, sh.nd, FLT_MAX, sh.nd, -1.0f, t_hit, prim_hit, unused);
+                trace_flat<false, UNI>(S, sh.no, sh.nd, FLT_MAX, sh.nd, -1.0f, t_hit, prim_hit, unused);
             }
             const bool hit = cont && prim_hit != kInvalid;
             const bool lit = kDiffuse && sh.want_shadow && !blocked;
@@ -1952,7 +1985,7 @@ __device__ __forceinline__ void bounce_flat_body(const PassArgs& a, const int bo
                     bool unused;
                     float t2;
                     uint32_t k2;
-                    trace_flat<false>(S, s2.no, s2.w, s2.tmax_s, s2.w, -1.0f, t2, k2, unused);
+                    trace_flat<false, UNI>(S, s2.no, s2.w, s2.tmax_s, s2.w, -1.0f, t2, k2, unused);
                     const bool lit2 = k2 == kInvalid;
                     cnt_b += 1u + (lit2 ? 0x10000u : 0u);
                     if (lit2) Lp = Lp + s2.lit_rgb;
@@ -2001,28 +2034,32 @@ __device__ __forceinline__ void bounce_flat_body(const PassArgs& a, const int bo
 }
 
 // One material queue per launch (diffuse-only scenes, and the last bounce of any scene).
-template <int KIND, bool FIRST, bool LAST, bool SPEC, int OCC = 3, bool FOLD = false>
-__global__ void __launch_bounds__(kThreads, KIND != Q_DIFFUSE ? 4 : OCC) bounce_flat_kernel(const PassArgs a, const int bounce) {
+template <int KIND, bool FIRST, bool LAST, bool SPEC, int OCC = 3, bool FOLD = false, bool UNI = false>
+__global__ void __launch_bounds__(kThreads, KIND != Q_DIFFUSE ? 4 : OCC)
+    bounce_flat_kernel(const PassArgs a, const int bounce, const __grid_constant__ FlatPairsU up) {
     pdl_launch_dependents();
     if (LAST && KIND != Q_DIFFUSE) return; // a specular vertex on the last segment contributes nothing
-    const SceneAccess<true> S = stage_scene<true>(a); // does not depend on earlier kernels: overlaps their tail
+    SceneAccess<true> S = stage_scene<true>(a); // does not depend on earlier kernels: overlaps their tail
+    S.upairs = &up;
     pdl_wait();
     const uint32_t n = a.counts[bounce * 4 + KIND];
     if (blockIdx.x * kThreads >= n) return; // short queue: surplus CTAs leave
     __shared__ RecStage<!FIRST> stage;
-    bounce_flat_body<KIND, FIRST, LAST, SPEC, OCC == 4, false, FOLD>(a, bounce, S, n, blockIdx.x, gridDim.x, stage);
+    bounce_flat_body<KIND, FIRST, LAST, SPEC, OCC == 4, false, FOLD, UNI>(a, bounce, S, n, blockIdx.x, gridDim.x, stage);
 }
 
 // Diffuse-only flat scenes: camera segment + first vertex in one launch (bounce_flat_body<FUSED>), over the path slots of
 // the pass instead of a queue.
-template <bool LAST, bool FOLD = false, bool SPEC = false> __global__ void __launch_bounds__(kThreads, 3) bounce_flat_fused_kernel(const PassArgs a) {
+template <bool LAST, bool FOLD = false, bool SPEC = false, bool UNI = false>
+__global__ void __launch_bounds__(kThreads, 3) bounce_flat_fused_kernel(const PassArgs a, const __grid_constant__ FlatPairsU up) {
     pdl_launch_dependents();
     const uint32_t n = a.n_slots;
     if (blockIdx.x * kThreads >= n) return;
-    const SceneAccess<true> S = stage_scene<true>(a);
+    SceneAccess<true> S = stage_scene<true>(a);
+    S.upairs = &up;
     pdl_wait(); // the previous pass's accumulate cleared the queue lengths
     RecStage<false>& unused = *reinterpret_cast<RecStage<false>*>(g19_dyn_smem); // (the fused body prefetches no records)
-    bounce_flat_body<Q_DIFFUSE, true, LAST, SPEC, false, true, FOLD>(a, 0, S, n, blockIdx.x, gridDim.x, unused);
+    bounce_flat_body<Q_DIFFUSE, true, LAST, SPEC, false, true, FOLD, UNI>(a, 0, S, n, blockIdx.x, gridDim.x, unused);
 }
 
 // All three material queues of one bounce in ONE launch (scenes with mirror / glass). The mirror and
@@ -2032,10 +2069,11 @@ template <bool LAST, bool FOLD = false, bool SPEC = false> __global__ void __lau
 // Here the grid's CTAs are split between the queues in proportion to their estimated work, so the
 // specular vertices fill issue slots beside the diffuse ones and a pass is 13 launches, not 34.
 // The per-material queues and kernels' code are unchanged: a CTA runs exactly one KIND.
-template <bool FIRST, bool FOLD = false>
-__global__ void __launch_bounds__(kThreads, 3) bounce_flat_all_kernel(const PassArgs a, const int bounce) {
+template <bool FIRST, bool FOLD = false, bool UNI = false>
+__global__ void __launch_bounds__(kThreads, 3) bounce_flat_all_kernel(const PassArgs a, const int bounce, const __grid_constant__ FlatPairsU up) {
     pdl_launch_dependents();
-    const SceneAccess<true> S = stage_scene<true>(a);
+    SceneAccess<true> S = stage_scene<true>(a);
+    S.upairs = &up;
     pdl_wait();
     const uint32_t n1 = a.counts[bounce * 4 + Q_DIFFUSE], n2 = a.counts[bounce * 4 + Q_MIRROR], n3 = a.counts[bounce * 4 + Q_GLASS];
     // estimated work per queue entry relative to a diffuse vertex (two rays, light sample): measured
@@ -2050,9 +2088,9 @@ __global__ void __launch_bounds__(kThreads, 3) bounce_flat_all_kernel(const Pass
     const uint32_t g1 = n1 ? min(G - g2 - g3, (n1 + kThreads - 1) / kThreads) : 0u;
     __shared__ RecStage<!FIRST> stage;
     const uint32_t b = blockIdx.x;
-    if (b < g1) bounce_flat_body<Q_DIFFUSE, FIRST, false, true, false, false, FOLD>(a, bounce, S, n1, b, g1, stage);
-    else if (b < g1 + g2) bounce_flat_body<Q_MIRROR, FIRST, false, true, false, false, FOLD>(a, bounce, S, n2, b - g1, g2, stage);
-    else if (b < g1 + g2 + g3) bounce_flat_body<Q_GLASS, FIRST, false, true, false, false, FOLD>(a, bounce, S, n3, b - g1 - g2, g3, stage);
+    if (b < g1) bounce_flat_body<Q_DIFFUSE, FIRST, false, true, false, false, FOLD, UNI>(a, bounce, S, n1, b, g1, stage);
+    else if (b < g1 + g2) bounce_flat_body<Q_MIRROR, FIRST, false, true, false, false, FOLD, UNI>(a, bounce, S, n2, b - g1, g2, stage);
+    else if (b < g1 + g2 + g3) bounce_flat_body<Q_GLASS, FIRST, false, true, false, false, FOLD, UNI>(a, bounce, S, n3, b - g1 - g2, g3, stage);
 }
 
 // ---- bounce, tree scenes: shade and queue the rays -----------------------------------------
@@ -2623,23 +2661,41 @@ static cudaError_t launch_pdl(void (*kernel)(KArgs...), int grid, size_t smem, c
     return cudaLaunchKernelEx(&cfg, kernel, args...);
 }
 
+// The flat bounce kernel of these template arguments, in its FlatPairsU form when the pass uses that (not for the
+// bounce_occ = 4 experiment).
+template <int KIND, bool FIRST, bool LAST, bool SPEC, int OCC = 3, bool FOLD = false>
+static void (*flat_bounce_kernel(const PassArgs& a))(PassArgs, int, FlatPairsU) {
+    if constexpr (OCC == 3)
+        if (a.flat_uniform) return bounce_flat_kernel<KIND, FIRST, LAST, SPEC, OCC, FOLD, true>;
+    return bounce_flat_kernel<KIND, FIRST, LAST, SPEC, OCC, FOLD, false>;
+}
+
+// What the flat bounce kernels get as their FlatPairsU parameter.
+static const FlatPairsU& launch_pairs(const PassArgs& a) {
+    static const FlatPairsU none{};
+    return a.flat_uniform ? *a.upairs : none;
+}
+
 template <int KIND, bool FIRST, bool LAST, bool ALL>
 static void launch_bounce_k(const PassArgs& a, int bounce, size_t smem, int sm_count, cudaStream_t s) {
-    void (*kernel)(PassArgs, int);
     if constexpr (ALL) {
+        void (*kernel)(PassArgs, int, FlatPairsU);
         if constexpr (KIND == Q_DIFFUSE) {
-            if (a.bounce_occ == 4) kernel = (a.kind_mask & 6u) ? bounce_flat_kernel<KIND, FIRST, LAST, true, 4> : bounce_flat_kernel<KIND, FIRST, LAST, false, 4>;
-            else if (!LAST && a.fold_last) kernel = (a.kind_mask & 6u) ? bounce_flat_kernel<KIND, FIRST, LAST, true, 3, true> : bounce_flat_kernel<KIND, FIRST, LAST, false, 3, true>;
-            else kernel = (a.kind_mask & 6u) ? bounce_flat_kernel<KIND, FIRST, LAST, true> : bounce_flat_kernel<KIND, FIRST, LAST, false>;
+            if (a.bounce_occ == 4) kernel = (a.kind_mask & 6u) ? flat_bounce_kernel<KIND, FIRST, LAST, true, 4>(a) : flat_bounce_kernel<KIND, FIRST, LAST, false, 4>(a);
+            else if (!LAST && a.fold_last) kernel = (a.kind_mask & 6u) ? flat_bounce_kernel<KIND, FIRST, LAST, true, 3, true>(a) : flat_bounce_kernel<KIND, FIRST, LAST, false, 3, true>(a);
+            else kernel = (a.kind_mask & 6u) ? flat_bounce_kernel<KIND, FIRST, LAST, true>(a) : flat_bounce_kernel<KIND, FIRST, LAST, false>(a);
         }
-        else if (!LAST && a.fold_last) kernel = bounce_flat_kernel<KIND, FIRST, LAST, true, 3, true>;
-        else kernel = bounce_flat_kernel<KIND, FIRST, LAST, true>;
+        else if (!LAST && a.fold_last) kernel = flat_bounce_kernel<KIND, FIRST, LAST, true, 3, true>(a);
+        else kernel = flat_bounce_kernel<KIND, FIRST, LAST, true>(a);
+        const int grid = persistent_grid(kernel, smem, sm_count);
+        cudaError_t e = launch_pdl(kernel, grid, smem, s, a, bounce, launch_pairs(a));
+        if (e != cudaSuccess) note_launch_error("bounce kernel launch", e, smem, grid);
     } else {
-        kernel = bounce_kernel<KIND, FIRST, LAST>;
+        void (*kernel)(PassArgs, int) = bounce_kernel<KIND, FIRST, LAST>;
+        const int grid = persistent_grid(kernel, smem, sm_count);
+        cudaError_t e = launch_pdl(kernel, grid, smem, s, a, bounce);
+        if (e != cudaSuccess) note_launch_error("bounce kernel launch", e, smem, grid);
     }
-    const int grid = persistent_grid(kernel, smem, sm_count);
-    cudaError_t e = launch_pdl(kernel, grid, smem, s, a, bounce);
-    if (e != cudaSuccess) note_launch_error("bounce kernel launch", e, smem, grid);
 }
 
 template <int KIND, bool ALL> static void launch_bounce_fl(const PassArgs& a, int bounce, size_t smem, int sm_count, cudaStream_t s) {
@@ -2698,14 +2754,18 @@ bool path_scene_is_flat(const PassArgs& a) { return all_staged(a); }
 bool launch_bounce_first_fused(const PassArgs& a, int sm_count, cudaStream_t s) {
     if (!all_staged(a) || a.bounce_occ == 4) return false;
     const size_t smem = path_smem_bytes(a);
-    void (*kernel)(PassArgs);
+    void (*kernel)(PassArgs, FlatPairsU);
+    const bool u = a.flat_uniform != 0;
     if (a.kind_mask & 6u) // mirror / glass in the scene: diffuse camera hits shaded in place, specular ones queued
-        kernel = a.max_depth <= 1 ? bounce_flat_fused_kernel<true, false, true>
-                                  : (a.fold_last ? bounce_flat_fused_kernel<false, true, true> : bounce_flat_fused_kernel<false, false, true>);
+        kernel = a.max_depth <= 1 ? (u ? bounce_flat_fused_kernel<true, false, true, true> : bounce_flat_fused_kernel<true, false, true>)
+                 : a.fold_last    ? (u ? bounce_flat_fused_kernel<false, true, true, true> : bounce_flat_fused_kernel<false, true, true>)
+                                  : (u ? bounce_flat_fused_kernel<false, false, true, true> : bounce_flat_fused_kernel<false, false, true>);
     else
-        kernel = a.max_depth <= 1 ? bounce_flat_fused_kernel<true> : (a.fold_last ? bounce_flat_fused_kernel<false, true> : bounce_flat_fused_kernel<false>);
+        kernel = a.max_depth <= 1 ? (u ? bounce_flat_fused_kernel<true, false, false, true> : bounce_flat_fused_kernel<true>)
+                 : a.fold_last    ? (u ? bounce_flat_fused_kernel<false, true, false, true> : bounce_flat_fused_kernel<false, true>)
+                                  : (u ? bounce_flat_fused_kernel<false, false, false, true> : bounce_flat_fused_kernel<false>);
     const int grid = persistent_grid(kernel, smem, sm_count);
-    cudaError_t e = launch_pdl(kernel, grid, smem, s, a);
+    cudaError_t e = launch_pdl(kernel, grid, smem, s, a, launch_pairs(a));
     if (e != cudaSuccess) note_launch_error("fused first bounce kernel launch", e, smem, grid);
     return true;
 }
@@ -2715,10 +2775,15 @@ bool launch_bounce_merged(const PassArgs& a, int bounce, int sm_count, cudaStrea
     const bool first = bounce == 0, last = bounce + 1 >= a.max_depth;
     if (!all_staged(a) || last || !(a.kind_mask & 6u)) return false;
     const size_t smem = path_smem_bytes(a);
-    void (*kernel)(PassArgs, int) = a.fold_last ? (first ? bounce_flat_all_kernel<true, true> : bounce_flat_all_kernel<false, true>)
-                                                : (first ? bounce_flat_all_kernel<true> : bounce_flat_all_kernel<false>);
+    void (*kernel)(PassArgs, int, FlatPairsU);
+    if (a.flat_uniform)
+        kernel = a.fold_last ? (first ? bounce_flat_all_kernel<true, true, true> : bounce_flat_all_kernel<false, true, true>)
+                             : (first ? bounce_flat_all_kernel<true, false, true> : bounce_flat_all_kernel<false, false, true>);
+    else
+        kernel = a.fold_last ? (first ? bounce_flat_all_kernel<true, true> : bounce_flat_all_kernel<false, true>)
+                             : (first ? bounce_flat_all_kernel<true> : bounce_flat_all_kernel<false>);
     const int grid = persistent_grid(kernel, smem, sm_count);
-    cudaError_t e = launch_pdl(kernel, grid, smem, s, a, bounce);
+    cudaError_t e = launch_pdl(kernel, grid, smem, s, a, bounce, launch_pairs(a));
     if (e != cudaSuccess) note_launch_error("merged bounce kernel launch", e, smem, grid);
     return true;
 }
