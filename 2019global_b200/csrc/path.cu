@@ -173,8 +173,8 @@ static inline float cell_edge(float root_lo, float root_size, int level, uint32_
 }
 
 void path_tuning_from_env(PathTuning& t) {
-    static const char* const keys[] = {"lanes", "pass_slots", "no_merge", "leaf_max", "refill", "coop_leaf", "walk_steps",
-                                       "leaf_batch", "raygen_occ", "tree_build", "debug_tree", "walk", "trace_occ", "l2_persist", "bounce_occ", "top_level", "ref_heavy", "sort_rays", "upload_threads", "bvh_leaf", "bvh_spec", "bvh_stack", "fuse_first", "fold_last", "overlap_frames", "flat_uniform"};
+    static const char* const keys[] = {"lanes", "pass_slots", "leaf_max", "refill", "coop_leaf", "walk_steps", "leaf_batch",
+                                       "tree_build", "debug_tree", "walk", "trace_occ", "top_level", "ref_heavy", "sort_rays", "upload_threads", "bvh_leaf", "bvh_spec", "bvh_stack", "overlap_frames", "flat_uniform"};
     for (const char* k : keys) {
         std::string env = "G19_";
         for (const char* c = k; *c; ++c) env += char(std::toupper(*c));
@@ -188,22 +188,17 @@ bool path_tuning_set(PathTuning& t, const char* key, const char* value) {
     auto num = [&](int dflt, int lo, int hi) { return value ? std::max(lo, std::min(hi, std::atoi(value))) : dflt; };
     if (k == "lanes") t.lanes = num(def.lanes, 1, kMaxLanes);
     else if (k == "pass_slots") t.pass_slots = value ? std::max<long long>(kTilePix, std::atoll(value)) : 0;
-    else if (k == "no_merge") t.no_merge = value ? 1 : 0; // present = on (as the environment variable was)
     else if (k == "leaf_max") t.leaf_max = num(def.leaf_max, 1, 1 << 20);
     else if (k == "refill") t.refill = num(def.refill, 1, 32);
     else if (k == "coop_leaf") t.coop_leaf = num(def.coop_leaf, 0, 1);
     else if (k == "walk_steps") t.walk_steps = num(def.walk_steps, 0, 16);
     else if (k == "leaf_batch") t.leaf_batch = num(def.leaf_batch, 0, 16);
-    else if (k == "raygen_occ") t.raygen_occ = num(def.raygen_occ, 2, 3);
     else if (k == "tree_build") t.tree_build = !value ? -1 : (std::strcmp(value, "device") == 0 ? 1 : (std::strcmp(value, "host") == 0 ? 0 : -1));
     else if (k == "debug_tree") t.debug_tree = value ? 1 : 0;
-    else if (k == "walk") { t.walk = num(def.walk, 0, 4); if (t.walk == 2) t.walk = 1; }
+    else if (k == "walk") { t.walk = num(def.walk, 1, 4); if (t.walk == 2) t.walk = 1; }
     else if (k == "trace_occ") t.trace_occ = num(def.trace_occ, 3, 4);
-    else if (k == "bounce_occ") t.bounce_occ = num(def.bounce_occ, 3, 4);
     else if (k == "top_level") t.top_level = num(def.top_level, 0, 8);
     else if (k == "overlap_frames") t.overlap_frames = num(def.overlap_frames, 0, 1);
-    else if (k == "fold_last") t.fold_last = num(def.fold_last, 0, 1);
-    else if (k == "fuse_first") t.fuse_first = num(def.fuse_first, 0, 1);
     else if (k == "flat_uniform") t.flat_uniform = num(def.flat_uniform, 0, 1);
     else if (k == "bvh_stack") t.bvh_stack = num(def.bvh_stack, 4, 64);
     else if (k == "bvh_spec") t.bvh_spec = num(def.bvh_spec, 0, 3);
@@ -211,7 +206,6 @@ bool path_tuning_set(PathTuning& t, const char* key, const char* value) {
     else if (k == "upload_threads") t.upload_threads = num(def.upload_threads, 0, 64);
     else if (k == "sort_rays") t.sort_rays = num(def.sort_rays, -1, 1);
     else if (k == "ref_heavy") t.ref_heavy = num(def.ref_heavy, 0, 1 << 30);
-    else if (k == "l2_persist") t.l2_persist = num(def.l2_persist, 0, 1);
     else return false;
     return true;
 }
@@ -863,16 +857,14 @@ PassArgs path_pass_setup(const PathSceneBuffers& b, const PathTuning& tune, bool
     // tree walk: leaf tests spread over the whole warp, 8 primitives per ray and round (heightfield 1080p x 32 spp:
     // sequential 4 per round 107.1 ms, cooperative 4 / 8 / 16 per round 115.4 / 104.9 / 105.4)
     pa.coop_leaf = tune.coop_leaf;
-    pa.walk_steps = tune.walk_steps > 0 ? tune.walk_steps : (tune.walk ? 2 : 4); // measured (room scene, ms per 1080p x 64 spp): new walk 2 / 4 / 8 steps = 780 / 838 / 961
+    pa.walk_steps = tune.walk_steps > 0 ? tune.walk_steps : 2; // measured (room scene, ms per 1080p x 64 spp): octree walk 2 / 4 / 8 steps = 780 / 838 / 961
     pa.leaf_batch = tune.leaf_batch > 0 ? tune.leaf_batch : (pa.coop_leaf ? 16 : 4); // cooperative: the whole leaf in one go (leaf max 8 / 12 / 16 at batch 16: 97.7 / 96.9 / 97.8 ms)
-    pa.raygen_occ = tune.raygen_occ;
     pa.trace_occ = tune.trace_occ;
-    pa.bounce_occ = tune.bounce_occ;
     pa.bvh_spec = tune.bvh_spec;
     pa.fold_last = 0;
     pa.flat_uniform = tune.flat_uniform && b.upairs_fit ? 1 : 0;
     pa.upairs = &b.upairs;
-    pa.walk = tune.walk ? (count ? 2 : 1) : 0; // the new walk counts its node / primitive tests when asked (params.profile)
+    pa.walk = count ? 2 : 1; // the octree walk counts its node / primitive tests when asked (params.profile)
     if (tune.walk >= 3 && b.view.bvh_root != 0xffffffffu && b.view.bvh_nodes) {
         pa.walk = tune.walk == 4 ? (count ? 6 : 5) : 3; // bounding-volume hierarchy, binary / 4-wide (the latter counts its tests when asked)
         // node visits per round, room scene: binary 4 / 6 / 8 / 12 = 437 / 423 / 418 / 418 ms; 4-wide 4 / 6 / 8 / 12 = 346 / 345 / 364 / 382 ms
@@ -1091,30 +1083,6 @@ int path_render(PathSceneBuffers& b, PathWork& w, const PathRenderArgs& a, g19_s
             }
         }
     }
-    // Tree scenes: the primitive records are what the incoherent rays of the deep bounces fetch from all over the scene
-    // (ncu, profiles/r02b: L2 hit rate 67 %, 2.8 GB of DRAM traffic per trace launch); the wavefront state streaming
-    // past them must not evict them. An access policy window on every lane's stream asks L2 to keep the records
-    // (persisting) while everything else stays normal; the ray queue is read / written with streaming hints.
-    if (!fused && a.tune.l2_persist && b.hot.bytes > 0) {
-        static thread_local int limit_device = -1;
-        int device = 0;
-        cudaGetDevice(&device);
-        cudaDeviceProp prop;
-        if (cudaGetDeviceProperties(&prop, device) == cudaSuccess && prop.persistingL2CacheMaxSize > 0 && prop.accessPolicyMaxWindowSize > 0) {
-            if (limit_device != device) {
-                cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, size_t(prop.persistingL2CacheMaxSize));
-                limit_device = device;
-            }
-            cudaStreamAttrValue attr = {};
-            attr.accessPolicyWindow.base_ptr = b.hot.p;
-            attr.accessPolicyWindow.num_bytes = std::min(b.hot.bytes, size_t(prop.accessPolicyMaxWindowSize));
-            attr.accessPolicyWindow.hitRatio = float(std::min(1.0, double(prop.persistingL2CacheMaxSize) / double(attr.accessPolicyWindow.num_bytes)));
-            attr.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-            attr.accessPolicyWindow.missProp = cudaAccessPropertyNormal;
-            for (int i = 0; i < n_lanes; ++i) cudaStreamSetAttribute(lane_stream[i], cudaStreamAttributeAccessPolicyWindow, &attr);
-            cudaGetLastError(); // best effort: a refused hint is not an error of the render
-        }
-    }
     {
         size_t lane_bytes_after = 0;
         for (const PathLane& l : w.lane) lane_bytes_after += l.capacity + l.L.bytes + l.recs.bytes + l.rays.bytes + l.queues.bytes + l.counts.bytes + l.rkeys.bytes;
@@ -1132,7 +1100,6 @@ int path_render(PathSceneBuffers& b, PathWork& w, const PathRenderArgs& a, g19_s
             }
         }
     }
-    const bool merge_kinds = !a.tune.no_merge; // tuning knob: one launch per material queue
     ClassClock clk{w, s, p.profile != 0};
     int rc = G19_OK;
     auto last_refresh = std::chrono::steady_clock::now();
@@ -1155,35 +1122,34 @@ int path_render(PathSceneBuffers& b, PathWork& w, const PathRenderArgs& a, g19_s
             pa.pix_base = uint32_t(pix0);
             pa.pix_count = uint32_t(std::min(window, npix - pix0));
             pa.n_slots = uint32_t(size_t(pa.pix_count) * size_t(pa.spp_pass));
-            // diffuse-only flat scenes: camera segment and first vertex in one launch
-            const bool fused_first = fused && a.tune.fuse_first && pa.bounce_occ != 4;
-            const bool spec_scene = (pa.kind_mask & 6u) != 0u;
-            if (!fused_first) {
+            if (!fused) { // flat scenes trace the camera segment in the first bounce's launch
                 clk.begin();
-                launch_raygen_extend(pa, a.sm_count, ls); // camera segment
+                launch_raygen_extend(pa, a.sm_count, ls);
                 clk.end(G19_K_EXTEND);
                 stats.class_launches[G19_K_EXTEND] += 1;
             }
-            // ... and the launch before the last shades the last vertex in place: the last launch disappears
-            const bool fold_last = fused && a.tune.fold_last && pa.bounce_occ != 4 && p.max_depth >= 2;
-            for (int bounce = 0; bounce < p.max_depth; ++bounce) {
-                if (fold_last && bounce == p.max_depth - 1) break; // folded into the previous launch
-                pa.fold_last = (fold_last && bounce == p.max_depth - 2) ? 1 : 0;
+            // flat scenes: the launch before the last shades the last vertex in place, so the last bounce has no launch
+            const int n_launch = fused && p.max_depth >= 2 ? p.max_depth - 1 : p.max_depth;
+            for (int bounce = 0; bounce < n_launch; ++bounce) {
                 clk.begin();
                 int n = 0;
-                if (bounce == 0 && fused_first && launch_bounce_first_fused(pa, a.sm_count, ls)) {
-                    ++n;
-                    if (!spec_scene || p.max_depth <= 1) { // (with mirror / glass the camera hits on those still have their launch below)
-                        clk.end(G19_K_SHADE);
-                        stats.class_launches[G19_K_SHADE] += n;
-                        continue;
+                if (fused) {
+                    pa.fold_last = bounce == p.max_depth - 2 ? 1 : 0;
+                    if (bounce == 0) {
+                        launch_bounce_first_fused(pa, a.sm_count, ls);
+                        ++n;
                     }
+                    // (at bounce 0 with mirror / glass: the camera hits on those, which the fused launch queued)
+                    if ((bounce > 0 || ((pa.kind_mask & 6u) && p.max_depth > 1)) && launch_bounce_flat(pa, bounce, a.sm_count, ls)) ++n;
+                    clk.end(G19_K_SHADE);
+                    stats.class_launches[G19_K_SHADE] += n;
+                    continue;
                 }
                 // the first bounce's rays leave the camera rays' hit points in pixel order: coherent as they are
                 // ... and a queue that stayed short the last time is walked in a blink: not worth three more launches.
                 const size_t ray_cap = 2 * pa.plane + kQueueSlack;
                 size_t n_sort = 0;
-                if (!fused && pa.rkey && bounce > 0) {
+                if (pa.rkey && bounce > 0) {
                     const uint32_t hint = w.ray_hint_h[bounce]; // 0 = not known yet: the whole queue
                     n_sort = hint == 0 ? ray_cap : std::min(ray_cap, size_t(hint) + size_t(hint) / 8 + 65536);
                     if (hint != 0 && hint < (1u << 19)) n_sort = 0;
@@ -1193,16 +1159,11 @@ int path_render(PathSceneBuffers& b, PathWork& w, const PathRenderArgs& a, g19_s
                 pb.perm_n = uint32_t(n_sort);
                 if (!sort_this) pb.rkey = nullptr, pb.perm = nullptr;
                 if (sort_this) PATH_CUDA(cudaMemsetAsync(pa.rkey, 0xff, n_sort * sizeof(uint16_t), ls));
-                if (merge_kinds && launch_bounce_merged(pa, bounce, a.sm_count, ls)) {
-                    n += 1;
-                } else {
-                    for (int kind = Q_DIFFUSE; kind <= Q_GLASS; ++kind) {
-                        if (!b.has_bsdf[kind - 1]) continue; // no such material in the scene: queue is always empty
-                        if (bounce == 0 && fused_first && kind == Q_DIFFUSE) continue; // shaded by the fused launch above
-                        if (launch_bounce(pb, bounce, kind, a.sm_count, ls)) ++n;
-                    }
+                for (int kind = Q_DIFFUSE; kind <= Q_GLASS; ++kind) {
+                    if (!b.has_bsdf[kind - 1]) continue; // no such material in the scene: queue is always empty
+                    if (launch_bounce(pb, bounce, kind, a.sm_count, ls)) ++n;
                 }
-                if (!fused && n > 0) { // tree scenes: one walk over the rays this bounce's vertices produced
+                if (n > 0) { // one walk over the rays this bounce's vertices produced
                     if (sort_this) {
                         PATH_CUDA(launch_ray_sort(w.lane[li].sort_tmp.p, w.lane[li].sort_tmp.bytes, pa.rkey, pa.rkey + ray_cap,
                                                   static_cast<const uint32_t*>(w.iota.p), static_cast<uint32_t*>(w.lane[li].perm.p), n_sort, ls));

@@ -163,25 +163,20 @@ struct PathWork {
 struct PathTuning {
     int lanes = 4;            // passes kept in flight
     long long pass_slots = 0; // path slots per pass (0 = auto)
-    int no_merge = 0;         // one launch per material queue instead of one per bounce
     int leaf_max = 8;         // primitives per octree leaf (read at scene upload)
     int refill = 8;           // trace_kernel: idle lanes per warp that trigger a ray fetch
     int coop_leaf = 1;        // warp-cooperative leaf tests
-    int walk_steps = 0;       // cell moves per round of the tree walk (0 = auto: 2 for the restart walk, 4 for the stack walk)
+    int walk_steps = 0;       // cell moves / node visits per round of the tree walk (0 = auto: 2 for the octree walk, 8 / 5 for the binary / 4-wide BVH)
     int leaf_batch = 0;       // primitives per ray and round (0 = auto: 16 cooperative, 4 sequential)
-    int raygen_occ = 3;       // CTAs per SM of the tree-scene camera-ray kernel
     int tree_build = -1;      // -1 auto (device from 4096 primitives), 0 host, 1 device
     int debug_tree = 0;       // print octree statistics at upload
     int walk = 4;             // tree walk: 4 = 4-wide quantised bounding-volume hierarchy (Bvh4Walk, bvh_build.cu), 3 = its binary form (BvhWalk),
-                              // 1 = point-location restart walk over the linear octree (TreeWalk2), 0 = round 1's parametric stack walk (TreeWalk).
-                              // Room scene, 1080p x 64 spp: 866 / 566 / 378 / 345 ms for 0 / 1 / 3 / 4
+                              // 1 = point-location restart walk over the linear octree (TreeWalk2); 0 and 2 are taken as 1.
+                              // Room scene, 1080p x 64 spp: 566 / 378 / 345 ms for 1 / 3 / 4 (866 for round 1's parametric stack walk)
     int trace_occ = 4;        // CTAs per SM of trace_kernel (4 = 64 registers, 114 bytes of spills: the walk is bound by memory
                               // latency, a third more warps in flight buys more than the spills cost -- room scene 775 -> 687 ms)
-    int bounce_occ = 3;       // CTAs per SM of the diffuse flat-scene bounce kernel (4 = 64 registers, some spills)
     int top_level = 7;        // levels covered by the walk's direct-index table (0 = none; capped at tree depth - 2): 16 MB at 7; ROOM 668 / 630 / 611 ms at 0 / 6 / 7
     int overlap_frames = 1;   // frames rendered back to back: the side lanes start the next frame's passes behind their own, not behind the join
-    int fold_last = 1;        // flat scenes: a path's last vertex (next-event estimation only) is shaded by the launch that finds it
-    int fuse_first = 1;       // flat scenes: trace the camera segment inside the first bounce's launch (no raygen kernel; camera records only for hits on mirror / glass)
     int flat_uniform = 1;     // flat scenes whose pairs fit FlatPairsU: the bounce kernels' pair loops read them from the launch parameters
     int bvh_stack = kBvhSmemStack; // walk=3/4: levels of the postponed-children stack in shared memory (1 KB per level and CTA)
     int bvh_spec = 1;         // walk=3: a lane that reaches a leaf postpones it and keeps descending
@@ -191,8 +186,6 @@ struct PathTuning {
                               // -1 = auto: on for the octree walks (room scene 611 -> 566 ms), off for the BVH walk (397 with, 378 without:
                               // its walk is short enough for the sort to cost more than the coherence brings)
     int ref_heavy = 128;      // REF mode: node expansions after which a ray is spread over many warps (ref_heavy_kernel; 0 = never)
-    int l2_persist = 0;       // tree scenes: pin the primitive records in L2 (access policy window on the lanes' streams). Measured
-                              // on the room scene: 869 ms with the window, 775 ms without -- the set-aside starves everything else; off
 };
 void path_tuning_from_env(PathTuning& t);
 bool path_tuning_set(PathTuning& t, const char* key, const char* value); // false: unknown key
@@ -296,11 +289,9 @@ struct PassArgs {
     // shared-memory staging (see path_kernels.cu stage_scene)
     int32_t stage_nodes, stage_prims, stage_cold, stage_lights, stack_levels;
     int32_t refill;        // trace_kernel: idle lanes per warp that trigger a fetch of new rays
-    int32_t walk_steps, leaf_batch; // tree walk: cell moves / primitives tested per round (TreeWalk::step)
+    int32_t walk_steps, leaf_batch; // tree walk: cell moves / primitives tested per round (TreeWalk2::step)
     int32_t coop_leaf;     // tree walk: leaf tests spread over the whole warp (default; G19_COOP_LEAF=0: sequential)
-    int32_t raygen_occ;    // tree scenes: CTAs per SM of the camera-ray kernel (2 or 3)
     int32_t trace_occ;     // CTAs per SM of trace_kernel (3 or 4)
-    int32_t bounce_occ;    // CTAs per SM of bounce_flat_kernel<diffuse> (3 or 4)
     int32_t bvh_spec;      // BvhWalk: speculative traversal (PathTuning::bvh_spec)
     int32_t fold_last;     // this launch shades the path's last vertex in place (flat scenes, bounce max_depth - 2)
     int32_t walk;          // tree walk variant (PathTuning::walk); +2 when the walk counts its node / primitive tests
@@ -311,11 +302,10 @@ struct PassArgs {
 // path.cu: the PassArgs fields that follow from the scene and the tuning alone (staging sizes, walk and its knobs);
 // count = the walk tallies its node / primitive tests
 PassArgs path_pass_setup(const PathSceneBuffers& b, const PathTuning& tune, bool count);
+// tree scenes: the camera segment
 void launch_raygen_extend(const PassArgs& a, int sm_count, cudaStream_t s);
-// false = nothing to launch for this (bounce, kind): specular vertices on the last segment
+// tree scenes: one material queue; false = nothing to launch for this (bounce, kind): specular vertices on the last segment
 bool launch_bounce(const PassArgs& a, int bounce, int kind, int sm_count, cudaStream_t s);
-// flat scenes with mirror / glass: the three material queues of a bounce in one launch; false = not applicable
-bool launch_bounce_merged(const PassArgs& a, int bounce, int sm_count, cudaStream_t s);
 void launch_trace(const PassArgs& a, int bounce, int sm_count, cudaStream_t s); // tree scenes: after the bounce's shade launches
 // ray_sort.cu
 size_t ray_sort_temp_bytes(size_t n);
@@ -323,8 +313,11 @@ void launch_iota(uint32_t* out, size_t n, cudaStream_t s);
 cudaError_t launch_ray_sort(void* temp, size_t temp_bytes, const uint16_t* keys_in, uint16_t* keys_out, const uint32_t* iota,
                             uint32_t* perm, size_t n, cudaStream_t s);
 bool path_scene_is_flat(const PassArgs& a);
-// diffuse-only flat scenes: the camera segment and the first vertex in ONE launch; false = not applicable
-bool launch_bounce_first_fused(const PassArgs& a, int sm_count, cudaStream_t s);
+// flat scenes, bounce 0: the camera segment and the first vertex in ONE launch (at max_depth 1 the only one)
+void launch_bounce_first_fused(const PassArgs& a, int sm_count, cudaStream_t s);
+// flat scenes, a bounce before the last (bounce 0 only with mirror / glass, whose camera hits the fused launch queued):
+// one launch for all material queues; false = no launch (the scene has no surface a path goes on from)
+bool launch_bounce_flat(const PassArgs& a, int bounce, int sm_count, cudaStream_t s);
 void launch_accumulate(const PassArgs& a, cudaStream_t s);
 void launch_primary(const PassArgs& a, int32_t* ids_l, double* points_l, double* normals_l, int sm_count, cudaStream_t s);
 // batched ray queries (g19_cast_rays): n ray records of two float4 (origin, tmax) (direction, -) -> entity id per ray and,

@@ -4,15 +4,16 @@
 // flight on their own streams (path.cu). Two families of kernels share the shading code:
 //
 // FLAT scenes (the whole scene is one leaf of <= 192 primitives, staged in shared memory):
-//   raygen_extend_flat   camera ray from the pixel index, nearest hit, vertex record written at the
-//                        position the warp's ballot compaction reserved in the material's queue
-//   bounce_flat<KIND>    one material queue of one bounce (diffuse / mirror / glass; scenes with
-//                        specular materials run the three queues of a bounce in ONE launch,
-//                        bounce_flat_all): next-event estimation, BSDF sample, the shadow ray and
-//                        the continuation ray traced in one loop over primitive PAIRS (packed
-//                        FP32), the new vertex record written into the next bounce's queue. The
-//                        queues hold the records themselves (four float4 planes), the path's
-//                        radiance rides in the record and is stored once when the path ends.
+//   bounce_flat_fused    camera ray from the pixel index, nearest hit, and the first vertex shaded
+//                        in place; camera hits on mirror / glass go to their material's queue
+//   bounce_flat          one bounce of a diffuse-only scene (scenes with specular materials run
+//                        the three queues of a bounce in ONE launch, bounce_flat_all): next-event
+//                        estimation, BSDF sample, the shadow ray and the continuation ray traced in
+//                        one loop over primitive PAIRS (packed FP32), the new vertex record written
+//                        into the next bounce's queue. The queues hold the records themselves (four
+//                        float4 planes), the path's radiance rides in the record and is stored once
+//                        when the path ends. The bounce before the last shades the last vertex in
+//                        place (FOLD): the last bounce has no launch.
 // TREE scenes (linear octree in HBM / L2):
 //   raygen_extend        camera ray + ordered octree walk (all 32 lanes of a warp in fixed-trip rounds)
 //   bounce<KIND>         shades a queue of slot indices and queues the vertex's rays
@@ -456,21 +457,7 @@ __device__ __forceinline__ void trace_flat(const SceneAccess<true>& S, float3 o,
     occluded = DUAL && tmax0 > 0.0f && lim0 == 0u;
 }
 
-// Ordered traversal of the linear octree (tree scenes). Parametric front-to-back walk (after
-// Revelles et al. 2000): in the frame where the ray direction is positive on every axis (octant
-// bits XOR a), a cell is described per axis by the ray parameters of its entry plane t0, mid
-// plane tm and exit plane t1. The first child is the one whose mid planes lie before the entry
-// point; the next child is reached through the exit plane with the smallest parameter. Only the
-// (at most four) children the ray pierces are visited, strictly in order, so the walk stops at
-// the first leaf whose hit lies inside its own cell.
-//
-// Per level the state is one 4-bit child code in a 64-bit register, the child base index on a
-// short stack in shared memory (one column per thread, conflict free) and the integer cell
-// coordinates. Plane parameters are linear in the plane index, t(i) = A + i * (B * 2^-(level+1))
-// with A = (root_lo - o) / d and B = root_size / d per axis, evaluated with one FMA each: the
-// planes a child shares with its parent get bit-identical parameters (same exact product), so
-// the walk is consistent from level to level.
-//
+// ---- octree walk (tree scenes) ---------------------------------------------------------------
 // What the ncu capture of the 1M-triangle heightfield drove (profiles/r01b_heightfield_*):
 //   * 4.4 of 32 threads active per instruction: the one-big-loop form serialised "step",
 //     "descend", "test leaf" and "pop" branches -> WHILE-WHILE form: every lane first walks to
@@ -479,42 +466,21 @@ __device__ __forceinline__ void trace_flat(const SceneAccess<true>& S, float3 o,
 //   * 443 MB of leaf-ordered primitive copies (6.9 references per primitive) streamed from DRAM
 //     -> leaves hold 4-byte indices into the 64-byte records: nodes + indices + records = 108 MB,
 //     L2-resident on B200 (126 MB)
-//   * 51 instructions per plane update -> 21 with the linear form
-// `any` = stop at the first hit (shadow rays).
-// The walk as a resumable state machine: init() places the ray at the root, step() advances it
+// The walk is a resumable state machine: init() places the ray at the root, step() advances it
 // to its next non-empty leaf and tests that leaf (one while-while round), returning true when
 // the ray is finished. traverse() below runs it to completion; trace_kernel interleaves the
 // steps of 32 rays per warp and hands a finished lane the next ray of the queue.
-struct TreeWalk {
-    float3 o, d, A, B;
+
+// The leaf test of the octree walk's sequential form and of a scene that is one whole leaf: the ray (o, d) against up to
+// `limit` primitives of the leaf list [first, first + n), nearest hit within `best`, two per step (independent FMA chains,
+// all loads of the step issued up front). `any` = stop at the first hit (shadow rays).
+struct LeafTest {
+    float3 o, d;
     float best;
-    uint32_t best_prim, a;
-    int level;
-    uint32_t ix, iy, iz;
-    float t0x, t0y, t0z, tmx, tmy, tmz, t1x, t1y, t1z;
-    unsigned long long codes; // 4 bits per level: 0xF = not started, else current child (mirrored)
-    uint32_t leaf_first, leaf_n; // the part of the current leaf's list still to be tested
-    float leaf_exit;             // parameter at which the ray leaves the current leaf's cell
+    uint32_t best_prim;
     bool any;
 
-    __device__ __forceinline__ void planes() { // entry / mid / exit parameters of the cell (level; ix,iy,iz)
-        const float s1 = __int_as_float((127 - (level + 1)) << 23); // 2^-(level+1), exact
-        const float hx = B.x * s1, hy = B.y * s1, hz = B.z * s1;
-        const float fx = float(2u * ix), fy = float(2u * iy), fz = float(2u * iz);
-        const float ax = fmaf(fx, hx, A.x), bx = fmaf(fx + 2.0f, hx, A.x);
-        const float ay = fmaf(fy, hy, A.y), by = fmaf(fy + 2.0f, hy, A.y);
-        const float az = fmaf(fz, hz, A.z), bz = fmaf(fz + 2.0f, hz, A.z);
-        t0x = fminf(ax, bx); t1x = fmaxf(ax, bx);
-        t0y = fminf(ay, by); t1y = fmaxf(ay, by);
-        t0z = fminf(az, bz); t1z = fmaxf(az, bz);
-        tmx = fmaf(fx + 1.0f, hx, A.x);
-        tmy = fmaf(fy + 1.0f, hy, A.y);
-        tmz = fmaf(fz + 1.0f, hz, A.z);
-    }
-
-    // tests up to `limit` primitives of the list [first, first + n), two per step (independent FMA
-    // chains, all loads of the step issued up front)
-    __device__ __forceinline__ void leaf(const PathSceneD& g, uint32_t first, uint32_t n, uint32_t limit) {
+    __device__ __forceinline__ void run(const PathSceneD& g, uint32_t first, uint32_t n, uint32_t limit) {
         const uint32_t* __restrict__ index = g.index;
         const float4* __restrict__ hot = reinterpret_cast<const float4*>(g.hot);
         if (n > limit) n = limit;
@@ -536,179 +502,11 @@ struct TreeWalk {
             if (any && best_prim != kInvalid) break;
         }
     }
-
-    // returns true when the ray is already finished (missed the root box, or the scene is one leaf)
-    template <bool ALL>
-    __device__ __forceinline__ bool init(const SceneAccess<ALL>& S, float3 o_, float3 d_, float tmax, bool any_) {
-        const PathSceneD& g = *S.g;
-        o = o_;
-        d = d_;
-        best = tmax;
-        best_prim = kInvalid;
-        any = any_;
-        const uint2 root = S.node(0);
-        leaf_n = 0;
-        if (root.y & kLeafBit) { // the whole scene is one leaf (but not staged as a flat scene)
-            leaf(g, root.x, root.y & ~kLeafBit, 0x7fffffffu);
-            return true;
-        }
-        float3 dd = d;
-        if (fabsf(dd.x) < 1.0e-20f) dd.x = copysignf(1.0e-20f, dd.x);
-        if (fabsf(dd.y) < 1.0e-20f) dd.y = copysignf(1.0e-20f, dd.y);
-        if (fabsf(dd.z) < 1.0e-20f) dd.z = copysignf(1.0e-20f, dd.z);
-        const float3 inv = f3(__fdividef(1.0f, dd.x), __fdividef(1.0f, dd.y), __fdividef(1.0f, dd.z));
-        a = (dd.x < 0.0f ? 1u : 0u) | (dd.y < 0.0f ? 2u : 0u) | (dd.z < 0.0f ? 4u : 0u);
-        A = f3((g.root_lo[0] - o.x) * inv.x, (g.root_lo[1] - o.y) * inv.y, (g.root_lo[2] - o.z) * inv.z);
-        B = f3(g.root_size[0] * inv.x, g.root_size[1] * inv.y, g.root_size[2] * inv.z);
-        level = 0;
-        ix = iy = iz = 0;
-        planes();
-        const float tn = fmaxf(fmaxf(t0x, t0y), t0z), tf = fminf(fminf(t1x, t1y), t1z);
-        if (tn > fminf(tf, best) + 1.0e-5f || tf < 0.0f) return true;
-        codes = 0xFull;
-        S.stack[0] = root.x;
-        return false;
-    }
-
-    // One ROUND, built so that the 32 rays of a warp stay in step: exactly kWalkSteps cell moves
-    // towards the next non-empty leaf (predicated off for lanes that have arrived or are finished),
-    // then one batch of at most kLeafBatch primitives of the current leaf. MUST be called by all 32
-    // lanes of the warp (`active` = this lane has a ray): the loop re-converges the warp at every
-    // move -- with `continue`/`break` in a data-dependent loop the lanes drifted apart and ran the
-    // loop body in ~2.5 separate groups of 5.6 lanes (ncu, profiles/r01_tuning_log.md).
-    // Returns true when the lane's ray is finished.
-    template <bool ALL, bool COOP> __device__ __forceinline__ bool step(const SceneAccess<ALL>& S, bool active) {
-        uint32_t* const stack = S.stack;
-        bool done = false;
-        const int kWalkSteps = S.walk_steps;      // PassArgs::walk_steps (default 4)
-        const uint32_t kLeafBatch = S.leaf_batch; // PassArgs::leaf_batch (default 4)
-#pragma unroll 1
-        for (int it = 0; it < kWalkSteps; ++it) {
-            __syncwarp();
-            if (active && !done && leaf_n == 0u) {
-                // first child / next child, both evaluated branch-free (a branch here made the
-                // compiler run the rest of the move once per side: ncu, 2 x 5.6 lanes)
-                const uint32_t old = uint32_t(codes >> (4 * level)) & 0xFu;
-                const bool fresh = old == 0xFu;
-                const float te = fmaxf(fmaxf(fmaxf(t0x, t0y), t0z), 0.0f);
-                const uint32_t first = (tmx < te ? 1u : 0u) | (tmy < te ? 2u : 0u) | (tmz < te ? 4u : 0u);
-                const float ex = (old & 1u) ? t1x : tmx, ey = (old & 2u) ? t1y : tmy, ez = (old & 4u) ? t1z : tmz;
-                const uint32_t bit = (ex <= ey && ex <= ez) ? 1u : (ey <= ez ? 2u : 4u);
-                const bool leave = !fresh && (old & bit) != 0u;
-                const uint32_t cur = fresh ? first : (old | bit);
-                bool moved = false;
-                if (leave) { // the ray left this cell: back to the parent
-                    if (level == 0) {
-                        done = true;
-                    } else {
-                        --level;
-                        ix >>= 1; iy >>= 1; iz >>= 1;
-                        moved = true;
-                    }
-                } else {
-                    const float cen = fmaxf(fmaxf((cur & 1u) ? tmx : t0x, (cur & 2u) ? tmy : t0y), (cur & 4u) ? tmz : t0z);
-                    const float cex = fminf(fminf((cur & 1u) ? t1x : tmx, (cur & 2u) ? t1y : tmy), (cur & 4u) ? t1z : tmz);
-                    if (cen > best + fabsf(best) * 2.0e-6f + 1.0e-5f) {
-                        done = true; // everything from here on is farther than the hit
-                    } else {
-                        codes = (codes & ~(0xFull << (4 * level))) | ((unsigned long long)cur << (4 * level));
-                        if (cex >= 0.0f) {
-                            const uint32_t c = cur ^ a;
-                            const uint2 rec = S.node(stack[level * kThreads] + c);
-                            if (rec.y != kLeafBit) { // not an empty octant
-                                if (rec.y & kLeafBit) {
-                                    leaf_first = rec.x;
-                                    leaf_n = rec.y & ~kLeafBit;
-                                    leaf_exit = cex;
-                                } else {
-                                    ++level;
-                                    stack[level * kThreads] = rec.x;
-                                    ix = 2u * ix + (c & 1u); iy = 2u * iy + ((c >> 1) & 1u); iz = 2u * iz + ((c >> 2) & 1u);
-                                    codes |= 0xFull << (4 * level);
-                                    moved = true;
-                                }
-                            }
-                        }
-                    }
-                }
-                if (moved) planes();
-            }
-        }
-        __syncwarp();
-        // ---- test: the next batch of the current leaf's primitives ----
-        if constexpr (COOP) {
-            // COOPERATIVE form (default; G19_COOP_LEAF=0 selects the sequential one): ncu showed the leaf batches running at ~8 of 32 lanes (only
-            // the lanes that stand in a leaf) for 28 % of trace_kernel's instructions. Here the warp's pending
-            // (ray, primitive) pairs are spread over all 32 lanes: a lane looks up which ray task j belongs to
-            // (binary search over the inclusive prefix sum of the batch sizes), fetches that ray by shuffle,
-            // tests ONE primitive, and the nearest hit per ray is reduced with a 64-bit atomicMin on
-            // (t bits << 32 | primitive) in the warp's shared-memory slots. Same hits as the sequential form;
-            // a tie in t goes to the lower primitive id.
-            const uint32_t lane = threadIdx.x & 31u;
-            const bool mine = active && !done && leaf_n != 0u;
-            const uint32_t cnt = mine ? (leaf_n < kLeafBatch ? leaf_n : kLeafBatch) : 0u;
-            if (__ballot_sync(kFull, cnt != 0u) != 0u) {
-                uint32_t inc = cnt; // inclusive prefix sum over the lanes
-#pragma unroll
-                for (int off = 1; off < 32; off <<= 1) {
-                    const uint32_t v = __shfl_up_sync(kFull, inc, off);
-                    if (lane >= uint32_t(off)) inc += v;
-                }
-                const uint32_t total = __shfl_sync(kFull, inc, 31);
-                const uint32_t exc = inc - cnt;
-                S.coop[lane] = ~0ull;
-                __syncwarp();
-                const uint32_t* __restrict__ index = S.g->index;
-                const float4* __restrict__ hot = reinterpret_cast<const float4*>(S.g->hot);
-                for (uint32_t base = 0; base < total; base += 32u) {
-                    const uint32_t j = base + lane;
-                    uint32_t own = 0; // number of lanes whose tasks all lie before j = the owner of task j
-#pragma unroll
-                    for (int stepw = 16; stepw > 0; stepw >>= 1) {
-                        const uint32_t probe = __shfl_sync(kFull, inc, int(own) + stepw - 1);
-                        if (probe <= j) own += uint32_t(stepw);
-                    }
-                    const bool valid = j < total;
-                    if (!valid) own = 0;
-                    const uint32_t k = j - __shfl_sync(kFull, exc, int(own));
-                    const uint32_t lf = __shfl_sync(kFull, leaf_first, int(own));
-                    const float rox = __shfl_sync(kFull, o.x, int(own)), roy = __shfl_sync(kFull, o.y, int(own)), roz = __shfl_sync(kFull, o.z, int(own));
-                    const float rdx = __shfl_sync(kFull, d.x, int(own)), rdy = __shfl_sync(kFull, d.y, int(own)), rdz = __shfl_sync(kFull, d.z, int(own));
-                    const float rbest = __shfl_sync(kFull, best, int(own));
-                    if (valid) {
-                        const uint32_t id = __ldg(index + lf + k);
-                        const float4* pp = hot + 4 * (size_t)id;
-                        const float4 a0 = __ldg(pp), b0 = __ldg(pp + 1), c0 = __ldg(pp + 2), g0 = __ldg(pp + 3);
-                        const float t = hit_prim(a0, b0, c0, g0, f3(rox, roy, roz), f3(rdx, rdy, rdz), rbest);
-                        if (t >= 0.0f) atomicMin(S.coop + own, ((unsigned long long)__float_as_uint(t) << 32) | id);
-                    }
-                }
-                __syncwarp();
-                if (cnt != 0u) {
-                    const unsigned long long r = S.coop[lane];
-                    if (r != ~0ull) { best = __uint_as_float(uint32_t(r >> 32)); best_prim = uint32_t(r); }
-                    leaf_first += cnt;
-                    leaf_n -= cnt;
-                    if (any && best_prim != kInvalid) done = true;
-                    else if (leaf_n == 0u && best_prim != kInvalid && best <= leaf_exit) done = true;
-                }
-                __syncwarp();
-            }
-        } else if (active && !done && leaf_n != 0u) { // sequential form: every lane tests its own leaf's primitives
-            leaf(*S.g, leaf_first, leaf_n, kLeafBatch);
-            const uint32_t tested = leaf_n < kLeafBatch ? leaf_n : kLeafBatch;
-            leaf_first += tested;
-            leaf_n -= tested;
-            if (any && best_prim != kInvalid) done = true;                                // any hit ends a shadow ray
-            else if (leaf_n == 0u && best_prim != kInvalid && best <= leaf_exit) done = true; // a hit inside its own cell cannot be beaten
-        }
-        __syncwarp();
-        return done;
-    }
 };
 
 // ---- TreeWalk2: point-location restart walk ---------------------------------------------------
-// What the round-1 capture of the parametric walk above showed (profiles/r01f_tree_kernels_ncu.json): ~870 warp
+// What the round-1 capture of the walk this one replaced, a parametric front-to-back walk after Revelles et al. 2000
+// (profiles/r01f_tree_kernels_ncu.json), showed: ~870 warp
 // instructions per ray at 13.7 of 32 lanes, 62 % of them cell MOVES at ~130 instructions each -- every move
 // recomputes nine plane parameters, edits a 64-bit code word with variable shifts and runs a four-way
 // leave / descend / skip / arrive decision, and going from one leaf to a neighbour under another ancestor costs one
@@ -718,8 +516,9 @@ struct TreeWalk {
 //   descend   from the deepest ancestor still valid for (X, Y, Z) -- its child base sits on the per-thread stack in
 //             shared memory -- follow the coordinate bits down to the leaf or empty cell: three bit extracts, one
 //             8-byte node record, ~12 instructions per level, typically 1-3 levels
-//   exit      the parameter at which the ray leaves the cell: one FMA per axis on the same linear plane form
-//             t(i) = A + i * (B * 2^-level) as before (shared planes get bit-identical parameters), minimum of three
+//   exit      the parameter at which the ray leaves the cell: one FMA per axis on the linear plane form
+//             t(i) = A + i * (B * 2^-level), A = (root_lo - o) / d and B = root_size / d per axis (the planes a cell
+//             shares with its parent get bit-identical parameters: same exact product), minimum of three
 //   advance   step the exit axis' coordinate to the neighbouring cell (exact integer arithmetic: no epsilon nudging),
 //             re-derive the other two from the exit point clamped to the current cell's range, and find the common
 //             ancestor with one XOR + CLZ
@@ -749,9 +548,9 @@ template <bool COUNT> struct TreeWalk2 {
         leaf_n = 0;
         const uint2 root = S.node(0);
         if (root.y & kLeafBit) { // the whole scene is one leaf (but not staged as a flat scene)
-            TreeWalk w0 = {};
+            LeafTest w0 = {}; // (set member by member: aggregate initialisation compiles the same arithmetic to other SASS)
             w0.o = o; w0.d = d; w0.best = best; w0.best_prim = kInvalid; w0.any = any_;
-            w0.leaf(g, root.x, root.y & ~kLeafBit, 0x7fffffffu);
+            w0.run(g, root.x, root.y & ~kLeafBit, 0x7fffffffu);
             best = w0.best;
             best_prim = w0.best_prim;
             return true;
@@ -788,7 +587,9 @@ template <bool COUNT> struct TreeWalk2 {
     // One ROUND for the 32 rays of a warp (MUST be called by all lanes, `active` = this lane has a ray): walk_steps
     // times [advance out of the finished cell, descend to the next leaf / empty cell, compute its exit], then one
     // batch of at most leaf_batch primitives of the lanes that stand in a leaf. Returns true when the lane's ray is
-    // finished.
+    // finished. The fixed-trip loop re-converges the warp at every move: with `continue` / `break` in a data-dependent
+    // loop the lanes drifted apart and ran the loop body in ~2.5 separate groups of 5.6 lanes (ncu,
+    // profiles/r01_tuning_log.md).
     template <bool ALL, bool COOP> __device__ __forceinline__ bool step(const SceneAccess<ALL>& S, bool active) {
         uint32_t* const stack = S.stack;
         const PathSceneD& g = *S.g;
@@ -883,9 +684,15 @@ template <bool COUNT> struct TreeWalk2 {
             }
         }
         __syncwarp();
-        // ---- test: the next batch of the current leaf's primitives (same two forms as TreeWalk::step) ----
+        // ---- test: the next batch of the current leaf's primitives ----
         const bool any = (state & 1u) != 0u;
         if constexpr (COOP) {
+            // COOPERATIVE form (default; coop_leaf = 0 selects the sequential one): ncu showed the leaf batches running at
+            // ~8 of 32 lanes (only the lanes that stand in a leaf) for 28 % of trace_kernel's instructions. Here the warp's
+            // pending (ray, primitive) pairs are spread over all 32 lanes: a lane looks up which ray task j belongs to
+            // (binary search over the inclusive prefix sum of the batch sizes), fetches that ray by shuffle, tests ONE
+            // primitive, and the nearest hit per ray is reduced with a 64-bit atomicMin on (t bits << 32 | primitive) in
+            // the warp's shared-memory slots. Same hits as the sequential form; a tie in t goes to the lower primitive id.
             const uint32_t lane = threadIdx.x & 31u;
             const bool mine = active && !done && leaf_n != 0u;
             const uint32_t cnt = mine ? (leaf_n < kLeafBatch ? leaf_n : kLeafBatch) : 0u;
@@ -938,9 +745,9 @@ template <bool COUNT> struct TreeWalk2 {
                 __syncwarp();
             }
         } else if (active && !done && leaf_n != 0u) { // sequential form: every lane tests its own leaf's primitives
-            TreeWalk w0 = {};
+            LeafTest w0 = {};
             w0.o = o; w0.d = d; w0.best = best; w0.best_prim = best_prim; w0.any = any;
-            w0.leaf(g, leaf_first, leaf_n, kLeafBatch);
+            w0.run(g, leaf_first, leaf_n, kLeafBatch);
             best = w0.best;
             best_prim = w0.best_prim;
             const uint32_t tested = leaf_n < kLeafBatch ? leaf_n : kLeafBatch;
@@ -1268,7 +1075,7 @@ template <bool COUNT> struct Bvh4Walk { // COUNT: box and primitive tests are ta
     }
 };
 
-template <int WALK> struct WalkOf { using type = TreeWalk; };
+template <int WALK> struct WalkOf;
 template <> struct WalkOf<1> { using type = TreeWalk2<false>; };
 template <> struct WalkOf<2> { using type = TreeWalk2<true>; };
 template <> struct WalkOf<3> { using type = BvhWalk; };
@@ -1295,7 +1102,7 @@ __device__ __forceinline__ void flush_walk_counts(const PassArgs& a, unsigned no
 
 // Runs the walks of a whole warp to completion; MUST be called by all 32 lanes (`active` = this
 // lane has a ray). Used for camera rays; secondary rays go through trace_kernel.
-template <bool ALL, bool COOP, int WALK = 0>
+template <bool ALL, bool COOP, int WALK>
 __device__ bool traverse(const SceneAccess<ALL>& S, bool active, float3 o, float3 d, float tmax, bool any, float& t_hit,
                          uint32_t& prim_hit, unsigned* n_node = nullptr, unsigned* n_prim = nullptr) {
     typename WalkOf<WALK>::type w = {};
@@ -1462,7 +1269,7 @@ struct Sorter {
 };
 
 // Nearest hit of one ray, flat or tree. Called by all 32 lanes; `active` = the lane has a ray.
-template <bool ALL, bool COOP = false, int WALK = 0>
+template <bool ALL, bool COOP, int WALK>
 __device__ __forceinline__ bool nearest(const SceneAccess<ALL>& S, bool active, float3 o, float3 d, float& t, uint32_t& prim,
                                         unsigned* n_node = nullptr, unsigned* n_prim = nullptr) {
     if constexpr (ALL) {
@@ -1482,7 +1289,8 @@ __device__ __forceinline__ void store_vertex(const PassArgs& a, uint32_t slot, f
 }
 
 // ---- raygen + extend (camera segment), tree scenes: slot-indexed state ----------------------
-template <int OCC, bool COOP, int WALK> __global__ void __launch_bounds__(kThreads, OCC) raygen_extend_kernel(const PassArgs a) {
+// 3 CTAs per SM at 80 registers (68 bytes of spills) beat 2 at 95 on the octree walk: 23.8 vs 26.4 ms per 66 M camera rays
+template <bool COOP, int WALK> __global__ void __launch_bounds__(kThreads, 3) raygen_extend_kernel(const PassArgs a) {
     pdl_launch_dependents();
     const uint32_t n = a.n_slots;
     if (blockIdx.x * kThreads >= n) return;
@@ -1729,59 +1537,6 @@ template <bool SPEC> struct RecSorter {
     }
 };
 
-// ---- raygen + extend, flat scenes ------------------------------------------------------
-template <bool SPEC> __global__ void __launch_bounds__(kThreads, 4) raygen_extend_flat_kernel(const PassArgs a) {
-    pdl_launch_dependents();
-    const uint32_t n = a.n_slots;
-    if (blockIdx.x * kThreads >= n) return;
-    const SceneAccess<true> S = stage_scene<true>(a);
-    pdl_wait(); // the previous pass's accumulate cleared the queue lengths and the radiance planes
-    RecSorter<SPEC> out;
-    out.init(a, 0);
-    const uint32_t stride = gridDim.x * kThreads;
-    const uint32_t lane = threadIdx.x & 31u;
-    for (uint32_t q = blockIdx.x * kThreads + threadIdx.x; q - lane < n; q += stride) { // warp-uniform trip count
-        const uint32_t slot = q;
-        int kind = -1;
-        bool live = false;
-        uint32_t pixel = 0, prim = kInvalid, sample = 0;
-        float3 o = f3(0.f, 0.f, 0.f), d = f3(0.f, 0.f, 1.f);
-        float t = 0.0f;
-        if (q < n) {
-            int x, y;
-            live = slot_pixel(a, slot, x, y, sample);
-            if (live) {
-                pixel = uint32_t(y) * uint32_t(a.map.w) + uint32_t(x);
-                camera_ray(a, x, y, pixel, sample, o, d);
-            }
-        }
-        float4 seen = make_float4(0.f, 0.f, 0.f, 0.f); // what a path that ends on the camera segment delivers
-        if (nearest<true>(S, live, o, d, t, prim)) {
-            const float4 tag = S.hot_row(prim, 3);
-            const int bsdf = __float_as_int(tag.y); // material class rides in the hot record
-            if (bsdf == G19_BSDF_EMITTER) {          // directly visible light: the path ends here
-                const MaterialD& m = a.scene.materials[__float_as_int(tag.x)];
-                seen = make_float4(m.emission[0], m.emission[1], m.emission[2], 0.0f);
-            } else if (bsdf == G19_BSDF_DIFFUSE || a.max_depth > 1) {
-                kind = bsdf;
-            }
-        }
-        // Every slot of the pass gets its radiance stored exactly once, by whichever kernel ends its
-        // path (here: miss, emitter, or a slot outside the frame), so `accumulate` only reads.
-        if (q < n && kind < 0) reinterpret_cast<float4*>(a.L)[slot] = seen;
-        const uint32_t pos = out.reserve(kind);
-        if (pos != kInvalid) { // throughput is 1 and the radiance 0 on the camera segment: not stored
-            const RecView r = rec_queue(a, kind);
-            const float3 p = o + d * t;
-            const ptrdiff_t at = r.at(pos);
-            r.ls[at] = make_float4(__uint_as_float(sample), 0.f, 0.f, __uint_as_float(slot)); // radiance is 0 here: x carries the sample index
-            r.hp[at] = make_float4(p.x, p.y, p.z, __uint_as_float(prim));
-            r.dw[at] = make_float4(d.x, d.y, d.z, __uint_as_float(pixel));
-        }
-    }
-    out.flush(a);
-}
-
 // Asynchronous prefetch of the NEXT record into shared memory (LDGSTS): a register prefetch gets
 // sunk to its first use by the compiler (ncu: 20 % of the kernel's stall samples sat on that one
 // instruction); a cp.async cannot be, and it holds no registers while in flight. Two buffers per
@@ -1806,18 +1561,18 @@ __device__ __forceinline__ void prefetch_rec(const RecView& r, uint32_t pos, boo
     cp_async_commit();
 }
 
-// KIND: Q_DIFFUSE / Q_MIRROR / Q_GLASS. FIRST: the vertex of the camera segment. LAST: the path's
-// final segment ended here -- next-event estimation only, no continuation.
-// One launch per material queue and bounce: next-event estimation, BSDF sample, the trace of BOTH
-// rays in one loop over the staged primitives, and the new vertex record written straight into
-// the next bounce's material queue.
-// FUSED (flat scenes, first bounce): the camera segment is traced right here instead of by
-// raygen_extend_flat_kernel -- the vertex record of the camera hit (48 B written, 48 B read back, a fifth of the frame's
-// HBM traffic), its queue reservation and a launch per pass disappear; `n` is then the number of path slots of the pass.
-// FOLD (flat scenes, the bounce before the last): the vertex the continuation ray finds would be the path's
+// One material queue of one bounce: next-event estimation, BSDF sample, the trace of BOTH rays in one loop over the
+// staged primitives, and the new vertex record written straight into the next bounce's material queue.
+// KIND: Q_DIFFUSE / Q_MIRROR / Q_GLASS. FIRST: the queue holds the 48-byte records of camera hits. SPEC: the scene has
+// mirror / glass queues to feed.
+// FUSED (the first bounce): the camera segment of each path slot of the pass is traced right here, so the vertex record
+// of a diffuse camera hit (48 B written, 48 B read back, a fifth of the frame's HBM traffic), its queue reservation and
+// a camera launch per pass do not exist; `n` is then the number of path slots of the pass. LAST (FUSED at max_depth 1):
+// the camera segment ended at the path's last vertex -- next-event estimation only, no continuation.
+// FOLD (the bounce before the last): the vertex the continuation ray finds would be the path's
 // last one -- next-event estimation only. It is shaded right here (light sample + shadow ray) instead of being written as a
 // 64-byte record for a launch of its own to read back: same arithmetic in the same order, one launch per pass fewer.
-template <int KIND, bool FIRST, bool LAST, bool SPEC, bool SPLIT = false, bool FUSED = false, bool FOLD = false, bool UNI = false>
+template <int KIND, bool FIRST, bool LAST, bool SPEC, bool FUSED, bool FOLD, bool UNI>
 __device__ __forceinline__ void bounce_flat_body(const PassArgs& a, const int bounce, const SceneAccess<true>& S, const uint32_t n,
                                                  const uint32_t cta, const uint32_t n_cta, RecStage<!FIRST>& stage) {
     constexpr bool kDiffuse = KIND == Q_DIFFUSE;
@@ -1841,7 +1596,7 @@ __device__ __forceinline__ void bounce_flat_body(const PassArgs& a, const int bo
         float3 p = f3(0.f, 0.f, 0.f), d = f3(0.f, 0.f, 1.f);
         uint32_t prim = kInvalid, pixel = 0, sample = 0;
         if (FUSED) {
-            // ---- the camera segment of path slot q (what raygen_extend_flat_kernel does for scenes with specular materials) ----
+            // ---- the camera segment of path slot q ----
             bool live = false;
             float3 o = f3(0.f, 0.f, 0.f);
             if (q < n) {
@@ -1857,7 +1612,7 @@ __device__ __forceinline__ void bounce_flat_body(const PassArgs& a, const int bo
             int spec_kind = -1; // SPEC: the camera ray met a mirror / glass surface: that vertex goes to its material's queue
             float4 seen = make_float4(0.f, 0.f, 0.f, 0.f); // what a path that ends on the camera segment delivers
             bool unused_occ;
-            trace_flat<false, UNI>(S, o, d, live ? FLT_MAX : -1.0f, d, -1.0f, t, pr, unused_occ); // = nearest<true>
+            trace_flat<false, UNI>(S, o, d, live ? FLT_MAX : -1.0f, d, -1.0f, t, pr, unused_occ); // = nearest's flat form
             if (pr != kInvalid) {
                 const float4 tag = S.hot_row(pr, 3);
                 const int bsdf = __float_as_int(tag.y);
@@ -1930,21 +1685,7 @@ __device__ __forceinline__ void bounce_flat_body(const PassArgs& a, const int bo
             bool blocked = false;
             float t_hit = FLT_MAX;
             uint32_t prim_hit = kInvalid;
-            if (kDiffuse && !LAST && SPLIT) {
-                // (bounce_occ = 4 experiment: one ray at a time through the primitive loops -- fewer live registers, the
-                // origin half of the affine maps computed twice)
-                if (sh.want_shadow) {
-                    bool unused;
-                    float ts;
-                    uint32_t ps;
-                    trace_flat<false, UNI>(S, sh.no, sh.w, sh.tmax_s, sh.w, -1.0f, ts, ps, unused);
-                    blocked = ps != kInvalid;
-                }
-                if (cont) {
-                    bool unused;
-                    trace_flat<false, UNI>(S, sh.no, sh.nd, FLT_MAX, sh.nd, -1.0f, t_hit, prim_hit, unused);
-                }
-            } else if (kDiffuse && !LAST) {
+            if (kDiffuse && !LAST) {
                 if (sh.want_shadow || cont)
                     trace_flat<true, UNI>(S, sh.no, sh.nd, cont ? FLT_MAX : -1.0f, sh.w, sh.tmax_s, t_hit, prim_hit, blocked);
             } else if (kDiffuse) { // LAST: the shadow ray alone
@@ -2033,24 +1774,22 @@ __device__ __forceinline__ void bounce_flat_body(const PassArgs& a, const int bo
     }
 }
 
-// One material queue per launch (diffuse-only scenes, and the last bounce of any scene).
-template <int KIND, bool FIRST, bool LAST, bool SPEC, int OCC = 3, bool FOLD = false, bool UNI = false>
-__global__ void __launch_bounds__(kThreads, KIND != Q_DIFFUSE ? 4 : OCC)
-    bounce_flat_kernel(const PassArgs a, const int bounce, const __grid_constant__ FlatPairsU up) {
+// A bounce after the first of a diffuse-only scene: its one material queue.
+template <bool FOLD, bool UNI>
+__global__ void __launch_bounds__(kThreads, 3) bounce_flat_kernel(const PassArgs a, const int bounce, const __grid_constant__ FlatPairsU up) {
     pdl_launch_dependents();
-    if (LAST && KIND != Q_DIFFUSE) return; // a specular vertex on the last segment contributes nothing
     SceneAccess<true> S = stage_scene<true>(a); // does not depend on earlier kernels: overlaps their tail
     S.upairs = &up;
     pdl_wait();
-    const uint32_t n = a.counts[bounce * 4 + KIND];
+    const uint32_t n = a.counts[bounce * 4 + Q_DIFFUSE];
     if (blockIdx.x * kThreads >= n) return; // short queue: surplus CTAs leave
-    __shared__ RecStage<!FIRST> stage;
-    bounce_flat_body<KIND, FIRST, LAST, SPEC, OCC == 4, false, FOLD, UNI>(a, bounce, S, n, blockIdx.x, gridDim.x, stage);
+    __shared__ RecStage<true> stage;
+    bounce_flat_body<Q_DIFFUSE, false, false, false, false, FOLD, UNI>(a, bounce, S, n, blockIdx.x, gridDim.x, stage);
 }
 
-// Diffuse-only flat scenes: camera segment + first vertex in one launch (bounce_flat_body<FUSED>), over the path slots of
-// the pass instead of a queue.
-template <bool LAST, bool FOLD = false, bool SPEC = false, bool UNI = false>
+// The first bounce: camera segment + first vertex in one launch (bounce_flat_body<FUSED>), over the path slots of the pass
+// instead of a queue.
+template <bool LAST, bool FOLD, bool SPEC, bool UNI>
 __global__ void __launch_bounds__(kThreads, 3) bounce_flat_fused_kernel(const PassArgs a, const __grid_constant__ FlatPairsU up) {
     pdl_launch_dependents();
     const uint32_t n = a.n_slots;
@@ -2059,7 +1798,7 @@ __global__ void __launch_bounds__(kThreads, 3) bounce_flat_fused_kernel(const Pa
     S.upairs = &up;
     pdl_wait(); // the previous pass's accumulate cleared the queue lengths
     RecStage<false>& unused = *reinterpret_cast<RecStage<false>*>(g19_dyn_smem); // (the fused body prefetches no records)
-    bounce_flat_body<Q_DIFFUSE, true, LAST, SPEC, false, true, FOLD, UNI>(a, 0, S, n, blockIdx.x, gridDim.x, unused);
+    bounce_flat_body<Q_DIFFUSE, true, LAST, SPEC, true, FOLD, UNI>(a, 0, S, n, blockIdx.x, gridDim.x, unused);
 }
 
 // All three material queues of one bounce in ONE launch (scenes with mirror / glass). The mirror and
@@ -2069,7 +1808,7 @@ __global__ void __launch_bounds__(kThreads, 3) bounce_flat_fused_kernel(const Pa
 // Here the grid's CTAs are split between the queues in proportion to their estimated work, so the
 // specular vertices fill issue slots beside the diffuse ones and a pass is 13 launches, not 34.
 // The per-material queues and kernels' code are unchanged: a CTA runs exactly one KIND.
-template <bool FIRST, bool FOLD = false, bool UNI = false>
+template <bool FIRST, bool FOLD, bool UNI>
 __global__ void __launch_bounds__(kThreads, 3) bounce_flat_all_kernel(const PassArgs a, const int bounce, const __grid_constant__ FlatPairsU up) {
     pdl_launch_dependents();
     SceneAccess<true> S = stage_scene<true>(a);
@@ -2088,9 +1827,9 @@ __global__ void __launch_bounds__(kThreads, 3) bounce_flat_all_kernel(const Pass
     const uint32_t g1 = n1 ? min(G - g2 - g3, (n1 + kThreads - 1) / kThreads) : 0u;
     __shared__ RecStage<!FIRST> stage;
     const uint32_t b = blockIdx.x;
-    if (b < g1) bounce_flat_body<Q_DIFFUSE, FIRST, false, true, false, false, FOLD, UNI>(a, bounce, S, n1, b, g1, stage);
-    else if (b < g1 + g2) bounce_flat_body<Q_MIRROR, FIRST, false, true, false, false, FOLD, UNI>(a, bounce, S, n2, b - g1, g2, stage);
-    else if (b < g1 + g2 + g3) bounce_flat_body<Q_GLASS, FIRST, false, true, false, false, FOLD, UNI>(a, bounce, S, n3, b - g1 - g2, g3, stage);
+    if (b < g1) bounce_flat_body<Q_DIFFUSE, FIRST, false, true, false, FOLD, UNI>(a, bounce, S, n1, b, g1, stage);
+    else if (b < g1 + g2) bounce_flat_body<Q_MIRROR, FIRST, false, true, false, FOLD, UNI>(a, bounce, S, n2, b - g1, g2, stage);
+    else if (b < g1 + g2 + g3) bounce_flat_body<Q_GLASS, FIRST, false, true, false, FOLD, UNI>(a, bounce, S, n3, b - g1 - g2, g3, stage);
 }
 
 // ---- bounce, tree scenes: shade and queue the rays -----------------------------------------
@@ -2240,7 +1979,7 @@ __global__ void __launch_bounds__(kThreads, KIND != Q_DIFFUSE ? 4 : 3) bounce_ke
 
 // ---- trace (tree scenes): persistent walk with dynamic ray fetch -----------------------------
 // One launch per bounce over the ray queue the bounce kernels filled. Every lane owns at most one
-// ray; a round = every lane with a ray walks to its next non-empty leaf and tests it (TreeWalk::step).
+// ray; a round = every lane with a ray walks to its next non-empty leaf and tests it (TreeWalk2::step).
 // Lanes whose ray finished deliver the result -- shadow ray: add the light sample unless occluded;
 // continuation ray: hit point + primitive into the vertex record, slot into its material queue --
 // and, once PassArgs::refill lanes are idle, the warp pulls that many new rays with ONE atomic. A warp's
@@ -2661,76 +2400,48 @@ static cudaError_t launch_pdl(void (*kernel)(KArgs...), int grid, size_t smem, c
     return cudaLaunchKernelEx(&cfg, kernel, args...);
 }
 
-// The flat bounce kernel of these template arguments, in its FlatPairsU form when the pass uses that (not for the
-// bounce_occ = 4 experiment).
-template <int KIND, bool FIRST, bool LAST, bool SPEC, int OCC = 3, bool FOLD = false>
-static void (*flat_bounce_kernel(const PassArgs& a))(PassArgs, int, FlatPairsU) {
-    if constexpr (OCC == 3)
-        if (a.flat_uniform) return bounce_flat_kernel<KIND, FIRST, LAST, SPEC, OCC, FOLD, true>;
-    return bounce_flat_kernel<KIND, FIRST, LAST, SPEC, OCC, FOLD, false>;
-}
-
 // What the flat bounce kernels get as their FlatPairsU parameter.
 static const FlatPairsU& launch_pairs(const PassArgs& a) {
     static const FlatPairsU none{};
     return a.flat_uniform ? *a.upairs : none;
 }
 
-template <int KIND, bool FIRST, bool LAST, bool ALL>
-static void launch_bounce_k(const PassArgs& a, int bounce, size_t smem, int sm_count, cudaStream_t s) {
-    if constexpr (ALL) {
-        void (*kernel)(PassArgs, int, FlatPairsU);
-        if constexpr (KIND == Q_DIFFUSE) {
-            if (a.bounce_occ == 4) kernel = (a.kind_mask & 6u) ? flat_bounce_kernel<KIND, FIRST, LAST, true, 4>(a) : flat_bounce_kernel<KIND, FIRST, LAST, false, 4>(a);
-            else if (!LAST && a.fold_last) kernel = (a.kind_mask & 6u) ? flat_bounce_kernel<KIND, FIRST, LAST, true, 3, true>(a) : flat_bounce_kernel<KIND, FIRST, LAST, false, 3, true>(a);
-            else kernel = (a.kind_mask & 6u) ? flat_bounce_kernel<KIND, FIRST, LAST, true>(a) : flat_bounce_kernel<KIND, FIRST, LAST, false>(a);
-        }
-        else if (!LAST && a.fold_last) kernel = flat_bounce_kernel<KIND, FIRST, LAST, true, 3, true>(a);
-        else kernel = flat_bounce_kernel<KIND, FIRST, LAST, true>(a);
-        const int grid = persistent_grid(kernel, smem, sm_count);
-        cudaError_t e = launch_pdl(kernel, grid, smem, s, a, bounce, launch_pairs(a));
-        if (e != cudaSuccess) note_launch_error("bounce kernel launch", e, smem, grid);
-    } else {
-        void (*kernel)(PassArgs, int) = bounce_kernel<KIND, FIRST, LAST>;
-        const int grid = persistent_grid(kernel, smem, sm_count);
-        cudaError_t e = launch_pdl(kernel, grid, smem, s, a, bounce);
-        if (e != cudaSuccess) note_launch_error("bounce kernel launch", e, smem, grid);
-    }
+// Flat scenes, a bounce after the camera segment's: the three material queues in one launch when the scene has mirror /
+// glass (at bounce 0 only their queues hold records: the fused launch shaded the diffuse camera hits), else the diffuse
+// queue (bounces >= 1).
+template <bool FOLD, bool UNI> static void (*flat_bounce_kernel(const PassArgs& a, bool first))(PassArgs, int, FlatPairsU) {
+    if (a.kind_mask & 6u) return first ? bounce_flat_all_kernel<true, FOLD, UNI> : bounce_flat_all_kernel<false, FOLD, UNI>;
+    return bounce_flat_kernel<FOLD, UNI>;
 }
 
-template <int KIND, bool ALL> static void launch_bounce_fl(const PassArgs& a, int bounce, size_t smem, int sm_count, cudaStream_t s) {
+// Tree scenes only shade here: no scene staging, no dynamic shared memory.
+template <int KIND, bool FIRST, bool LAST> static void launch_bounce_k(const PassArgs& a, int bounce, int sm_count, cudaStream_t s) {
+    void (*kernel)(PassArgs, int) = bounce_kernel<KIND, FIRST, LAST>;
+    const int grid = persistent_grid(kernel, 0, sm_count);
+    cudaError_t e = launch_pdl(kernel, grid, 0, s, a, bounce);
+    if (e != cudaSuccess) note_launch_error("bounce kernel launch", e, 0, grid);
+}
+
+template <int KIND> static void launch_bounce_fl(const PassArgs& a, int bounce, int sm_count, cudaStream_t s) {
     const bool first = bounce == 0, last = bounce + 1 >= a.max_depth;
-    if (first && last) launch_bounce_k<KIND, true, true, ALL>(a, bounce, smem, sm_count, s);
-    else if (first) launch_bounce_k<KIND, true, false, ALL>(a, bounce, smem, sm_count, s);
-    else if (last) launch_bounce_k<KIND, false, true, ALL>(a, bounce, smem, sm_count, s);
-    else launch_bounce_k<KIND, false, false, ALL>(a, bounce, smem, sm_count, s);
+    if (first && last) launch_bounce_k<KIND, true, true>(a, bounce, sm_count, s);
+    else if (first) launch_bounce_k<KIND, true, false>(a, bounce, sm_count, s);
+    else if (last) launch_bounce_k<KIND, false, true>(a, bounce, sm_count, s);
+    else launch_bounce_k<KIND, false, false>(a, bounce, sm_count, s);
 }
 
 } // namespace
 
 void launch_raygen_extend(const PassArgs& a, int sm_count, cudaStream_t s) {
     const size_t smem = path_smem_bytes(a);
-    cudaError_t e;
-    int grid;
-    if (all_staged(a)) {
-        auto kernel = (a.kind_mask & 6u) ? raygen_extend_flat_kernel<true> : raygen_extend_flat_kernel<false>;
-        grid = persistent_grid(kernel, smem, sm_count);
-        e = launch_pdl(kernel, grid, smem, s, a);
-    } else {
-        const int occ = a.raygen_occ; // tuning knob
-        // 3 CTAs per SM at 80 registers (68 bytes of spills) beat 2 at 95: 23.8 vs 26.4 ms per 66 M camera rays
-        void (*kernel)(PassArgs);
-        if (a.walk == 6) kernel = raygen_extend_kernel<3, false, 6>;
-        else if (a.walk == 5) kernel = raygen_extend_kernel<3, false, 5>;
-        else if (a.walk == 3) kernel = raygen_extend_kernel<3, false, 3>;
-        else if (a.walk == 2) kernel = a.coop_leaf ? raygen_extend_kernel<3, true, 2> : raygen_extend_kernel<3, false, 2>;
-        else if (a.walk == 1) kernel = a.coop_leaf ? (occ == 2 ? raygen_extend_kernel<2, true, 1> : raygen_extend_kernel<3, true, 1>)
-                                                   : (occ == 2 ? raygen_extend_kernel<2, false, 1> : raygen_extend_kernel<3, false, 1>);
-        else kernel = a.coop_leaf ? (occ == 2 ? raygen_extend_kernel<2, true, 0> : raygen_extend_kernel<3, true, 0>)
-                                  : (occ == 2 ? raygen_extend_kernel<2, false, 0> : raygen_extend_kernel<3, false, 0>);
-        grid = persistent_grid(kernel, smem, sm_count);
-        e = launch_pdl(kernel, grid, smem, s, a);
-    }
+    void (*kernel)(PassArgs);
+    if (a.walk == 6) kernel = raygen_extend_kernel<false, 6>;
+    else if (a.walk == 5) kernel = raygen_extend_kernel<false, 5>;
+    else if (a.walk == 3) kernel = raygen_extend_kernel<false, 3>;
+    else if (a.walk == 2) kernel = a.coop_leaf ? raygen_extend_kernel<true, 2> : raygen_extend_kernel<false, 2>;
+    else kernel = a.coop_leaf ? raygen_extend_kernel<true, 1> : raygen_extend_kernel<false, 1>;
+    const int grid = persistent_grid(kernel, smem, sm_count);
+    const cudaError_t e = launch_pdl(kernel, grid, smem, s, a);
     if (e != cudaSuccess) note_launch_error("raygen_extend kernel launch", e, smem, grid);
 }
 
@@ -2741,8 +2452,7 @@ void launch_trace(const PassArgs& a, int bounce, int sm_count, cudaStream_t s) {
     else if (a.walk == 5) kernel = a.trace_occ == 4 ? trace_kernel<false, 5, 4> : trace_kernel<false, 5, 3>;
     else if (a.walk == 3) kernel = a.trace_occ == 4 ? trace_kernel<false, 3, 4> : trace_kernel<false, 3, 3>;
     else if (a.walk == 2) kernel = a.coop_leaf ? trace_kernel<true, 2> : trace_kernel<false, 2>;
-    else if (a.walk == 1) kernel = a.coop_leaf ? (a.trace_occ == 4 ? trace_kernel<true, 1, 4> : trace_kernel<true, 1, 3>) : trace_kernel<false, 1>;
-    else kernel = a.coop_leaf ? trace_kernel<true, 0> : trace_kernel<false, 0>;
+    else kernel = a.coop_leaf ? (a.trace_occ == 4 ? trace_kernel<true, 1, 4> : trace_kernel<true, 1, 3>) : trace_kernel<false, 1>;
     const int grid = persistent_grid(kernel, smem, sm_count);
     cudaError_t e = launch_pdl(kernel, grid, smem, s, a, bounce);
     if (e != cudaSuccess) note_launch_error("trace kernel launch", e, smem, grid);
@@ -2750,62 +2460,43 @@ void launch_trace(const PassArgs& a, int bounce, int sm_count, cudaStream_t s) {
 
 bool path_scene_is_flat(const PassArgs& a) { return all_staged(a); }
 
-// Diffuse-only flat scenes: raygen + first bounce in one launch; false = not applicable (the caller launches the two).
-bool launch_bounce_first_fused(const PassArgs& a, int sm_count, cudaStream_t s) {
-    if (!all_staged(a) || a.bounce_occ == 4) return false;
+void launch_bounce_first_fused(const PassArgs& a, int sm_count, cudaStream_t s) {
     const size_t smem = path_smem_bytes(a);
     void (*kernel)(PassArgs, FlatPairsU);
     const bool u = a.flat_uniform != 0;
     if (a.kind_mask & 6u) // mirror / glass in the scene: diffuse camera hits shaded in place, specular ones queued
-        kernel = a.max_depth <= 1 ? (u ? bounce_flat_fused_kernel<true, false, true, true> : bounce_flat_fused_kernel<true, false, true>)
-                 : a.fold_last    ? (u ? bounce_flat_fused_kernel<false, true, true, true> : bounce_flat_fused_kernel<false, true, true>)
-                                  : (u ? bounce_flat_fused_kernel<false, false, true, true> : bounce_flat_fused_kernel<false, false, true>);
+        kernel = a.max_depth <= 1 ? (u ? bounce_flat_fused_kernel<true, false, true, true> : bounce_flat_fused_kernel<true, false, true, false>)
+                 : a.fold_last    ? (u ? bounce_flat_fused_kernel<false, true, true, true> : bounce_flat_fused_kernel<false, true, true, false>)
+                                  : (u ? bounce_flat_fused_kernel<false, false, true, true> : bounce_flat_fused_kernel<false, false, true, false>);
     else
-        kernel = a.max_depth <= 1 ? (u ? bounce_flat_fused_kernel<true, false, false, true> : bounce_flat_fused_kernel<true>)
-                 : a.fold_last    ? (u ? bounce_flat_fused_kernel<false, true, false, true> : bounce_flat_fused_kernel<false, true>)
-                                  : (u ? bounce_flat_fused_kernel<false, false, false, true> : bounce_flat_fused_kernel<false>);
+        kernel = a.max_depth <= 1 ? (u ? bounce_flat_fused_kernel<true, false, false, true> : bounce_flat_fused_kernel<true, false, false, false>)
+                 : a.fold_last    ? (u ? bounce_flat_fused_kernel<false, true, false, true> : bounce_flat_fused_kernel<false, true, false, false>)
+                                  : (u ? bounce_flat_fused_kernel<false, false, false, true> : bounce_flat_fused_kernel<false, false, false, false>);
     const int grid = persistent_grid(kernel, smem, sm_count);
     cudaError_t e = launch_pdl(kernel, grid, smem, s, a, launch_pairs(a));
     if (e != cudaSuccess) note_launch_error("fused first bounce kernel launch", e, smem, grid);
-    return true;
 }
 
-// Flat scenes with specular materials: one launch serves the three queues of a bounce (not the last).
-bool launch_bounce_merged(const PassArgs& a, int bounce, int sm_count, cudaStream_t s) {
-    const bool first = bounce == 0, last = bounce + 1 >= a.max_depth;
-    if (!all_staged(a) || last || !(a.kind_mask & 6u)) return false;
+bool launch_bounce_flat(const PassArgs& a, int bounce, int sm_count, cudaStream_t s) {
+    if (!(a.kind_mask & 7u)) return false; // no surface a path goes on from
     const size_t smem = path_smem_bytes(a);
+    const bool first = bounce == 0;
     void (*kernel)(PassArgs, int, FlatPairsU);
-    if (a.flat_uniform)
-        kernel = a.fold_last ? (first ? bounce_flat_all_kernel<true, true, true> : bounce_flat_all_kernel<false, true, true>)
-                             : (first ? bounce_flat_all_kernel<true, false, true> : bounce_flat_all_kernel<false, false, true>);
-    else
-        kernel = a.fold_last ? (first ? bounce_flat_all_kernel<true, true> : bounce_flat_all_kernel<false, true>)
-                             : (first ? bounce_flat_all_kernel<true> : bounce_flat_all_kernel<false>);
+    if (a.fold_last) kernel = a.flat_uniform ? flat_bounce_kernel<true, true>(a, first) : flat_bounce_kernel<true, false>(a, first);
+    else kernel = a.flat_uniform ? flat_bounce_kernel<false, true>(a, first) : flat_bounce_kernel<false, false>(a, first);
     const int grid = persistent_grid(kernel, smem, sm_count);
     cudaError_t e = launch_pdl(kernel, grid, smem, s, a, bounce, launch_pairs(a));
-    if (e != cudaSuccess) note_launch_error("merged bounce kernel launch", e, smem, grid);
+    if (e != cudaSuccess) note_launch_error("flat bounce kernel launch", e, smem, grid);
     return true;
 }
 
 bool launch_bounce(const PassArgs& a, int bounce, int kind, int sm_count, cudaStream_t s) {
     const bool last = bounce + 1 >= a.max_depth;
     if (last && kind != Q_DIFFUSE) return false; // nothing to do: no launch
-    const bool all = all_staged(a);
-    const size_t smem = all ? path_smem_bytes(a) : 0; // tree scenes only shade here: no scene staging
     switch (kind) {
-    case Q_DIFFUSE:
-        if (all) launch_bounce_fl<Q_DIFFUSE, true>(a, bounce, smem, sm_count, s);
-        else launch_bounce_fl<Q_DIFFUSE, false>(a, bounce, smem, sm_count, s);
-        break;
-    case Q_MIRROR:
-        if (all) launch_bounce_fl<Q_MIRROR, true>(a, bounce, smem, sm_count, s);
-        else launch_bounce_fl<Q_MIRROR, false>(a, bounce, smem, sm_count, s);
-        break;
-    default:
-        if (all) launch_bounce_fl<Q_GLASS, true>(a, bounce, smem, sm_count, s);
-        else launch_bounce_fl<Q_GLASS, false>(a, bounce, smem, sm_count, s);
-        break;
+    case Q_DIFFUSE: launch_bounce_fl<Q_DIFFUSE>(a, bounce, sm_count, s); break;
+    case Q_MIRROR: launch_bounce_fl<Q_MIRROR>(a, bounce, sm_count, s); break;
+    default: launch_bounce_fl<Q_GLASS>(a, bounce, sm_count, s); break;
     }
     return true;
 }
@@ -2840,8 +2531,7 @@ template <bool ANY> static void (*cast_tree_kernel(const PassArgs& a))(PassArgs,
     if (a.walk == 5) return a.trace_occ == 4 ? cast_kernel<false, 5, ANY, 4> : cast_kernel<false, 5, ANY, 3>;
     if (a.walk == 3) return a.trace_occ == 4 ? cast_kernel<false, 3, ANY, 4> : cast_kernel<false, 3, ANY, 3>;
     if (a.walk == 2) return a.coop_leaf ? cast_kernel<true, 2, ANY> : cast_kernel<false, 2, ANY>;
-    if (a.walk == 1) return a.coop_leaf ? (a.trace_occ == 4 ? cast_kernel<true, 1, ANY, 4> : cast_kernel<true, 1, ANY, 3>) : cast_kernel<false, 1, ANY>;
-    return a.coop_leaf ? cast_kernel<true, 0, ANY> : cast_kernel<false, 0, ANY>;
+    return a.coop_leaf ? (a.trace_occ == 4 ? cast_kernel<true, 1, ANY, 4> : cast_kernel<true, 1, ANY, 3>) : cast_kernel<false, 1, ANY>;
 }
 
 void launch_cast(const PassArgs& a, const CastArgs& c, bool any, int sm_count, cudaStream_t s) {

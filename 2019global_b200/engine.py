@@ -337,7 +337,7 @@ class RayTracer:
                                                         C.c_void_p(d_t), C.c_void_p(d_normals), C.c_void_p(stream)))
 
     def tune(self, key, value=None):
-        """g19_tune: set one tuning knob ("lanes", "no_merge", ...); value None = back to the default."""
+        """g19_tune: set one tuning knob ("lanes", "walk", ...); value None = back to the default."""
         v = None if value is None else str(value).encode()
         self._check(self._L.g19_tune(self.h, key.encode(), v))
 

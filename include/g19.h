@@ -344,8 +344,8 @@ int g19_frame_read(g19_ctx* ctx, g19_frame* frame, uint8_t* rgb888_out, float* r
 int g19_frame_timeouts(g19_ctx* ctx, g19_frame* frame, unsigned* out);
 int g19_frame_status(g19_ctx* ctx, g19_frame* frame, void* stream);
 
-/* Tuning knobs (DESIGN.md section 9): "lanes", "pass_slots", "no_merge", "leaf_max", "refill", "coop_leaf",
- * "walk_steps", "leaf_batch", "raygen_occ", "tree_build", "debug_tree". g19_create reads them ONCE from the
+/* Tuning knobs (DESIGN.md section 9): "lanes", "pass_slots", "leaf_max", "refill", "coop_leaf", "walk_steps",
+ * "leaf_batch", "walk", "tree_build", "debug_tree", ... g19_create reads them ONCE from the
  * environment (G19_LANES, ...); this call changes one afterwards (value NULL = back to the default). Nothing
  * on the render path reads the environment. No counterpart in the reference (it has no knobs, SURVEY.md 5). */
 int g19_tune(g19_ctx* ctx, const char* key, const char* value);

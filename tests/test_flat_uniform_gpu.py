@@ -1,10 +1,9 @@
 """Flat scenes whose primitive pairs fit the flat bounce kernels' FlatPairsU launch parameter (tune flat_uniform, default on) trace
 through pair loops unrolled to that capacity, with the coefficients as constant-bank operands, instead of the loops over
 the pairs staged in shared memory. Same operations in the same order per lane, so every frame must be bit-identical to
-the shared-memory form, with the same segment counts: on the Cornell boxes (diffuse-only; mirror / glass, merged and one
-launch per material queue), on flat scenes just under and just over the capacity (8 parallelogram pairs, 8 triangle
-pairs, 4 sphere pairs: the larger scene keeps the shared-memory loops either way), and on odd, even and empty kind
-groups."""
+the shared-memory form, with the same segment counts: on the Cornell boxes (diffuse-only; mirror / glass), on flat
+scenes just under and just over the capacity (8 parallelogram pairs, 8 triangle pairs, 4 sphere pairs: the larger scene
+keeps the shared-memory loops either way), and on odd, even and empty kind groups."""
 import numpy as np
 import pytest
 
@@ -39,11 +38,11 @@ def test_cornell_bit_identical(g19, abi, depth, spp, spp_pass):
 
 
 @pytest.mark.parametrize("depth", [1, 2, 5, 8])
-@pytest.mark.parametrize("no_merge", [None, "1"])
-def test_cornell_glass_bit_identical(g19, abi, depth, no_merge):
+@pytest.mark.parametrize("spp_pass", [2, 5])  # three passes of 2, 2 and 1 samples / one pass
+def test_cornell_glass_bit_identical(g19, abi, depth, spp_pass):
     w, h = 150, 97
     sc, cam, light = g19.Octree.builtin(abi.SCENE_CORNELL_GLASS, w=w, h=h)
-    _same(g19, abi, sc, cam, light, w, h, tune=(("no_merge", no_merge),), spp=5, max_depth=depth, seed=3, spp_per_pass=2)
+    _same(g19, abi, sc, cam, light, w, h, spp=5, max_depth=depth, seed=3, spp_per_pass=spp_pass)
 
 
 def _scene(g19, abi, n_quads, n_tris, n_spheres, seed=4):

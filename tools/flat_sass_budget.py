@@ -5,9 +5,9 @@
 Compiles DIR/2019global_b200/csrc/path_kernels.cu (default: this checkout) with the build's flags (build.py) into a
 cubin, or reads --cubin, disassembles it with nvdisasm's inlining line info, and prints for
 
-    bounce_flat_fused_kernel<false, false, false>      camera segment + first vertex (bounce 0)
-    bounce_flat_kernel<1, false, false, false, 3, false>  the middle bounces
-    bounce_flat_kernel<1, false, false, false, 3, true>   the bounce before the last, which shades the last vertex (FOLD)
+    bounce_flat_fused_kernel<false, false, false>  camera segment + first vertex (bounce 0)
+    bounce_flat_kernel<false>                      the middle bounces
+    bounce_flat_kernel<true>                       the bounce before the last, which shades the last vertex (FOLD)
 
 the registers and spill bytes (ptxas), and the static instructions of the vertex loop (the loop over queue entries in
 bounce_flat_body) split by the innermost project function they come from. The primitive-pair code is counted per call of
@@ -30,8 +30,8 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CUDA = "/usr/local/cuda/bin/"
 C2_KERNELS = [
     ("fused (bounce 0)", r"bounce_flat_fused_kernel<false, false, false(, %s)?>"),
-    ("plain (middle bounces)", r"bounce_flat_kernel<1, false, false, false, 3, false(, %s)?>"),
-    ("FOLD (bounce before the last)", r"bounce_flat_kernel<1, false, false, false, 3, true(, %s)?>"),
+    ("plain (middle bounces)", r"bounce_flat_kernel<false, %s>"),
+    ("FOLD (bounce before the last)", r"bounce_flat_kernel<true, %s>"),
 ]
 # pair code: planar pair functions / sphere pair functions (the parent's sphere loop body lived in trace_flat itself)
 PLANAR = {"plane_pairs", "plane_pairs_u", "plane_pair", "plane_origin2", "plane_uvt2", "plane_inside"}
