@@ -70,6 +70,11 @@ class Params(C.Structure):
                 ("spp_per_pass", C.c_int32), ("profile", C.c_int32), ("pixels_per_pass", C.c_int32)]
 
 
+class Adaptive(C.Structure):
+    """g19_adaptive: a tile stops once its error is <= noise_target; every owned pixel first takes min_spp samples."""
+    _fields_ = [("noise_target", C.c_float), ("min_spp", C.c_int32)]
+
+
 class Stats(C.Structure):
     _fields_ = [("samples", C.c_uint64), ("extend_segments", C.c_uint64), ("shadow_segments", C.c_uint64),
                 ("kernel_launches", C.c_uint64), ("render_ms", C.c_double), ("class_ms", C.c_double * 8),

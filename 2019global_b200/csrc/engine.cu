@@ -81,7 +81,7 @@ struct g19_ctx {
     DevBuf ids_l, points_l, normals_l, rgb_l, colour_l, counters;
     DevBuf heavy; // REF mode: heavy-ray lists, one set per band in flight (RefHeavyD)
     // frame buffers for the host-pointer entry point
-    DevBuf rgb_f, ids_f, rad_f;
+    DevBuf rgb_f, ids_f, rad_f, var_f, spp_f; // (variance and sample counts: g19_render_adaptive)
     PathWork work;
     // ray queries (g19_cast_rays*): their own state, no render buffer
     PathCastWork cast;
@@ -612,7 +612,7 @@ void g19_destroy(g19_ctx* ctx) {
     cudaDeviceSynchronize();
     for (DevBuf* b : {&ctx->heavy, &ctx->ref_nodes, &ctx->ref_ents, &ctx->ref_entities, &ctx->ref_tris, &ctx->ids_l, &ctx->points_l,
                       &ctx->normals_l, &ctx->rgb_l, &ctx->colour_l, &ctx->counters, &ctx->rgb_f, &ctx->ids_f,
-                      &ctx->rad_f, &ctx->cast_io})
+                      &ctx->rad_f, &ctx->var_f, &ctx->spp_f, &ctx->cast_io})
         b->release();
     path_release(ctx->path, ctx->work);
     ctx->cast.counters.release();
@@ -666,6 +666,28 @@ int g19_upload_scene(g19_ctx* ctx, const g19_scene* scene) {
     return G19_OK;
 }
 
+// What path_render / path_render_adaptive get from the context and the call.
+static PathRenderArgs path_args(g19_ctx* ctx, const g19_camera* cam, const double light[3], const g19_params* p, const TileMap& map,
+                                cudaStream_t s) {
+    PathRenderArgs a;
+    a.tune = ctx->tune;
+    a.cam = make_camera(*cam, light, p->width);
+    a.params = *p;
+    a.map = map;
+    a.d_rgb = nullptr;
+    a.d_rad = nullptr;
+    a.d_ids = nullptr;
+    a.t_rgb = nullptr;
+    a.t_rad = nullptr;
+    a.stream = s;
+    a.sm_count = ctx->sm_count;
+    a.cancel = &ctx->cancel;
+    a.progress_milli = &ctx->progress_milli;
+    a.cls0 = ctx->cls0;
+    a.cls1 = ctx->cls1;
+    return a;
+}
+
 static int render_any(g19_ctx* ctx, const g19_camera* cam, const double light[3], const g19_params* p,
                       uint8_t* d_rgb, int32_t* d_ids, float* d_rad, uint8_t* t_rgb, int32_t* t_ids, float* t_rad,
                       void* stream, g19_frame* frame = nullptr) {
@@ -683,23 +705,13 @@ static int render_any(g19_ctx* ctx, const g19_camera* cam, const double light[3]
         if (frame && map.n_local_pix == 0) launch_frame_signal(frame->flags, s); // no tiles: still counted
         else rc = render_ref(ctx, cam, light, p, map, d_rgb, d_ids, d_rad, t_rgb, t_ids, t_rad, s, frame);
     } else {
-        RefCamera rc64 = make_camera(*cam, light, p->width);
-        PathRenderArgs a;
-        a.tune = ctx->tune;
-        a.cam = rc64;
-        a.params = *p;
-        a.map = map;
+        PathRenderArgs a = path_args(ctx, cam, light, p, map, s);
+        const RefCamera& rc64 = a.cam;
         a.d_rgb = d_rgb;
         a.d_rad = d_rad;
         a.d_ids = d_ids;
         a.t_rgb = t_rgb;
         a.t_rad = t_rad;
-        a.stream = s;
-        a.sm_count = ctx->sm_count;
-        a.cancel = &ctx->cancel;
-        a.progress_milli = &ctx->progress_milli;
-        a.cls0 = ctx->cls0;
-        a.cls1 = ctx->cls1;
         if (ctx->hook.fn) {
             a.on_pass = ctx->hook.fn;
             a.pass_user = ctx->hook.user;
@@ -821,6 +833,82 @@ int g19_render(g19_ctx* ctx, const g19_camera* cam, const double light[3], const
     if (rad) G19_CUDA(ctx, cudaMemcpyAsync(rad, ctx->rad_f.p, npx * 12, cudaMemcpyDeviceToHost, s));
     G19_CUDA(ctx, cudaStreamSynchronize(s));
     return rc;
+}
+
+// ---- adaptive sampling (PATH mode) -------------------------------------------------------------
+static int check_adaptive(g19_ctx* ctx, const g19_camera* cam, const g19_params* p, const g19_adaptive* ad) {
+    if (!ctx) return G19_ERR_INVALID;
+    const char* bad = nullptr;
+    if (!p || !ad) bad = "params and adaptive are required";
+    else if (p->mode != G19_MODE_PATH) bad = "only G19_MODE_PATH renders adaptively";
+    else if (!(ad->noise_target > 0.0f) || !std::isfinite(ad->noise_target)) bad = "noise_target must be finite and > 0";
+    else if (ad->min_spp < 2 || ad->min_spp > p->spp) bad = "min_spp must be in [2, spp]";
+    else if (p->max_depth < 1) bad = "max_depth must be >= 1";
+    if (bad) {
+        ctx->err = std::string("g19_render_adaptive: ") + bad;
+        return G19_ERR_INVALID;
+    }
+    return check_params(ctx, cam, p);
+}
+
+int g19_render_adaptive_device(g19_ctx* ctx, const g19_camera* cam, const double light[3], const g19_params* p,
+                               const g19_adaptive* ad, uint8_t* d_rgb, float* d_rad, float* d_var, int32_t* d_spp, void* stream) {
+    int rc = check_adaptive(ctx, cam, p, ad);
+    if (rc != G19_OK) return rc;
+    G19_CUDA(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    ctx->cancel.store(0);
+    ctx->progress_milli.store(0);
+    ctx->stats = g19_stats{};
+    ctx->cast.counts_pending = false; // (the statistics now belong to this render)
+    const TileMap map = make_tile_map(p->width, p->height, p->rank, p->world);
+    G19_CUDA(ctx, cudaEventRecord(ctx->ev0, s));
+    PathRenderArgs a = path_args(ctx, cam, light, p, map, s);
+    a.d_rgb = d_rgb;
+    a.d_rad = d_rad;
+    std::string perr;
+    rc = path_render_adaptive(ctx->path, ctx->work, a, ad->noise_target, ad->min_spp, d_var, d_spp, ctx->stats, perr);
+    if (rc != G19_OK && rc != G19_ERR_CANCELLED) {
+        ctx->err = perr;
+        return rc;
+    }
+    G19_CUDA(ctx, cudaEventRecord(ctx->ev1, s));
+    ctx->stats_pending = true;
+    if (rc == G19_OK) ctx->progress_milli.store(1000);
+    return rc;
+}
+
+int g19_render_adaptive(g19_ctx* ctx, const g19_camera* cam, const double light[3], const g19_params* p, const g19_adaptive* ad,
+                        uint8_t* rgb, float* rad, float* var, int32_t* spp) {
+    int rc = check_adaptive(ctx, cam, p, ad);
+    if (rc != G19_OK) return rc;
+    G19_CUDA(ctx, cudaSetDevice(ctx->device));
+    const size_t npx = size_t(p->width) * size_t(p->height);
+    if (npx == 0) return G19_OK;
+    cudaStream_t s = ctx->stream;
+    if (rgb) G19_CUDA(ctx, ctx->rgb_f.ensure(npx * 3));
+    if (rad) G19_CUDA(ctx, ctx->rad_f.ensure(npx * 3 * sizeof(float)));
+    if (var) G19_CUDA(ctx, ctx->var_f.ensure(npx * sizeof(float)));
+    if (spp) G19_CUDA(ctx, ctx->spp_f.ensure(npx * sizeof(int32_t)));
+    // pixels owned by other ranks stay as the caller left them (as g19_render)
+    if (p->world > 1) {
+        if (rgb) G19_CUDA(ctx, cudaMemcpyAsync(ctx->rgb_f.p, rgb, npx * 3, cudaMemcpyHostToDevice, s));
+        if (rad) G19_CUDA(ctx, cudaMemcpyAsync(ctx->rad_f.p, rad, npx * 12, cudaMemcpyHostToDevice, s));
+        if (var) G19_CUDA(ctx, cudaMemcpyAsync(ctx->var_f.p, var, npx * 4, cudaMemcpyHostToDevice, s));
+        if (spp) G19_CUDA(ctx, cudaMemcpyAsync(ctx->spp_f.p, spp, npx * 4, cudaMemcpyHostToDevice, s));
+    }
+    rc = g19_render_adaptive_device(ctx, cam, light, p, ad, rgb ? ctx->rgb_f.as<uint8_t>() : nullptr, rad ? ctx->rad_f.as<float>() : nullptr,
+                                    var ? ctx->var_f.as<float>() : nullptr, spp ? ctx->spp_f.as<int32_t>() : nullptr, s);
+    if (rc != G19_OK) {
+        if (rc == G19_ERR_CANCELLED) G19_CUDA(ctx, cudaStreamSynchronize(s));
+        return rc;
+    }
+    if (rgb) G19_CUDA(ctx, cudaMemcpyAsync(rgb, ctx->rgb_f.p, npx * 3, cudaMemcpyDeviceToHost, s));
+    if (rad) G19_CUDA(ctx, cudaMemcpyAsync(rad, ctx->rad_f.p, npx * 12, cudaMemcpyDeviceToHost, s));
+    if (var) G19_CUDA(ctx, cudaMemcpyAsync(var, ctx->var_f.p, npx * 4, cudaMemcpyDeviceToHost, s));
+    if (spp) G19_CUDA(ctx, cudaMemcpyAsync(spp, ctx->spp_f.p, npx * 4, cudaMemcpyDeviceToHost, s));
+    G19_CUDA(ctx, cudaStreamSynchronize(s));
+    return G19_OK;
 }
 
 // ---- shared frame (multi-GPU, fused gather) ---------------------------------------------------

@@ -785,6 +785,12 @@ void path_release(PathSceneBuffers& b, PathWork& w) {
                            &w.rad_l, &w.rgb_l, &w.iota})
         d->release();
     w.iota_n = 0;
+    w.tile_n.release();
+    w.tile_flag.release();
+    w.tile_list.release();
+    if (w.tile_h) cudaFreeHost(w.tile_h);
+    w.tile_h = nullptr;
+    w.tile_h_n = 0;
     w.ray_hint_d.release();
     if (w.ray_hint_h) cudaFreeHost(w.ray_hint_h);
     w.ray_hint_h = nullptr;
@@ -876,16 +882,35 @@ PassArgs path_pass_setup(const PathSceneBuffers& b, const PathTuning& tune, bool
     return pa;
 }
 
-int path_render(PathSceneBuffers& b, PathWork& w, const PathRenderArgs& a, g19_stats& stats, std::string& err) {
+#define PATH_CUDA(call)                                                        \
+    do {                                                                       \
+        cudaError_t e__ = (call);                                              \
+        if (e__ != cudaSuccess) {                                              \
+            err = std::string(#call) + ": " + cudaGetErrorString(e__);         \
+            return G19_ERR_CUDA;                                               \
+        }                                                                      \
+    } while (0)
+
+namespace {
+
+// What the passes of one frame share (path_render, path_render_adaptive): frame_begin sets it up, frame_pass enqueues one
+// pass, frame_join puts the caller's stream behind every lane.
+struct Frame {
+    PassArgs pa0;                        // the frame's arguments; per-lane copies below
+    PassArgs lanes[kMaxLanes];
+    cudaStream_t lane_stream[kMaxLanes];
+    bool fused = false;                  // flat scenes trace the camera segment in the first bounce's launch
+    size_t window = 0;                   // local pixels (or tile-list positions) per pass, whole tiles
+    int spp_pass = 0;                    // samples per pass
+    size_t P = 0;                        // path slots per pass
+    int n_lanes = 1, first_side = 1, parity = 0;
+    int prev_lane = -1;                  // lane of the previous pass
+    size_t pass_index = 0;
+    unsigned long long key = 0;          // the frame's shape (PathWork::overlap_key)
+};
+
+PassArgs frame_args(const PathSceneBuffers& b, const PathRenderArgs& a) {
     const g19_params& p = a.params;
-    if (p.spp < 1 || p.max_depth < 0 || p.max_depth > kMaxPathDepth || (p.max_depth == 0 && !a.ids_l)) {
-        err = "PATH mode needs spp >= 1 and 0 <= max_depth <= 64";
-        return G19_ERR_INVALID;
-    }
-    cudaStream_t s = a.stream;
-    const size_t npix = size_t(a.map.n_local_pix);
-    if (npix == 0) return G19_OK;
-    path_clear_launch_error();
     PassArgs pa0 = path_pass_setup(b, a.tune, p.profile != 0);
     for (int k = 0; k < 3; ++k) {
         pa0.cam.pos[k] = float(a.cam.pos[k]);
@@ -896,22 +921,17 @@ int path_render(PathSceneBuffers& b, PathWork& w, const PathRenderArgs& a, g19_s
     pa0.map = a.map;
     pa0.seed = p.seed;
     pa0.max_depth = p.max_depth;
-    const bool fused = path_scene_is_flat(pa0); // flat scenes trace inside the bounce kernels
-    // primary-hit AOV: the un-jittered ray of every pixel (the reference's ray) through this engine's structures
-    if (a.ids_l) {
-        launch_primary(pa0, a.ids_l, a.points_l, a.normals_l, a.sm_count, s);
-        stats.class_launches[G19_K_EXTEND] += 1;
-        stats.kernel_launches += 1;
-    }
-    if (p.max_depth == 0) { // depth-0 slice: nothing to bounce; the caller shades the primary hits (engine.cu)
-        if (const char* le = path_launch_error()) {
-            err = le;
-            path_clear_launch_error();
-            return G19_ERR_CUDA;
-        }
-        return G19_OK;
-    }
+    return pa0;
+}
 
+// Pass size, lanes and their buffers, the frame's statistics block and accum (accum_planes planes, zeroed), and the side
+// lanes started behind the caller's stream -- or, for a frame behind a frame of the same shape with overlap_frames,
+// behind their own previous passes (allow_overlap).
+int frame_begin(PathSceneBuffers& b, PathWork& w, const PathRenderArgs& a, Frame& f, int accum_planes, bool allow_overlap,
+                std::string& err) {
+    const g19_params& p = a.params;
+    cudaStream_t s = a.stream;
+    const size_t npix = size_t(a.map.n_local_pix);
     // Pass size. Flat scenes keep dense vertex records in their queues, so a bounce streams exactly
     // the live vertices whatever the pass size: bigger passes only amortise launch tails (measured on
     // B200, ms per 1080p x 64 spp frame at 2 / 4 / 8 / 16 M slots, one pass in flight: Cornell depth 5
@@ -942,18 +962,14 @@ int path_render(PathSceneBuffers& b, PathWork& w, const PathRenderArgs& a, g19_s
         err = "pass too large";
         return G19_ERR_LIMIT;
     }
-#define PATH_CUDA(call)                                                        \
-    do {                                                                       \
-        cudaError_t e__ = (call);                                              \
-        if (e__ != cudaSuccess) {                                              \
-            err = std::string(#call) + ": " + cudaGetErrorString(e__);         \
-            return G19_ERR_CUDA;                                               \
-        }                                                                      \
-    } while (0)
+    f.window = window;
+    f.spp_pass = spp_pass;
+    f.P = P;
     // passes of this frame, and how many are kept in flight (see PathWork)
     const size_t n_windows = (npix + window - 1) / window;
     const size_t n_passes = n_windows * size_t((p.spp + spp_pass - 1) / spp_pass);
     const int n_lanes = (p.profile || a.on_pass) ? 1 : int(std::min<size_t>(size_t(a.tune.lanes), n_passes)); // profiling and progressive refresh: one at a time
+    f.n_lanes = n_lanes;
     if (n_lanes > 1 && !w.ev_fork) PATH_CUDA(cudaEventCreateWithFlags(&w.ev_fork, cudaEventDisableTiming));
     for (int i = 0; i < n_lanes; ++i) {
         if ((i > 0 || n_lanes > 1) && !w.side[i]) PATH_CUDA(cudaStreamCreateWithFlags(&w.side[i], cudaStreamNonBlocking));
@@ -967,59 +983,60 @@ int path_render(PathSceneBuffers& b, PathWork& w, const PathRenderArgs& a, g19_s
     const size_t bytes_before = w.totals.bytes + w.accum.bytes + w.rad_l.bytes + w.rgb_l.bytes + w.iota.bytes + w.ray_hint_d.bytes;
     size_t lane_bytes_before = 0;
     for (const PathLane& l : w.lane) lane_bytes_before += l.capacity + l.L.bytes + l.recs.bytes + l.rays.bytes + l.queues.bytes + l.counts.bytes + l.rkeys.bytes;
-    const unsigned long long this_key = ((b.upload_serial + 1) << 44) ^ (static_cast<unsigned long long>(P) << 12) ^
-                                        (static_cast<unsigned long long>(n_lanes) << 8) ^ static_cast<unsigned long long>(p.max_depth) ^
-                                        (static_cast<unsigned long long>(npix) << 20) ^ reinterpret_cast<unsigned long long>(s);
+    f.key = ((b.upload_serial + 1) << 44) ^ (static_cast<unsigned long long>(P) << 12) ^
+            (static_cast<unsigned long long>(n_lanes) << 8) ^ static_cast<unsigned long long>(p.max_depth) ^
+            (static_cast<unsigned long long>(npix) << 20) ^ reinterpret_cast<unsigned long long>(s);
     PATH_CUDA(w.totals.ensure(2 * 10 * sizeof(unsigned long long)));
-    PATH_CUDA(w.accum.ensure(npix * 3 * sizeof(float)));
+    PATH_CUDA(w.accum.ensure(npix * accum_planes * sizeof(float)));
     PATH_CUDA(w.rad_l.ensure(npix * 3 * sizeof(float)));
     PATH_CUDA(w.rgb_l.ensure(npix * 3));
     for (cudaEvent_t& e : w.ev_start)
         if (!e) PATH_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    const bool may_overlap = a.tune.overlap_frames && n_lanes > 1 && w.overlap_key == this_key && !p.profile && !a.on_pass;
+    const bool may_overlap = allow_overlap && a.tune.overlap_frames && n_lanes > 1 && w.overlap_key == f.key && !p.profile && !a.on_pass;
     w.overlap_key = 0; // set again once this frame is enqueued whole
     const int parity = int(w.frame_serial & 1ull);
+    f.parity = parity;
     unsigned long long* const totals2 = static_cast<unsigned long long*>(w.totals.p);
     if (!may_overlap) PATH_CUDA(cudaMemsetAsync(totals2, 0, 2 * 10 * sizeof(unsigned long long), s));
     else PATH_CUDA(cudaMemsetAsync(totals2 + 10 * (parity ^ 1), 0, 10 * sizeof(unsigned long long), s)); // the NEXT frame's block
-    PATH_CUDA(cudaMemsetAsync(w.accum.p, 0, npix * 3 * sizeof(float), s));
+    PATH_CUDA(cudaMemsetAsync(w.accum.p, 0, npix * accum_planes * sizeof(float), s));
     if (p.profile && !w.events) {
         w.n_events = 65536;
         w.events = new cudaEvent_t[w.n_events];
         for (int i = 0; i < w.n_events; ++i) PATH_CUDA(cudaEventCreate(&w.events[i]));
     }
     w.used_events = 0;
+    PassArgs& pa0 = f.pa0;
     pa0.totals = totals2 + 10 * parity;
     w.totals_parity = parity;
     pa0.accum = static_cast<float*>(w.accum.p);
 
     // per-lane buffers
-    PassArgs lanes[kMaxLanes];
-    cudaStream_t lane_stream[kMaxLanes];
+    const bool fused = f.fused;
     for (int i = 0; i < kMaxLanes; ++i) {
-        lanes[i] = pa0;
-        lane_stream[i] = s;
+        f.lanes[i] = pa0;
+        f.lane_stream[i] = s;
     }
     // Several lanes: with overlap_frames ALL of them run on streams of their own (the caller's stream only zeroes, joins and
     // resolves), so that the next frame's passes can follow this frame's on every lane; otherwise lane 0 is the caller's stream.
-    const int first_side = (n_lanes > 1 && a.tune.overlap_frames) ? 0 : 1;
-    for (int i = first_side; i < n_lanes; ++i) lane_stream[i] = w.side[i];
+    f.first_side = (n_lanes > 1 && a.tune.overlap_frames) ? 0 : 1;
+    for (int i = f.first_side; i < n_lanes; ++i) f.lane_stream[i] = w.side[i];
     for (int li = 0; li < n_lanes; ++li) {
         PathLane& l = w.lane[li];
-        PassArgs& pa = lanes[li];
+        PassArgs& pa = f.lanes[li];
         if (P > l.capacity) {
             PATH_CUDA(l.L.ensure(P * 4 * sizeof(float))); // flat scenes: float4 per slot; tree scenes: three planes
             l.capacity = P;
-            PATH_CUDA(cudaMemsetAsync(l.L.p, 0, P * 4 * sizeof(float), lane_stream[li]));
+            PATH_CUDA(cudaMemsetAsync(l.L.p, 0, P * 4 * sizeof(float), f.lane_stream[li]));
             l.L_written_whole = false;
         }
         // tree scenes ADD to zeroed planes (accumulate clears what it read); flat scenes store every slot
         // (a lane's own buffers are cleared on the lane's own stream: in order with its passes, whatever the caller's stream is at)
-        if (!fused && l.L_written_whole) PATH_CUDA(cudaMemsetAsync(l.L.p, 0, l.capacity * 4 * sizeof(float), lane_stream[li]));
+        if (!fused && l.L_written_whole) PATH_CUDA(cudaMemsetAsync(l.L.p, 0, l.capacity * 4 * sizeof(float), f.lane_stream[li]));
         l.L_written_whole = fused;
         const size_t plane = l.capacity;
         PATH_CUDA(l.counts.ensure((kMaxPathDepth + 1) * 5 * sizeof(uint32_t)));
-        PATH_CUDA(cudaMemsetAsync(l.counts.p, 0, (kMaxPathDepth + 1) * 5 * sizeof(uint32_t), lane_stream[li]));
+        PATH_CUDA(cudaMemsetAsync(l.counts.p, 0, (kMaxPathDepth + 1) * 5 * sizeof(uint32_t), f.lane_stream[li]));
         pa.L = static_cast<float*>(l.L.p);
         pa.plane = plane;
         pa.queue_cap = plane + kQueueSlack;
@@ -1093,99 +1110,175 @@ int path_render(PathSceneBuffers& b, PathWork& w, const PathRenderArgs& a, g19_s
             if (overlap) {
                 // a frame behind a frame of the same shape: the side lanes go on behind their own passes; all they need from the
                 // caller's stream is last frame's start (their statistics block was zeroed there)
-                for (int i = first_side; i < n_lanes; ++i) PATH_CUDA(cudaStreamWaitEvent(w.side[i], w.ev_start[parity ^ 1], 0));
+                for (int i = f.first_side; i < n_lanes; ++i) PATH_CUDA(cudaStreamWaitEvent(w.side[i], w.ev_start[parity ^ 1], 0));
             } else { // the other lanes start after everything enqueued so far on the caller's stream
                 PATH_CUDA(cudaEventRecord(w.ev_fork, s));
-                for (int i = first_side; i < n_lanes; ++i) PATH_CUDA(cudaStreamWaitEvent(w.side[i], w.ev_fork, 0));
+                for (int i = f.first_side; i < n_lanes; ++i) PATH_CUDA(cudaStreamWaitEvent(w.side[i], w.ev_fork, 0));
             }
         }
     }
+    return G19_OK;
+}
+
+// One pass: samples [base, base + batch_spp) of window positions [pix0, pix0 + pix_count) -- the camera segment, the
+// bounces (tree scenes: with their ray sorts and walks), then accumulate, behind the previous pass's accumulate whichever
+// lane that ran on, so that the per-pixel sums are taken in sample order.
+int frame_pass(const PathSceneBuffers& b, PathWork& w, const PathRenderArgs& a, Frame& f, ClassClock& clk, int base, int batch_spp,
+               size_t pix0, size_t pix_count, g19_stats& stats, std::string& err) {
+    const g19_params& p = a.params;
+    const bool fused = f.fused;
+    const int n_lanes = f.n_lanes;
+    const int li = int(f.pass_index++ % size_t(n_lanes));
+    PassArgs& pa = f.lanes[li];
+    cudaStream_t ls = f.lane_stream[li];
+    clk.s = ls;
+    pa.sample_base = base;
+    pa.spp_pass = batch_spp;
+    pa.pix_base = uint32_t(pix0);
+    pa.pix_count = uint32_t(pix_count);
+    pa.n_slots = uint32_t(size_t(pa.pix_count) * size_t(pa.spp_pass));
+    if (!fused) { // flat scenes trace the camera segment in the first bounce's launch
+        clk.begin();
+        launch_raygen_extend(pa, a.sm_count, ls);
+        clk.end(G19_K_EXTEND);
+        stats.class_launches[G19_K_EXTEND] += 1;
+    }
+    // flat scenes: the launch before the last shades the last vertex in place, so the last bounce has no launch
+    const int n_launch = fused && p.max_depth >= 2 ? p.max_depth - 1 : p.max_depth;
+    for (int bounce = 0; bounce < n_launch; ++bounce) {
+        clk.begin();
+        int n = 0;
+        if (fused) {
+            pa.fold_last = bounce == p.max_depth - 2 ? 1 : 0;
+            if (bounce == 0) {
+                launch_bounce_first_fused(pa, a.sm_count, ls);
+                ++n;
+            }
+            // (at bounce 0 with mirror / glass: the camera hits on those, which the fused launch queued)
+            if ((bounce > 0 || ((pa.kind_mask & 6u) && p.max_depth > 1)) && launch_bounce_flat(pa, bounce, a.sm_count, ls)) ++n;
+            clk.end(G19_K_SHADE);
+            stats.class_launches[G19_K_SHADE] += n;
+            continue;
+        }
+        // the first bounce's rays leave the camera rays' hit points in pixel order: coherent as they are
+        // ... and a queue that stayed short the last time is walked in a blink: not worth three more launches.
+        const size_t ray_cap = 2 * pa.plane + kQueueSlack;
+        size_t n_sort = 0;
+        if (pa.rkey && bounce > 0) {
+            const uint32_t hint = w.ray_hint_h[bounce]; // 0 = not known yet: the whole queue
+            n_sort = hint == 0 ? ray_cap : std::min(ray_cap, size_t(hint) + size_t(hint) / 8 + 65536);
+            if (hint != 0 && hint < (1u << 19)) n_sort = 0;
+        }
+        const bool sort_this = n_sort > 0;
+        PassArgs pb = pa;
+        pb.perm_n = uint32_t(n_sort);
+        if (!sort_this) pb.rkey = nullptr, pb.perm = nullptr;
+        if (sort_this) PATH_CUDA(cudaMemsetAsync(pa.rkey, 0xff, n_sort * sizeof(uint16_t), ls));
+        for (int kind = Q_DIFFUSE; kind <= Q_GLASS; ++kind) {
+            if (!b.has_bsdf[kind - 1]) continue; // no such material in the scene: queue is always empty
+            if (launch_bounce(pb, bounce, kind, a.sm_count, ls)) ++n;
+        }
+        if (n > 0) { // one walk over the rays this bounce's vertices produced
+            if (sort_this) {
+                PATH_CUDA(launch_ray_sort(w.lane[li].sort_tmp.p, w.lane[li].sort_tmp.bytes, pa.rkey, pa.rkey + ray_cap,
+                                          static_cast<const uint32_t*>(w.iota.p), static_cast<uint32_t*>(w.lane[li].perm.p), n_sort, ls));
+                n += 3; // histogram + two one-sweep passes
+            }
+            launch_trace(pb, bounce, a.sm_count, ls);
+            ++n;
+        }
+        clk.end(G19_K_SHADE);
+        stats.class_launches[G19_K_SHADE] += n;
+    }
+    // the per-pixel sums are taken in pass order whichever lane a pass ran on
+    if (n_lanes > 1 && f.prev_lane >= 0) PATH_CUDA(cudaStreamWaitEvent(ls, w.ev_acc[f.prev_lane], 0));
+    else if (n_lanes > 1 && ls != a.stream) PATH_CUDA(cudaStreamWaitEvent(ls, w.ev_start[f.parity], 0)); // the frame's first: behind the memset of accum
+    clk.begin();
+    launch_accumulate(pa, ls);
+    clk.end(G19_K_ACCUM);
+    stats.class_launches[G19_K_ACCUM] += 1;
+    if (n_lanes > 1) {
+        PATH_CUDA(cudaEventRecord(w.ev_acc[li], ls));
+        f.prev_lane = li;
+    }
+    return G19_OK;
+}
+
+// The caller's stream continues after the other lanes (and copies the ray-sort hints they raised).
+int frame_join(PathWork& w, const PathRenderArgs& a, Frame& f, ClassClock& clk, std::string& err) {
+    cudaStream_t s = a.stream;
+    for (int i = f.first_side; i < f.n_lanes; ++i) {
+        PATH_CUDA(cudaEventRecord(w.ev_join[i], w.side[i]));
+        PATH_CUDA(cudaStreamWaitEvent(s, w.ev_join[i], 0));
+    }
+    clk.s = s;
+    if (!f.fused && w.ray_hint_h && w.ray_hint_d.p && f.lanes[0].ray_hint)
+        PATH_CUDA(cudaMemcpyAsync(w.ray_hint_h, w.ray_hint_d.p, (kMaxPathDepth + 1) * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+    return G19_OK;
+}
+
+// A launch that failed during the frame: its lanes' radiance planes and queue lengths are dirty -- re-zero them before the
+// next render.
+int frame_launch_error(PathWork& w, std::string& err) {
+    const char* le = path_launch_error();
+    if (!le) return G19_OK;
+    err = le;
+    path_clear_launch_error();
+    cudaGetLastError();
+    for (PathLane& l : w.lane) l.capacity = 0;
+    return G19_ERR_CUDA;
+}
+
+uint64_t tile_pixels_in_frame(const TileMap& map, int lt) {
+    const int tile = lt * map.world + map.rank;
+    const int ty = tile / map.tiles_x, tx = tile % map.tiles_x;
+    return uint64_t(std::min(kTile, map.w - tx * kTile)) * uint64_t(std::min(kTile, map.h - ty * kTile));
+}
+
+} // namespace
+
+int path_render(PathSceneBuffers& b, PathWork& w, const PathRenderArgs& a, g19_stats& stats, std::string& err) {
+    const g19_params& p = a.params;
+    if (p.spp < 1 || p.max_depth < 0 || p.max_depth > kMaxPathDepth || (p.max_depth == 0 && !a.ids_l)) {
+        err = "PATH mode needs spp >= 1 and 0 <= max_depth <= 64";
+        return G19_ERR_INVALID;
+    }
+    cudaStream_t s = a.stream;
+    const size_t npix = size_t(a.map.n_local_pix);
+    if (npix == 0) return G19_OK;
+    path_clear_launch_error();
+    Frame f;
+    f.pa0 = frame_args(b, a);
+    f.fused = path_scene_is_flat(f.pa0); // flat scenes trace inside the bounce kernels
+    // primary-hit AOV: the un-jittered ray of every pixel (the reference's ray) through this engine's structures
+    if (a.ids_l) {
+        launch_primary(f.pa0, a.ids_l, a.points_l, a.normals_l, a.sm_count, s);
+        stats.class_launches[G19_K_EXTEND] += 1;
+        stats.kernel_launches += 1;
+    }
+    if (p.max_depth == 0) { // depth-0 slice: nothing to bounce; the caller shades the primary hits (engine.cu)
+        if (const char* le = path_launch_error()) {
+            err = le;
+            path_clear_launch_error();
+            return G19_ERR_CUDA;
+        }
+        return G19_OK;
+    }
+    int rc = frame_begin(b, w, a, f, 3, true, err);
+    if (rc != G19_OK) return rc;
+    const PassArgs& pa0 = f.pa0;
     ClassClock clk{w, s, p.profile != 0};
-    int rc = G19_OK;
     auto last_refresh = std::chrono::steady_clock::now();
-    size_t pass_index = 0;
-    int prev_lane = -1; // lane of the previous pass
     int batch_spp = 0;
-    for (int base = 0; base < p.spp; base += spp_pass) {
+    for (int base = 0; base < p.spp; base += f.spp_pass) {
         if (a.cancel && a.cancel->load()) { // RayTracer::stop(): honoured between passes
             rc = G19_ERR_CANCELLED;
             break;
         }
-        batch_spp = std::min(spp_pass, p.spp - base);
-        for (size_t pix0 = 0; pix0 < npix; pix0 += window, ++pass_index) { // the windows of this sample batch
-            const int li = int(pass_index % size_t(n_lanes));
-            PassArgs& pa = lanes[li];
-            cudaStream_t ls = lane_stream[li];
-            clk.s = ls;
-            pa.sample_base = base;
-            pa.spp_pass = batch_spp;
-            pa.pix_base = uint32_t(pix0);
-            pa.pix_count = uint32_t(std::min(window, npix - pix0));
-            pa.n_slots = uint32_t(size_t(pa.pix_count) * size_t(pa.spp_pass));
-            if (!fused) { // flat scenes trace the camera segment in the first bounce's launch
-                clk.begin();
-                launch_raygen_extend(pa, a.sm_count, ls);
-                clk.end(G19_K_EXTEND);
-                stats.class_launches[G19_K_EXTEND] += 1;
-            }
-            // flat scenes: the launch before the last shades the last vertex in place, so the last bounce has no launch
-            const int n_launch = fused && p.max_depth >= 2 ? p.max_depth - 1 : p.max_depth;
-            for (int bounce = 0; bounce < n_launch; ++bounce) {
-                clk.begin();
-                int n = 0;
-                if (fused) {
-                    pa.fold_last = bounce == p.max_depth - 2 ? 1 : 0;
-                    if (bounce == 0) {
-                        launch_bounce_first_fused(pa, a.sm_count, ls);
-                        ++n;
-                    }
-                    // (at bounce 0 with mirror / glass: the camera hits on those, which the fused launch queued)
-                    if ((bounce > 0 || ((pa.kind_mask & 6u) && p.max_depth > 1)) && launch_bounce_flat(pa, bounce, a.sm_count, ls)) ++n;
-                    clk.end(G19_K_SHADE);
-                    stats.class_launches[G19_K_SHADE] += n;
-                    continue;
-                }
-                // the first bounce's rays leave the camera rays' hit points in pixel order: coherent as they are
-                // ... and a queue that stayed short the last time is walked in a blink: not worth three more launches.
-                const size_t ray_cap = 2 * pa.plane + kQueueSlack;
-                size_t n_sort = 0;
-                if (pa.rkey && bounce > 0) {
-                    const uint32_t hint = w.ray_hint_h[bounce]; // 0 = not known yet: the whole queue
-                    n_sort = hint == 0 ? ray_cap : std::min(ray_cap, size_t(hint) + size_t(hint) / 8 + 65536);
-                    if (hint != 0 && hint < (1u << 19)) n_sort = 0;
-                }
-                const bool sort_this = n_sort > 0;
-                PassArgs pb = pa;
-                pb.perm_n = uint32_t(n_sort);
-                if (!sort_this) pb.rkey = nullptr, pb.perm = nullptr;
-                if (sort_this) PATH_CUDA(cudaMemsetAsync(pa.rkey, 0xff, n_sort * sizeof(uint16_t), ls));
-                for (int kind = Q_DIFFUSE; kind <= Q_GLASS; ++kind) {
-                    if (!b.has_bsdf[kind - 1]) continue; // no such material in the scene: queue is always empty
-                    if (launch_bounce(pb, bounce, kind, a.sm_count, ls)) ++n;
-                }
-                if (n > 0) { // one walk over the rays this bounce's vertices produced
-                    if (sort_this) {
-                        PATH_CUDA(launch_ray_sort(w.lane[li].sort_tmp.p, w.lane[li].sort_tmp.bytes, pa.rkey, pa.rkey + ray_cap,
-                                                  static_cast<const uint32_t*>(w.iota.p), static_cast<uint32_t*>(w.lane[li].perm.p), n_sort, ls));
-                        n += 3; // histogram + two one-sweep passes
-                    }
-                    launch_trace(pb, bounce, a.sm_count, ls);
-                    ++n;
-                }
-                clk.end(G19_K_SHADE);
-                stats.class_launches[G19_K_SHADE] += n;
-            }
-            // the per-pixel sums are taken in pass order whichever lane a pass ran on
-            if (n_lanes > 1 && prev_lane >= 0) PATH_CUDA(cudaStreamWaitEvent(ls, w.ev_acc[prev_lane], 0));
-            else if (n_lanes > 1 && ls != s) PATH_CUDA(cudaStreamWaitEvent(ls, w.ev_start[parity], 0)); // the frame's first: behind the memset of accum
-            clk.begin();
-            launch_accumulate(pa, ls);
-            clk.end(G19_K_ACCUM);
-            stats.class_launches[G19_K_ACCUM] += 1;
-            if (n_lanes > 1) {
-                PATH_CUDA(cudaEventRecord(w.ev_acc[li], ls));
-                prev_lane = li;
-            }
+        batch_spp = std::min(f.spp_pass, p.spp - base);
+        for (size_t pix0 = 0; pix0 < npix; pix0 += f.window) { // the windows of this sample batch
+            const int prc = frame_pass(b, w, a, f, clk, base, batch_spp, pix0, std::min(f.window, npix - pix0), stats, err);
+            if (prc != G19_OK) return prc;
         }
         stats.samples += uint64_t(batch_spp); // scaled by owned pixels below
         if (a.progress_milli) a.progress_milli->store(int(1000.0 * double(base + batch_spp) / double(p.spp)));
@@ -1206,13 +1299,8 @@ int path_render(PathSceneBuffers& b, PathWork& w, const PathRenderArgs& a, g19_s
             }
         }
     }
-    for (int i = first_side; i < n_lanes; ++i) { // join: the caller's stream continues after the other lanes
-        PATH_CUDA(cudaEventRecord(w.ev_join[i], w.side[i]));
-        PATH_CUDA(cudaStreamWaitEvent(s, w.ev_join[i], 0));
-    }
-    clk.s = s;
-    if (!fused && w.ray_hint_h && w.ray_hint_d.p && lanes[0].ray_hint)
-        PATH_CUDA(cudaMemcpyAsync(w.ray_hint_h, w.ray_hint_d.p, (kMaxPathDepth + 1) * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+    const int jrc = frame_join(w, a, f, clk, err);
+    if (jrc != G19_OK) return jrc;
     const int done_spp = int(stats.samples);
     clk.begin();
     if (a.frame_flags) {
@@ -1235,31 +1323,121 @@ int path_render(PathSceneBuffers& b, PathWork& w, const PathRenderArgs& a, g19_s
     }
     if (a.t_rad) PATH_CUDA(cudaMemcpyAsync(a.t_rad, w.rad_l.p, npix * 3 * sizeof(float), cudaMemcpyDeviceToDevice, s));
     if (a.t_rgb) PATH_CUDA(cudaMemcpyAsync(a.t_rgb, w.rgb_l.p, npix * 3, cudaMemcpyDeviceToDevice, s));
-    if (const char* le = path_launch_error()) {
-        err = le;
-        path_clear_launch_error();
-        cudaGetLastError();
-        // a pass stopped half way: its lanes' radiance planes and queue lengths are dirty -- re-zero them before the next render
-        for (PathLane& l : w.lane) l.capacity = 0;
-        return G19_ERR_CUDA;
-    }
+    const int lrc = frame_launch_error(w, err);
+    if (lrc != G19_OK) return lrc;
     PATH_CUDA(cudaGetLastError());
     for (int k = 0; k < 8; ++k) stats.kernel_launches += stats.class_launches[k];
     // owned in-frame pixels
     uint64_t owned = 0;
-    for (int lt = 0; lt < a.map.n_local_tiles; ++lt) {
-        int tile = lt * a.map.world + a.map.rank;
-        int ty = tile / a.map.tiles_x, tx = tile % a.map.tiles_x;
-        owned += uint64_t(std::min(kTile, a.map.w - tx * kTile)) * uint64_t(std::min(kTile, a.map.h - ty * kTile));
-    }
+    for (int lt = 0; lt < a.map.n_local_tiles; ++lt) owned += tile_pixels_in_frame(a.map, lt);
     stats.samples = owned * uint64_t(done_spp);
     w.totals_pending = true;
     w.totals_stream = s;
     ++w.frame_serial;
-    if (rc == G19_OK) w.overlap_key = this_key; // the next frame of the same shape may start behind this one's passes
+    if (rc == G19_OK) w.overlap_key = f.key; // the next frame of the same shape may start behind this one's passes
     return rc;
-#undef PATH_CUDA
 }
+
+// Rounds: round 0 gives every local tile samples [0, min_spp); after a round the tile test marks the tiles whose error is
+// still above tau (and below spp), the compaction lists them, and the next round gives those [n, min(2n, spp)). A round's
+// passes run over windows of the list (PassArgs::tiles), with the pass size and lanes path_render would use for this frame
+// at spp samples, so a tile's sums are those of path_render at its count.
+int path_render_adaptive(PathSceneBuffers& b, PathWork& w, const PathRenderArgs& a, float tau, int min_spp, float* d_var,
+                         int32_t* d_spp, g19_stats& stats, std::string& err) {
+    const g19_params& p = a.params;
+    if (p.max_depth < 1 || p.max_depth > kMaxPathDepth || min_spp < 2 || min_spp > p.spp || !(tau > 0.0f) || !std::isfinite(tau)) {
+        err = "adaptive PATH render needs 1 <= max_depth <= 64, 2 <= min_spp <= spp and a finite noise_target > 0";
+        return G19_ERR_INVALID;
+    }
+    cudaStream_t s = a.stream;
+    const TileMap& map = a.map;
+    const size_t n_tiles = size_t(map.n_local_tiles);
+    w.overlap_key = 0; // this frame's lanes and accum are not what the next g19_render's overlap expects
+    if (n_tiles == 0) return G19_OK;
+    path_clear_launch_error();
+    // per-tile state: [0] the length of the next list, [1 ..] the count of each local tile; the two lists; the flags
+    PATH_CUDA(w.tile_n.ensure((n_tiles + 1) * sizeof(int32_t)));
+    PATH_CUDA(w.tile_flag.ensure(n_tiles * sizeof(uint32_t)));
+    PATH_CUDA(w.tile_list.ensure(2 * n_tiles * sizeof(uint32_t)));
+    if (w.tile_h_n < n_tiles + 1) {
+        if (w.tile_h) cudaFreeHost(w.tile_h);
+        w.tile_h = nullptr;
+        w.tile_h_n = 0;
+        PATH_CUDA(cudaHostAlloc(reinterpret_cast<void**>(&w.tile_h), (n_tiles + 1) * sizeof(int32_t), cudaHostAllocDefault));
+        w.tile_h_n = n_tiles + 1;
+    }
+    int32_t* const d_tile = static_cast<int32_t*>(w.tile_n.p);
+    uint32_t* const d_flag = static_cast<uint32_t*>(w.tile_flag.p);
+    uint32_t* list[2] = {static_cast<uint32_t*>(w.tile_list.p), static_cast<uint32_t*>(w.tile_list.p) + n_tiles};
+    launch_iota(list[0], n_tiles, s); // round 0: every local tile (ahead of the side lanes' fork in frame_begin)
+    stats.class_launches[G19_K_OTHER] += 1;
+    Frame f;
+    f.pa0 = frame_args(b, a);
+    f.fused = path_scene_is_flat(f.pa0);
+    int rc = frame_begin(b, w, a, f, 4, false, err);
+    if (rc != G19_OK) return rc;
+    ClassClock clk{w, s, p.profile != 0};
+    uint32_t n_active = uint32_t(n_tiles);
+    int cur = 0, done = 0, upto = min_spp;
+    for (;;) {
+        for (int k = 0; k < f.n_lanes; ++k) f.lanes[k].tiles = list[cur];
+        const size_t positions = size_t(n_active) * kTilePix;
+        for (int base = done; base < upto; base += f.spp_pass) {
+            if (a.cancel && a.cancel->load()) { // g19_cancel: honoured between passes
+                rc = G19_ERR_CANCELLED;
+                break;
+            }
+            const int batch_spp = std::min(f.spp_pass, upto - base);
+            for (size_t pix0 = 0; pix0 < positions; pix0 += f.window) {
+                const int prc = frame_pass(b, w, a, f, clk, base, batch_spp, pix0, std::min(f.window, positions - pix0), stats, err);
+                if (prc != G19_OK) return prc;
+            }
+        }
+        const int jrc = frame_join(w, a, f, clk, err);
+        if (jrc != G19_OK) return jrc;
+        if (rc != G19_OK) break;
+        // the tile test sees the round's last accumulate through the join; the host reads the next list's length
+        clk.begin();
+        launch_tile_test(map, f.pa0.accum, list[cur], n_active, upto, p.spp, tau, d_tile + 1, d_flag, s);
+        launch_tile_compact(list[cur], n_active, d_flag, list[cur ^ 1], reinterpret_cast<uint32_t*>(d_tile), s);
+        clk.end(G19_K_OTHER);
+        stats.class_launches[G19_K_OTHER] += 2;
+        PATH_CUDA(cudaMemcpyAsync(w.tile_h, d_tile, (n_tiles + 1) * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+        PATH_CUDA(cudaStreamSynchronize(s));
+        const int lrc = frame_launch_error(w, err);
+        if (lrc != G19_OK) return lrc;
+        n_active = uint32_t(w.tile_h[0]);
+        if (a.progress_milli) a.progress_milli->store(int(1000.0 * double(upto) / double(p.spp)));
+        if (n_active == 0) break;
+        cur ^= 1;
+        done = upto;
+        upto = std::min(2 * upto, p.spp);
+        if (f.n_lanes > 1) { // the next round's passes read the new list: the side lanes start behind the compaction
+            PATH_CUDA(cudaEventRecord(w.ev_fork, s));
+            for (int i = f.first_side; i < f.n_lanes; ++i) PATH_CUDA(cudaStreamWaitEvent(w.side[i], w.ev_fork, 0));
+        }
+    }
+    if (rc == G19_OK) {
+        clk.begin();
+        launch_resolve_adaptive(map, f.pa0.accum, d_tile + 1, a.d_rgb, a.d_rad, d_var, d_spp, s);
+        clk.end(G19_K_OTHER);
+        stats.class_launches[G19_K_OTHER] += 1;
+    }
+    const int lrc = frame_launch_error(w, err);
+    if (lrc != G19_OK) return lrc;
+    PATH_CUDA(cudaGetLastError());
+    for (int k = 0; k < 8; ++k) stats.kernel_launches += stats.class_launches[k];
+    uint64_t samples = 0; // in-frame owned pixels times their tile's count (complete rounds only)
+    if (rc == G19_OK)
+        for (int lt = 0; lt < map.n_local_tiles; ++lt) samples += tile_pixels_in_frame(map, lt) * uint64_t(w.tile_h[1 + lt]);
+    stats.samples = samples;
+    w.totals_pending = true;
+    w.totals_stream = s;
+    ++w.frame_serial;
+    return rc;
+}
+
+#undef PATH_CUDA
 
 int path_finish_stats(PathWork& w, g19_stats& stats, std::string& err) {
     if (!w.totals_pending) return G19_OK;

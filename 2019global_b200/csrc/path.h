@@ -140,7 +140,13 @@ struct PathWork {
     unsigned long long overlap_key = 0; // (scene, pass size, lanes, depth ...) of the last frame that completed its enqueue, 0 = none
     int totals_parity = 0;
     DeviceArray totals;        // uint64[8]: extend segments, shadow segments, ...
-    DeviceArray accum;         // float[3][n_local_pix]
+    DeviceArray accum;         // float[3][n_local_pix]; adaptive renders: float[4][n_local_pix] (+ sum of Y^2 per pixel)
+    // adaptive renders only (path_render_adaptive), allocated by the first one: per local tile its sample count, the active
+    // flag the tile test sets, two compacted lists of active local tiles (this round's, the next round's) with their length
+    // at [0], and pinned host memory for the next list's length and the counts (read once per round)
+    DeviceArray tile_n, tile_flag, tile_list;
+    int32_t* tile_h = nullptr; // [0] active tiles, [1 ..] tile_n
+    size_t tile_h_n = 0;
     DeviceArray rad_l, rgb_l;  // resolved local-pixel outputs
     DeviceArray iota;          // uint32[2P + slack] 0, 1, 2, ...: the values the ray sort permutes
     size_t iota_n = 0;
@@ -235,6 +241,12 @@ int path_build_top_table(const PathNodeD* d_nodes, int top_level, uint2* d_table
 int path_upload(PathSceneBuffers& b, const g19_scene& scene, const PathTuning& tune, cudaStream_t stream, std::string& err);
 int path_render(PathSceneBuffers& b, PathWork& w, const PathRenderArgs& a, g19_stats& stats, std::string& err);
 int path_finish_stats(PathWork& w, g19_stats& stats, std::string& err);
+// Noise-targeted adaptive render (g19_render_adaptive, include/g19.h): rounds of passes over the compacted list of the
+// tiles whose error is still above tau; a.params.spp is the most samples a tile takes. Full-frame outputs (nullable): rgb and
+// radiance as path_render gives them at each tile's count, the variance of each pixel's mean, the tile's count.
+// Synchronises a.stream once per round. Host-pointer forms, progressive refresh and the shared frame are not served here.
+int path_render_adaptive(PathSceneBuffers& b, PathWork& w, const PathRenderArgs& a, float tau, int min_spp, float* d_var,
+                         int32_t* d_spp, g19_stats& stats, std::string& err);
 // Batched ray queries (g19_cast_rays) against the PATH view, on `stream`. Their state is their own, so a cast leaves every
 // render buffer as it was.
 struct PathCastWork {
@@ -297,6 +309,10 @@ struct PassArgs {
     int32_t walk;          // tree walk variant (PathTuning::walk); +2 when the walk counts its node / primitive tests
     int32_t flat_uniform;  // the flat bounce kernels trace through their FlatPairsU parameter (unrolled pair loops)
     const FlatPairsU* upairs; // host memory (PathSceneBuffers::upairs): what the launchers pass as that parameter
+    // adaptive passes (path_render_adaptive), nullptr otherwise: the window positions [pix_base, pix_base + pix_count) index
+    // a compacted list of local tiles, position pos = local pixel (tiles[pos >> 10] << 10) | (pos & 1023); the camera
+    // segment and accumulate run their LIST forms, and accumulate adds the per-sample luminance squared to accum's fourth plane
+    const uint32_t* tiles;
 };
 
 // path.cu: the PassArgs fields that follow from the scene and the tuning alone (staging sizes, walk and its knobs);
@@ -332,6 +348,17 @@ struct CastArgs {
 };
 void launch_cast(const PassArgs& a, const CastArgs& c, bool any, int sm_count, cudaStream_t s);
 void launch_resolve(const TileMap& map, const float* accum, int spp, float* rad_l, uint8_t* rgb_l, cudaStream_t s);
+// Adaptive renders. Tile test: one warp per entry of list[0 .. n_active): the tile's error E over its in-frame pixels at
+// n samples; tile_n[tile] = n, flag[entry] = E > tau and n < spp.
+void launch_tile_test(const TileMap& map, const float* accum, const uint32_t* list, uint32_t n_active, int n, int spp, float tau,
+                      int32_t* tile_n, uint32_t* flag, cudaStream_t s);
+// One CTA: the entries of list[0 .. n_active) whose flag is set, in order, to list_out; their number to *count_out.
+void launch_tile_compact(const uint32_t* list, uint32_t n_active, const uint32_t* flag, uint32_t* list_out, uint32_t* count_out,
+                         cudaStream_t s);
+// Per owned in-frame pixel at its tile's count: rgb / radiance (as resolve), variance of the mean, count (all nullable,
+// full-frame row-major).
+void launch_resolve_adaptive(const TileMap& map, const float* accum, const int32_t* tile_n, uint8_t* rgb, float* rad, float* var,
+                             int32_t* spp, cudaStream_t s);
 const char* path_launch_error(); // first failed launch/attribute call since the last clear, or nullptr
 void path_clear_launch_error();
 

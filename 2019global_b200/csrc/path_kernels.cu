@@ -1128,10 +1128,13 @@ __device__ __forceinline__ uint32_t fast_div(uint32_t n, uint32_t d, uint32_t& r
     return q;
 }
 
+// LIST (adaptive passes): the window runs over a compacted list of local tiles (PassArgs::tiles)
+template <bool LIST = false>
 __device__ __forceinline__ bool slot_pixel(const PassArgs& a, uint32_t slot, int& x, int& y, uint32_t& sample) {
     uint32_t lp, tx;
     uint32_t s = fast_div(slot, a.pix_count, lp); // slot = sample in pass * window size + pixel in window
     lp += a.pix_base;
+    if (LIST) lp = (a.tiles[lp >> 10] << 10) | (lp & 1023u);
     sample = (uint32_t)a.sample_base + s;
     uint32_t lt = lp >> 10, in = lp & 1023u;
     uint32_t t = lt * (uint32_t)a.map.world + (uint32_t)a.map.rank;
@@ -1290,7 +1293,7 @@ __device__ __forceinline__ void store_vertex(const PassArgs& a, uint32_t slot, f
 
 // ---- raygen + extend (camera segment), tree scenes: slot-indexed state ----------------------
 // 3 CTAs per SM at 80 registers (68 bytes of spills) beat 2 at 95 on the octree walk: 23.8 vs 26.4 ms per 66 M camera rays
-template <bool COOP, int WALK> __global__ void __launch_bounds__(kThreads, 3) raygen_extend_kernel(const PassArgs a) {
+template <bool COOP, int WALK, bool LIST = false> __global__ void __launch_bounds__(kThreads, 3) raygen_extend_kernel(const PassArgs a) {
     pdl_launch_dependents();
     const uint32_t n = a.n_slots;
     if (blockIdx.x * kThreads >= n) return;
@@ -1310,7 +1313,7 @@ template <bool COOP, int WALK> __global__ void __launch_bounds__(kThreads, 3) ra
         if (q < n) {
             int x, y;
             uint32_t sample;
-            live = slot_pixel(a, slot, x, y, sample);
+            live = slot_pixel<LIST>(a, slot, x, y, sample);
             if (live) {
                 pixel = uint32_t(y) * uint32_t(a.map.w) + uint32_t(x);
                 camera_ray(a, x, y, pixel, sample, o, d);
@@ -1572,7 +1575,7 @@ __device__ __forceinline__ void prefetch_rec(const RecView& r, uint32_t pos, boo
 // FOLD (the bounce before the last): the vertex the continuation ray finds would be the path's
 // last one -- next-event estimation only. It is shaded right here (light sample + shadow ray) instead of being written as a
 // 64-byte record for a launch of its own to read back: same arithmetic in the same order, one launch per pass fewer.
-template <int KIND, bool FIRST, bool LAST, bool SPEC, bool FUSED, bool FOLD, bool UNI>
+template <int KIND, bool FIRST, bool LAST, bool SPEC, bool FUSED, bool FOLD, bool UNI, bool LIST = false>
 __device__ __forceinline__ void bounce_flat_body(const PassArgs& a, const int bounce, const SceneAccess<true>& S, const uint32_t n,
                                                  const uint32_t cta, const uint32_t n_cta, RecStage<!FIRST>& stage) {
     constexpr bool kDiffuse = KIND == Q_DIFFUSE;
@@ -1601,7 +1604,7 @@ __device__ __forceinline__ void bounce_flat_body(const PassArgs& a, const int bo
             float3 o = f3(0.f, 0.f, 0.f);
             if (q < n) {
                 int x, y;
-                live = slot_pixel(a, q, x, y, sample);
+                live = slot_pixel<LIST>(a, q, x, y, sample);
                 if (live) {
                     pixel = uint32_t(y) * uint32_t(a.map.w) + uint32_t(x);
                     camera_ray(a, x, y, pixel, sample, o, d);
@@ -1788,8 +1791,8 @@ __global__ void __launch_bounds__(kThreads, 3) bounce_flat_kernel(const PassArgs
 }
 
 // The first bounce: camera segment + first vertex in one launch (bounce_flat_body<FUSED>), over the path slots of the pass
-// instead of a queue.
-template <bool LAST, bool FOLD, bool SPEC, bool UNI>
+// instead of a queue. LIST: an adaptive pass (slot_pixel).
+template <bool LAST, bool FOLD, bool SPEC, bool UNI, bool LIST = false>
 __global__ void __launch_bounds__(kThreads, 3) bounce_flat_fused_kernel(const PassArgs a, const __grid_constant__ FlatPairsU up) {
     pdl_launch_dependents();
     const uint32_t n = a.n_slots;
@@ -1798,7 +1801,7 @@ __global__ void __launch_bounds__(kThreads, 3) bounce_flat_fused_kernel(const Pa
     S.upairs = &up;
     pdl_wait(); // the previous pass's accumulate cleared the queue lengths
     RecStage<false>& unused = *reinterpret_cast<RecStage<false>*>(g19_dyn_smem); // (the fused body prefetches no records)
-    bounce_flat_body<Q_DIFFUSE, true, LAST, SPEC, true, FOLD, UNI>(a, 0, S, n, blockIdx.x, gridDim.x, unused);
+    bounce_flat_body<Q_DIFFUSE, true, LAST, SPEC, true, FOLD, UNI, LIST>(a, 0, S, n, blockIdx.x, gridDim.x, unused);
 }
 
 // All three material queues of one bounce in ONE launch (scenes with mirror / glass). The mirror and
@@ -2256,14 +2259,32 @@ __global__ void __launch_bounds__(kThreads, OCC) cast_kernel(const PassArgs a, c
 // ---- accumulate / resolve ---------------------------------------------------------------
 // FLAT: the finished paths' radiance is a float4 per slot, stored once for EVERY slot of the pass by the kernel
 // that ended its path, so it is only read here; otherwise three planes that paths add to and this kernel clears.
-template <bool FLAT> __global__ void __launch_bounds__(kThreads) accumulate_kernel(const PassArgs a) {
+// ADAPT (adaptive passes): the window positions go through the tile list (PassArgs::tiles), and a fourth plane of accum
+// takes the sum of Y^2 per pixel, Y = 0.2126 R + 0.7152 G + 0.0722 B of each sample, in the same sample order.
+__device__ __forceinline__ float luminance(float r, float g, float b) {
+    return __fmaf_rn(0.0722f, b, __fmaf_rn(0.7152f, g, __fmul_rn(0.2126f, r)));
+}
+template <bool ADAPT> struct Moment {
+    __device__ __forceinline__ void add(float, float, float) {}
+};
+template <> struct Moment<true> {
+    float s2;
+    __device__ __forceinline__ void add(float r, float g, float b) {
+        const float y = luminance(r, g, b);
+        s2 = __fmaf_rn(y, y, s2);
+    }
+};
+template <bool FLAT, bool ADAPT = false> __global__ void __launch_bounds__(kThreads) accumulate_kernel(const PassArgs a) {
     pdl_launch_dependents();
     pdl_wait();
     const uint32_t npix = (uint32_t)a.map.n_local_pix, nwin = a.pix_count;
     const uint32_t wp = blockIdx.x * kThreads + threadIdx.x; // pixel within the pass's window
     if (wp < nwin) {
-        const uint32_t lp = a.pix_base + wp;
+        uint32_t lp = a.pix_base + wp;
+        if (ADAPT) lp = (a.tiles[lp >> 10] << 10) | (lp & 1023u);
         float acc0 = a.accum[lp], acc1 = a.accum[(size_t)npix + lp], acc2 = a.accum[2 * (size_t)npix + lp];
+        Moment<ADAPT> mo;
+        if constexpr (ADAPT) mo.s2 = a.accum[3 * (size_t)npix + lp];
         // strictly in sample order (independent of the pass split); loads batched four samples deep
         if constexpr (FLAT) {
             float4* L = reinterpret_cast<float4*>(a.L) + wp;
@@ -2273,11 +2294,12 @@ template <bool FLAT> __global__ void __launch_bounds__(kThreads) accumulate_kern
 #pragma unroll
                 for (int k = 0; k < 4; ++k) v[k] = L[(size_t)(s + k) * nwin];
 #pragma unroll
-                for (int k = 0; k < 4; ++k) { acc0 += v[k].x; acc1 += v[k].y; acc2 += v[k].z; }
+                for (int k = 0; k < 4; ++k) { acc0 += v[k].x; acc1 += v[k].y; acc2 += v[k].z; mo.add(v[k].x, v[k].y, v[k].z); }
             }
             for (; s < a.spp_pass; ++s) {
                 const float4 v = L[(size_t)s * nwin];
                 acc0 += v.x; acc1 += v.y; acc2 += v.z;
+                mo.add(v.x, v.y, v.z);
             }
         } else {
             float* L0 = a.L + wp;
@@ -2295,6 +2317,7 @@ template <bool FLAT> __global__ void __launch_bounds__(kThreads) accumulate_kern
                 for (int k = 0; k < 4; ++k) {
                     size_t i = (size_t)(s + k) * nwin;
                     acc0 += v0[k]; acc1 += v1[k]; acc2 += v2[k];
+                    mo.add(v0[k], v1[k], v2[k]);
                     if (v0[k] != 0.0f) L0[i] = 0.0f;
                     if (v1[k] != 0.0f) L1[i] = 0.0f;
                     if (v2[k] != 0.0f) L2[i] = 0.0f;
@@ -2304,6 +2327,7 @@ template <bool FLAT> __global__ void __launch_bounds__(kThreads) accumulate_kern
                 size_t i = (size_t)s * nwin;
                 float v0 = L0[i], v1 = L1[i], v2 = L2[i];
                 acc0 += v0; acc1 += v1; acc2 += v2;
+                mo.add(v0, v1, v2);
                 if (v0 != 0.0f) L0[i] = 0.0f;
                 if (v1 != 0.0f) L1[i] = 0.0f;
                 if (v2 != 0.0f) L2[i] = 0.0f;
@@ -2312,6 +2336,7 @@ template <bool FLAT> __global__ void __launch_bounds__(kThreads) accumulate_kern
         a.accum[lp] = acc0;
         a.accum[(size_t)npix + lp] = acc1;
         a.accum[2 * (size_t)npix + lp] = acc2;
+        if constexpr (ADAPT) a.accum[3 * (size_t)npix + lp] = mo.s2;
     }
     // the pass is over: clear its queue lengths for the next one
     if (blockIdx.x == 0)
@@ -2330,6 +2355,99 @@ __global__ void __launch_bounds__(kThreads) resolve_kernel(TileMap map, const fl
         float cl = fminf(fmaxf(v, 0.0f), 1.0f);
         rgb_l[3 * (size_t)lp + c] = (uint8_t)(int)(255.0f * cl); // truncation, as Image::setPixel
     }
+}
+
+// ---- adaptive renders: tile test, compaction, resolve at each tile's count -----------------------------------
+// The variance of a pixel's mean after n samples, from its sums (accum planes 0-2: R, G, B; plane 3: Y^2):
+// m = 0.2126 R/n + 0.7152 G/n + 0.0722 B/n with the means resolve stores, v = max(S2 - n m^2, 0) / (n (n - 1)).
+__device__ __forceinline__ float pixel_variance(const float* __restrict__ accum, size_t npix, uint32_t lp, int n, float& m) {
+    const float fn = float(n);
+    m = luminance(__fdiv_rn(accum[lp], fn), __fdiv_rn(accum[npix + lp], fn), __fdiv_rn(accum[2 * npix + lp], fn));
+    const float d = __fsub_rn(accum[3 * npix + lp], __fmul_rn(fn, __fmul_rn(m, m)));
+    return __fdiv_rn(fmaxf(d, 0.0f), __fmul_rn(fn, fn - 1.0f));
+}
+
+// One warp per active tile; lane = column, 32 rows. Every pixel's error e = sqrt(v) / max(m, 0.05) is computed alone and
+// max is exact, so E does not depend on the reduction order.
+__global__ void __launch_bounds__(kThreads) tile_test_kernel(TileMap map, const float* __restrict__ accum, const uint32_t* __restrict__ list,
+                                                             uint32_t n_active, int n, int spp, float tau, int32_t* __restrict__ tile_n,
+                                                             uint32_t* __restrict__ flag) {
+    const uint32_t entry = (blockIdx.x * kThreads + threadIdx.x) >> 5, lane = threadIdx.x & 31u;
+    if (entry >= n_active) return;
+    const uint32_t lt = list[entry];
+    const uint32_t t = lt * (uint32_t)map.world + (uint32_t)map.rank;
+    const uint32_t ty = t / (uint32_t)map.tiles_x, tx = t - ty * (uint32_t)map.tiles_x;
+    const int x = int(tx * kTile + lane);
+    float E = 0.0f;
+    if (x < map.w)
+        for (int row = 0; row < kTile && int(ty * kTile) + row < map.h; ++row) {
+            float m;
+            const float v = pixel_variance(accum, (size_t)map.n_local_pix, (lt << 10) | (uint32_t(row) << 5) | lane, n, m);
+            E = fmaxf(E, __fdiv_rn(__fsqrt_rn(v), fmaxf(m, 0.05f)));
+        }
+    for (int off = 16; off > 0; off >>= 1) E = fmaxf(E, __shfl_xor_sync(kFull, E, off));
+    if (lane == 0) {
+        tile_n[lt] = n;
+        flag[entry] = (E > tau && n < spp) ? 1u : 0u;
+    }
+}
+
+// One CTA of 1024 threads walks the list in blocks of 1024 entries: warp ballots + a scan of the 32 warp totals. The
+// order of the list is kept (ascending local tile).
+__global__ void __launch_bounds__(1024) tile_compact_kernel(const uint32_t* __restrict__ list, uint32_t n_active,
+                                                            const uint32_t* __restrict__ flag, uint32_t* __restrict__ list_out,
+                                                            uint32_t* __restrict__ count_out) {
+    __shared__ uint32_t warp_base[32], block_total;
+    const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
+    uint32_t base = 0;
+    for (uint32_t i0 = 0; i0 < n_active; i0 += 1024u) {
+        const uint32_t i = i0 + threadIdx.x;
+        const bool keep = i < n_active && flag[i] != 0u;
+        const uint32_t m = __ballot_sync(kFull, keep);
+        if (lane == 0) warp_base[warp] = __popc(m);
+        __syncthreads();
+        if (warp == 0) { // exclusive scan of the warp totals
+            const uint32_t c = warp_base[lane];
+            uint32_t inc = c;
+            for (int off = 1; off < 32; off <<= 1) {
+                const uint32_t o = __shfl_up_sync(kFull, inc, off);
+                if (lane >= uint32_t(off)) inc += o;
+            }
+            warp_base[lane] = inc - c;
+            if (lane == 31) block_total = inc;
+        }
+        __syncthreads();
+        if (keep) list_out[base + warp_base[warp] + __popc(m & ((1u << lane) - 1u))] = list[i];
+        base += block_total;
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) *count_out = base;
+}
+
+__global__ void __launch_bounds__(kThreads) resolve_adaptive_kernel(TileMap map, const float* __restrict__ accum,
+                                                                    const int32_t* __restrict__ tile_n, uint8_t* rgb, float* rad,
+                                                                    float* var, int32_t* spp) {
+    const uint32_t lp = blockIdx.x * kThreads + threadIdx.x;
+    if (lp >= (uint32_t)map.n_local_pix) return;
+    const uint32_t lt = lp >> 10, in = lp & 1023u;
+    const uint32_t t = lt * (uint32_t)map.world + (uint32_t)map.rank;
+    const uint32_t ty = t / (uint32_t)map.tiles_x, tx = t - ty * (uint32_t)map.tiles_x;
+    const int x = int(tx * kTile + (in & 31u)), y = int(ty * kTile + (in >> 5));
+    if (y >= map.h || x >= map.w) return;
+    const int n = tile_n[lt];
+    const size_t npix = (size_t)map.n_local_pix, gpx = (size_t)y * map.w + x;
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+        const float v = __fdiv_rn(accum[c * npix + lp], float(n));
+        if (rad) rad[3 * gpx + c] = v;
+        const float cl = fminf(fmaxf(v, 0.0f), 1.0f);
+        if (rgb) rgb[3 * gpx + c] = (uint8_t)(int)(255.0f * cl); // truncation, as Image::setPixel
+    }
+    if (var) {
+        float m;
+        var[gpx] = pixel_variance(accum, npix, lp, n, m);
+    }
+    if (spp) spp[gpx] = n;
 }
 
 // Persistent grids: SM count x the CTAs the occupancy calculator says are resident.
@@ -2432,14 +2550,17 @@ template <int KIND> static void launch_bounce_fl(const PassArgs& a, int bounce, 
 
 } // namespace
 
+template <bool LIST> static void (*raygen_extend_k(const PassArgs& a))(PassArgs) {
+    if (a.walk == 6) return raygen_extend_kernel<false, 6, LIST>;
+    if (a.walk == 5) return raygen_extend_kernel<false, 5, LIST>;
+    if (a.walk == 3) return raygen_extend_kernel<false, 3, LIST>;
+    if (a.walk == 2) return a.coop_leaf ? raygen_extend_kernel<true, 2, LIST> : raygen_extend_kernel<false, 2, LIST>;
+    return a.coop_leaf ? raygen_extend_kernel<true, 1, LIST> : raygen_extend_kernel<false, 1, LIST>;
+}
+
 void launch_raygen_extend(const PassArgs& a, int sm_count, cudaStream_t s) {
     const size_t smem = path_smem_bytes(a);
-    void (*kernel)(PassArgs);
-    if (a.walk == 6) kernel = raygen_extend_kernel<false, 6>;
-    else if (a.walk == 5) kernel = raygen_extend_kernel<false, 5>;
-    else if (a.walk == 3) kernel = raygen_extend_kernel<false, 3>;
-    else if (a.walk == 2) kernel = a.coop_leaf ? raygen_extend_kernel<true, 2> : raygen_extend_kernel<false, 2>;
-    else kernel = a.coop_leaf ? raygen_extend_kernel<true, 1> : raygen_extend_kernel<false, 1>;
+    void (*kernel)(PassArgs) = a.tiles ? raygen_extend_k<true>(a) : raygen_extend_k<false>(a);
     const int grid = persistent_grid(kernel, smem, sm_count);
     const cudaError_t e = launch_pdl(kernel, grid, smem, s, a);
     if (e != cudaSuccess) note_launch_error("raygen_extend kernel launch", e, smem, grid);
@@ -2460,18 +2581,20 @@ void launch_trace(const PassArgs& a, int bounce, int sm_count, cudaStream_t s) {
 
 bool path_scene_is_flat(const PassArgs& a) { return all_staged(a); }
 
-void launch_bounce_first_fused(const PassArgs& a, int sm_count, cudaStream_t s) {
-    const size_t smem = path_smem_bytes(a);
-    void (*kernel)(PassArgs, FlatPairsU);
+template <bool LIST> static void (*first_fused_k(const PassArgs& a))(PassArgs, FlatPairsU) {
     const bool u = a.flat_uniform != 0;
     if (a.kind_mask & 6u) // mirror / glass in the scene: diffuse camera hits shaded in place, specular ones queued
-        kernel = a.max_depth <= 1 ? (u ? bounce_flat_fused_kernel<true, false, true, true> : bounce_flat_fused_kernel<true, false, true, false>)
-                 : a.fold_last    ? (u ? bounce_flat_fused_kernel<false, true, true, true> : bounce_flat_fused_kernel<false, true, true, false>)
-                                  : (u ? bounce_flat_fused_kernel<false, false, true, true> : bounce_flat_fused_kernel<false, false, true, false>);
-    else
-        kernel = a.max_depth <= 1 ? (u ? bounce_flat_fused_kernel<true, false, false, true> : bounce_flat_fused_kernel<true, false, false, false>)
-                 : a.fold_last    ? (u ? bounce_flat_fused_kernel<false, true, false, true> : bounce_flat_fused_kernel<false, true, false, false>)
-                                  : (u ? bounce_flat_fused_kernel<false, false, false, true> : bounce_flat_fused_kernel<false, false, false, false>);
+        return a.max_depth <= 1 ? (u ? bounce_flat_fused_kernel<true, false, true, true, LIST> : bounce_flat_fused_kernel<true, false, true, false, LIST>)
+               : a.fold_last    ? (u ? bounce_flat_fused_kernel<false, true, true, true, LIST> : bounce_flat_fused_kernel<false, true, true, false, LIST>)
+                                : (u ? bounce_flat_fused_kernel<false, false, true, true, LIST> : bounce_flat_fused_kernel<false, false, true, false, LIST>);
+    return a.max_depth <= 1 ? (u ? bounce_flat_fused_kernel<true, false, false, true, LIST> : bounce_flat_fused_kernel<true, false, false, false, LIST>)
+           : a.fold_last    ? (u ? bounce_flat_fused_kernel<false, true, false, true, LIST> : bounce_flat_fused_kernel<false, true, false, false, LIST>)
+                            : (u ? bounce_flat_fused_kernel<false, false, false, true, LIST> : bounce_flat_fused_kernel<false, false, false, false, LIST>);
+}
+
+void launch_bounce_first_fused(const PassArgs& a, int sm_count, cudaStream_t s) {
+    const size_t smem = path_smem_bytes(a);
+    void (*kernel)(PassArgs, FlatPairsU) = a.tiles ? first_fused_k<true>(a) : first_fused_k<false>(a);
     const int grid = persistent_grid(kernel, smem, sm_count);
     cudaError_t e = launch_pdl(kernel, grid, smem, s, a, launch_pairs(a));
     if (e != cudaSuccess) note_launch_error("fused first bounce kernel launch", e, smem, grid);
@@ -2507,7 +2630,9 @@ void path_clear_launch_error() { g_launch_error[0] = 0; }
 void launch_accumulate(const PassArgs& a, cudaStream_t s) {
     int blocks = int((a.pix_count + kThreads - 1) / kThreads);
     if (blocks < 1) blocks = 1;
-    cudaError_t e = all_staged(a) ? launch_pdl(accumulate_kernel<true>, blocks, 0, s, a) : launch_pdl(accumulate_kernel<false>, blocks, 0, s, a);
+    void (*kernel)(PassArgs) = all_staged(a) ? (a.tiles ? accumulate_kernel<true, true> : accumulate_kernel<true, false>)
+                                             : (a.tiles ? accumulate_kernel<false, true> : accumulate_kernel<false, false>);
+    cudaError_t e = launch_pdl(kernel, blocks, 0, s, a);
     if (e != cudaSuccess) note_launch_error("accumulate kernel launch", e, 0, blocks);
 }
 
@@ -2548,6 +2673,24 @@ void launch_cast(const PassArgs& a, const CastArgs& c, bool any, int sm_count, c
 void launch_resolve(const TileMap& map, const float* accum, int spp, float* rad_l, uint8_t* rgb_l, cudaStream_t s) {
     if (map.n_local_pix == 0) return;
     resolve_kernel<<<(map.n_local_pix + kThreads - 1) / kThreads, kThreads, 0, s>>>(map, accum, spp, rad_l, rgb_l);
+}
+
+void launch_tile_test(const TileMap& map, const float* accum, const uint32_t* list, uint32_t n_active, int n, int spp, float tau,
+                      int32_t* tile_n, uint32_t* flag, cudaStream_t s) {
+    if (n_active == 0) return;
+    const uint32_t blocks = (n_active * 32u + kThreads - 1) / kThreads;
+    tile_test_kernel<<<blocks, kThreads, 0, s>>>(map, accum, list, n_active, n, spp, tau, tile_n, flag);
+}
+
+void launch_tile_compact(const uint32_t* list, uint32_t n_active, const uint32_t* flag, uint32_t* list_out, uint32_t* count_out,
+                         cudaStream_t s) {
+    tile_compact_kernel<<<1, 1024, 0, s>>>(list, n_active, flag, list_out, count_out);
+}
+
+void launch_resolve_adaptive(const TileMap& map, const float* accum, const int32_t* tile_n, uint8_t* rgb, float* rad, float* var,
+                             int32_t* spp, cudaStream_t s) {
+    if (map.n_local_pix == 0) return;
+    resolve_adaptive_kernel<<<(map.n_local_pix + kThreads - 1) / kThreads, kThreads, 0, s>>>(map, accum, tile_n, rgb, rad, var, spp);
 }
 
 } // namespace g19

@@ -34,6 +34,7 @@ EXPORTS = [
     "g19_frame_read", "g19_render_progressive", "g19_render_tiles_device", "g19_untile_device", "g19_tile_pixels",
     "g19_probe_texcoord", "g19_probe_shade", "g19_probe_path_tree", "g19_entity_bbox", "g19_entity_triangles",
     "g19_frame_status", "g19_tune", "g19_scene_set_shapes", "g19_cast_rays", "g19_cast_rays_device",
+    "g19_render_adaptive", "g19_render_adaptive_device",
 ]
 
 
@@ -105,6 +106,11 @@ def lib():
         L.g19_cast_rays.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p]
         L.g19_cast_rays_device.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p,
                                            C.c_void_p]
+        L.g19_render_adaptive.argtypes = [C.c_void_p, C.POINTER(abi.Camera), C.c_void_p, C.POINTER(abi.Params),
+                                          C.POINTER(abi.Adaptive), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+        L.g19_render_adaptive_device.argtypes = [C.c_void_p, C.POINTER(abi.Camera), C.c_void_p, C.POINTER(abi.Params),
+                                                 C.POINTER(abi.Adaptive), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                 C.c_void_p]
         _lib = L
     return _lib
 
@@ -306,6 +312,32 @@ class RayTracer:
         return self._check(self._L.g19_render_device(self.h, C.byref(self.camera), abi.d3(self.light), C.byref(p),
                                                      C.c_void_p(d_rgb), C.c_void_p(d_ids), C.c_void_p(d_rad),
                                                      C.c_void_p(stream)), allow=(abi.ERR_CANCELLED,))
+
+    def run_adaptive(self, w, h, noise_target, min_spp, spp, max_depth, seed=0, want=("rgb", "radiance", "variance", "spp"),
+                     out=None, **kw):
+        """Blocking PATH-mode render with noise-targeted adaptive sampling (g19_render_adaptive): a 32x32 tile stops once
+        its worst pixel's relative standard error is <= noise_target; counts are min_spp * 2^k up to spp. Returns a dict of
+        numpy arrays: "rgb" (h,w,3) uint8, "radiance" (h,w,3) float32, "variance" (h,w) float32 (variance of each pixel's
+        mean luminance), "spp" (h,w) int32 (each pixel's sample count); None for what `want` leaves out. kw: the other
+        params() fields (rank, world, spp_per_pass, pixels_per_pass, profile)."""
+        p = self.params(w, h, abi.MODE_PATH, spp=spp, max_depth=max_depth, seed=seed, **kw)
+        ad = abi.Adaptive(float(noise_target), int(min_spp))
+        out = out or {}
+        shapes = {"rgb": ((h, w, 3), np.uint8), "radiance": ((h, w, 3), np.float32), "variance": ((h, w), np.float32),
+                  "spp": ((h, w), np.int32)}
+        res = {k: ((out[k] if k in out else np.zeros(*shapes[k])) if k in want else None) for k in shapes}
+        self._check(self._L.g19_render_adaptive(self.h, C.byref(self.camera), abi.d3(self.light), C.byref(p), C.byref(ad),
+                                                _ptr(res["rgb"]), _ptr(res["radiance"]), _ptr(res["variance"]), _ptr(res["spp"])),
+                    allow=(abi.ERR_CANCELLED,))
+        return res
+
+    def run_adaptive_device(self, p, adaptive, d_rgb=0, d_rad=0, d_var=0, d_spp=0, stream=0):
+        """g19_render_adaptive_device into device pointers (ints, e.g. torch.Tensor.data_ptr()); p: abi.Params, adaptive:
+        abi.Adaptive. Stream-ordered, but synchronises `stream` once per round."""
+        return self._check(self._L.g19_render_adaptive_device(self.h, C.byref(self.camera), abi.d3(self.light), C.byref(p),
+                                                              C.byref(adaptive), C.c_void_p(d_rgb), C.c_void_p(d_rad),
+                                                              C.c_void_p(d_var), C.c_void_p(d_spp), C.c_void_p(stream)),
+                           allow=(abi.ERR_CANCELLED,))
 
     def cast(self, origins, dirs, tmax=None, any_hit=False, want_normals=False, count=False):
         """Batched ray queries against the PATH view of the scene (g19_cast_rays, blocking). origins, dirs: (n, 3);

@@ -251,6 +251,41 @@ int g19_render_device(g19_ctx* ctx, const g19_camera* camera, const double light
                       float* d_radiance, void* stream);
 int g19_get_stats(g19_ctx* ctx, g19_stats* out);
 
+/* Noise-targeted adaptive sampling (PATH mode): samples go where the frame is still noisy, a 32x32 tile at a time. No
+ * counterpart in the reference (one sample per pixel).
+ *   mode        G19_MODE_PATH only. params->spp is the most samples a pixel takes; rank / world, spp_per_pass,
+ *               pixels_per_pass, profile and the g19_tune knobs mean what they mean for g19_render. Pixels of other
+ *               ranks are left untouched
+ *   rounds      round 0 gives every owned tile samples [0, min_spp). After each round every active tile is tested: one
+ *               whose error E <= noise_target stops; any other with n samples takes samples [n, min(2n, spp)) in the next
+ *               round. The render ends when no tile is active: counts are min_spp * 2^k, capped at spp
+ *   error       per sample Y = 0.2126 R + 0.7152 G + 0.0722 B (FP32, of the radiance g19_render averages); per pixel
+ *               S2 = sum of Y^2 (FP32, in sample order), m = 0.2126 sum(R)/n + 0.7152 sum(G)/n + 0.0722 sum(B)/n (the
+ *               radiance output's means), v = max(S2 - n m^2, 0) / (n (n - 1)) -- the variance of the pixel's mean --
+ *               and e = sqrt(v) / max(m, 0.05) (below 5 % of display white the test is absolute); E = the largest e
+ *               over the tile's in-frame pixels
+ *   outputs     all nullable, full frame, row-major. rgb888 (w*h*3 bytes) and radiance (w*h*3 floats): exactly what
+ *               g19_render gives at spp = the pixel's count, so a tile that stopped at n samples holds the bytes of a
+ *               uniform render at n; variance (w*h floats): v at that count; spp (w*h int32): that count
+ *   stats       samples = the sum over owned in-frame pixels of their count (g19_render's count when every tile
+ *               reaches spp); the other fields as for g19_render
+ *   errors      G19_ERR_INVALID: ctx, params or adaptive NULL, REF mode, noise_target not finite or <= 0, min_spp < 2
+ *               or > spp, max_depth < 1 (and whatever g19_render refuses); G19_ERR_NO_SCENE before an upload;
+ *               G19_ERR_CANCELLED: g19_cancel, seen between passes -- the outputs are then left as they were
+ *   device form stream-ordered on `stream` (a cudaStream_t, NULL = legacy default), but it synchronises `stream` once
+ *               per round to read how many tiles are still active (a pinned word): one host round trip per round,
+ *               and there are at most ceil(log2(spp / min_spp)) + 1 rounds. The host form blocks.                  */
+typedef struct g19_adaptive {
+    float noise_target; /* tau > 0, finite: a tile stops once its error E <= tau                   */
+    int32_t min_spp;    /* samples every owned pixel takes before the first test, 2 <= min_spp <= spp */
+} g19_adaptive;
+int g19_render_adaptive(g19_ctx* ctx, const g19_camera* camera, const double light[3], const g19_params* params,
+                        const g19_adaptive* adaptive, uint8_t* rgb888_out, float* radiance_out, float* variance_out,
+                        int32_t* spp_out);
+int g19_render_adaptive_device(g19_ctx* ctx, const g19_camera* camera, const double light[3], const g19_params* params,
+                               const g19_adaptive* adaptive, uint8_t* d_rgb888, float* d_radiance, float* d_variance,
+                               int32_t* d_spp, void* stream);
+
 /* Batched ray queries: what does each ray hit first, or is anything in its way (Embree's rtcIntersect /
  * rtcOccluded, OptiX's closest-hit / any-hit). No counterpart in the reference: its Octree::intersect
  * (octree.h:46-68) returns candidates, not hits.

@@ -29,7 +29,7 @@ import tempfile
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CUDA = "/usr/local/cuda/bin/"
 C2_KERNELS = [
-    ("fused (bounce 0)", r"bounce_flat_fused_kernel<false, false, false(, %s)?>"),
+    ("fused (bounce 0)", r"bounce_flat_fused_kernel<false, false, false(, %s)?(, false)?>"),
     ("plain (middle bounces)", r"bounce_flat_kernel<false, %s>"),
     ("FOLD (bounce before the last)", r"bounce_flat_kernel<true, %s>"),
 ]
